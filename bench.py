@@ -2,9 +2,14 @@
 """bench.py -- the sort hot path on B200, measured the way BASELINE.json's metric is quoted.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--algo radix|merge] [--dist uniform|...] [--log2n L]
+                    [--algo radix|merge] [--dist uniform|...] [--log2n L] [--dump-outputs DIR]
 
 A step is ONE full sort of one batch of keys.
+
+--dump-outputs DIR writes DIR/sorted_keys.npy: the sorted keys of the last timed step as float64 (exact for int32), all
+of them up to 2^22 keys, else the keys at the positions dump_positions(n) picks (a fixed, seeded sample).  The input
+depends only on the arguments, so two builds can be compared output for output.  Our arm on one GPU and the reference
+arm (its host sample, see below) write it; the multi-GPU sort does not.
 
 N = 1   workload = BASELINE configs[1..3]' single-GPU case at the size the metric is quoted on:
         n = 2^28 uniform int32 keys, onesweep radix sort (``--algo merge`` gives configs[2]).
@@ -132,6 +137,26 @@ class ClockSampler(threading.Thread):
                 "samples": len(inside), "how": how}
 
 
+# ---- --dump-outputs ----------------------------------------------------------------------------------
+DUMP_KEYS = 1 << 22          # 32 MiB of float64
+
+
+def dump_positions(n: int):
+    """Output positions --dump-outputs writes: all n up to DUMP_KEYS, else one position in each of DUMP_KEYS
+    equal strata, drawn from a fixed seed, so the sample covers the whole output and depends on n alone."""
+    import numpy as np
+    if n <= DUMP_KEYS:
+        return np.arange(n, dtype=np.int64)
+    stride = n // DUMP_KEYS
+    return np.arange(DUMP_KEYS, dtype=np.int64) * stride + np.random.default_rng(0).integers(0, stride, DUMP_KEYS)
+
+
+def _save_dump(dump_dir: str, sorted_keys_sample) -> None:
+    import numpy as np
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, "sorted_keys.npy"), sorted_keys_sample.astype(np.float64))
+
+
 # ---- reference arm -----------------------------------------------------------------------------------
 def _cpu_sorter():
     """(callable sorting a numpy int32 array in place, kind, description)."""
@@ -164,6 +189,8 @@ def reference_arm(args) -> None:
         t = time.perf_counter()
         sort_inplace(work)
         elapsed += time.perf_counter() - t
+    if args.dump_outputs:
+        _save_dump(args.dump_outputs, work[dump_positions(m)])
     value = m * args.steps / elapsed
     sample = (f"each step sorts a bounded sample of 2^{log2m} {args.dist} keys (seed 1) of the 2^{args.log2n} "
               f"workload on the host; {what}")
@@ -376,6 +403,8 @@ def ours_single(args) -> None:
     ms_per_step = ms_total / args.steps
     value = n / (ms_per_step / 1000.0)
     _check_sorted(torch, out, src)
+    if args.dump_outputs:                 # before the per-kernel timing below sorts into `out` again
+        _save_dump(args.dump_outputs, out[torch.from_numpy(dump_positions(n)).to(dev)].cpu().numpy())
 
     # ---- per-kernel timing (CUDA events between the kernels, on the launching stream) ----------
     peaks = _peaks()
@@ -515,11 +544,17 @@ def main() -> None:
                     help="multi-GPU: 2^T keys IN TOTAL split over the ranks (strong scaling; BASELINE config 5: 30)")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="multi-GPU exchange: fused peer-write scatter (default) or NCCL all-to-all")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's sorted keys to DIR/sorted_keys.npy (one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and args.impl == "ours" and (world > 1 or args.gpus > 1):
+        ap.error("--dump-outputs is not implemented for the multi-GPU sort")
     if args.impl == "reference":
         reference_arm(args)
         return
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1 or args.gpus > 1:
         from b200sort import dist as b200dist
         b200dist.bench_main(args, METRIC, UNIT, ClockSampler, _peaks)

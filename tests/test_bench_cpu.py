@@ -31,6 +31,28 @@ def test_reference_arm_other_ranks_stay_silent():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_arguments_it_cannot_honour_are_rejected():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--steps", "0"], ["--gpus", "2", "--dump-outputs", "d"]):
+        r = subprocess.run([sys.executable, "bench.py", *extra], cwd=ROOT, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and r.stdout == "" and "error:" in r.stderr, extra
+
+
+def test_reference_arm_dumps_the_sorted_sample_it_timed(tmp_path):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from b200sort import datagen
+    d = tmp_path / "dump"
+    r = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(d)], cwd=ROOT, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr
+    m = 1 << 24                                      # the arm's host sample at this step count
+    assert os.listdir(d) == ["sorted_keys.npy"]
+    got = np.load(d / "sorted_keys.npy")
+    assert got.dtype == np.float64 and got.shape == (bench.DUMP_KEYS,)
+    assert np.array_equal(got, np.sort(datagen.make("uniform", m, 1))[bench.dump_positions(m)].astype(np.float64))
+
+
 def test_roofline_traffic_comes_from_the_committed_ncu_summary():
     sys.path.insert(0, ROOT)
     import bench

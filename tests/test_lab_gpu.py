@@ -63,6 +63,19 @@ def test_streamed_host_operator_large_arrays(n):
         L.b200sort_host_set_streaming(1)
 
 
+def test_host_operator_matches_the_stored_reference_outputs(golden_small, golden_mixed):
+    """Both drop-in entry points against what the reference's own code returned (its CPU path, stored by
+    tests/golden/make_golden.py): the same bytes on its sign domain; on mixed signs its unsigned order rotated
+    to signed order."""
+    for fn in (b200sort.order_array, b200sort.order_with_trust):
+        for name, (keys, ref_out) in golden_small.items():
+            a = keys.copy(); fn(a)
+            assert_bit_exact(a, ref_out, f"{fn.__name__} {name}")
+        for name, (keys, ref_out) in golden_mixed.items():
+            a = keys.copy(); fn(a)
+            assert_bit_exact(a, np.roll(ref_out, int((keys < 0).sum())), f"{fn.__name__} {name}")
+
+
 def test_cxx_symbols_sort_in_place_like_the_reference_header_says():
     L = b200sort.lib()
     for sym in ("_Z11order_arrayPii", "_Z16order_with_trustPii"):
@@ -86,12 +99,12 @@ def test_reference_drivers_link_and_run_unmodified(tmp_path):
     assert rows[1].startswith("256,") and rows[1].endswith(",Our")
 
 
-def test_checked_driver():
+def test_checked_driver(tmp_path):
     path = os.path.join(ROOT, "build", "b200sort_driver")
     if not os.path.exists(path):
         pytest.skip("build/b200sort_driver not built")
     r = subprocess.run([path, "--min", "256", "--max", "1048576", "--dist", "uniform", "--check"],
-                       capture_output=True, text=True, timeout=300)
+                       cwd=tmp_path, capture_output=True, text=True, timeout=300)   # it writes output.txt
     assert r.returncode == 0, r.stdout + r.stderr
     assert "MISMATCH" not in r.stdout
 
