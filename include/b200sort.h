@@ -116,6 +116,37 @@ int    b200sort_sort_copy_i32(int algo, const int32_t *d_in, int32_t *d_out, int
 int    b200sort_sort_timed_i32(int algo, const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n,
                                void *d_ws, size_t ws_bytes, void *stream, float *ms);
 
+/* ---- other key types and descending order ------------------------------------------------------
+ * Keys are 32-bit words; key_type says how they compare:
+ *   B200SORT_KEY_I32  signed integers, numeric order (the _i32 entry points' order);
+ *   B200SORT_KEY_U32  unsigned integers, numeric order;
+ *   B200SORT_KEY_F32  IEEE-754 binary32 in totalOrder on the bit pattern:
+ *                     -NaN (sign bit set, any payload) < -inf < negatives < -0.0 < +0.0 < positives < +inf < +NaN,
+ *                     NaNs of one sign ordered by payload.  Bits are never changed: the output is the input's bit
+ *                     patterns permuted.  This is NOT the order of torch.sort / np.sort, which treat -0.0 == +0.0
+ *                     and put every NaN last.
+ * descending = 1 is the reverse order of the same key type.  Distinct bit patterns never compare equal, so a keys-only
+ * result is unique.  Sort-by-key stays STABLE in both directions (equal keys keep their input order), so a descending
+ * pairs result is not the reverse of the ascending one; without NaN or -0.0 it equals
+ * torch.sort(stable=True, descending=True).
+ * Internally every order is image(k) = k ^ (top bit of k set ? M_neg : M_pos) sorted as uint32 (DESIGN section 4.2c).
+ * (B200SORT_KEY_I32, ascending) runs exactly the code of the _i32 entry points. */
+#define B200SORT_KEY_I32            0
+#define B200SORT_KEY_U32            1
+#define B200SORT_KEY_F32            2
+/* d_out = d_in sorted (d_in may equal d_out; otherwise it is only read).  algo: RADIX or MERGE; LAB only with
+ * (B200SORT_KEY_I32, 0) -- its 1-bit split is signed by construction.  Workspace: b200sort_workspace_bytes(n, algo),
+ * unchanged.  Unknown key_type, descending not 0/1, NULL pointers, n > B200SORT_MAX_N, a radix shape selected with
+ * b200sort_radix_set_variant that has no generic instantiation (make EXPERIMENTS=1 shapes) -> B200SORT_ERR_INVALID;
+ * missing or small workspace -> B200SORT_ERR_WORKSPACE; all checked before any device work. */
+int    b200sort_sort_keys(int algo, int key_type, int descending, const void *d_in, void *d_out, void *d_tmp,
+                          size_t n, void *d_ws, size_t ws_bytes, void *stream);
+/* Stable sort-by-key on the radix path; same in-place / copy rules as b200sort_radix_pairs_copy_i32 (in place iff
+ * d_keys_in == d_keys_out and d_vals_in == d_vals_out). */
+int    b200sort_radix_pairs_keys(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                 void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                 size_t n, void *d_ws, size_t ws_bytes, void *stream);
+
 /* ---- stages, exposed for unit tests and per-kernel timing -------------------------------------- */
 
 /* d_hist[p*256+d] (uint32) = number of keys whose digit p of (key ^ 0x80000000) equals d.

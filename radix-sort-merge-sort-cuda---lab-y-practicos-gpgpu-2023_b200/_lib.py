@@ -44,6 +44,8 @@ SIGNATURES = {
     "b200sort_sort_i32": (_i, [_i, _vp, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_sort_copy_i32": (_i, [_i, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_sort_timed_i32": (_i, [_i, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _vp]),
+    "b200sort_sort_keys": (_i, [_i, _i, _i, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_radix_pairs_keys": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_radix_histogram_i32": (_i, [_vp, _sz, _vp, _vp]),
     "b200sort_radix_pass_i32": (_i, [_vp, _vp, _sz, _i, _vp, _sz, _vp]),
     "b200sort_block_sort_tile": (_sz, []),

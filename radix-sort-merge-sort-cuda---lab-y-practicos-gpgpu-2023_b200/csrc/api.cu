@@ -437,6 +437,37 @@ int b200sort_sort_timed_i32(int algo, const int32_t *d_in, int32_t *d_out, int32
     return sort_dispatch(algo, d_in, d_out, d_tmp, n, d_ws, ws_bytes, static_cast<cudaStream_t>(stream), ms);
 }
 
+int b200sort_sort_keys(int algo, int key_type, int descending, const void *d_in, void *d_out, void *d_tmp, size_t n,
+                       void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor order;
+    if (!key_order(key_type, descending, &order)) return B200SORT_ERR_INVALID;
+    B200_TRY(check_sort_args(d_out, d_tmp, n));
+    if (n > 0 && d_in == nullptr) return B200SORT_ERR_INVALID;
+    const auto *in = static_cast<const int32_t *>(d_in);
+    auto *out = static_cast<int32_t *>(d_out), *tmp = static_cast<int32_t *>(d_tmp);
+    const auto s = static_cast<cudaStream_t>(stream);
+    if (key_type == B200SORT_KEY_I32 && descending == 0) return sort_dispatch(algo, in, out, tmp, n, d_ws, ws_bytes, s);
+    switch (algo) {
+        case B200SORT_ALGO_RADIX: return radix_sort(in, out, tmp, n, d_ws, ws_bytes, s, &order);
+        case B200SORT_ALGO_MERGE: return merge_sort_keys(in, out, tmp, n, d_ws, ws_bytes, s, order);
+        default: return B200SORT_ERR_INVALID;      // the lab pipeline sorts int32 ascending only
+    }
+}
+
+int b200sort_radix_pairs_keys(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                              void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals, size_t n,
+                              void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor order;
+    if (!key_order(key_type, descending, &order)) return B200SORT_ERR_INVALID;
+    B200_TRY(check_sort_args(d_keys_out, d_tmp_keys, n));
+    B200_TRY(check_sort_args(d_vals_out, d_tmp_vals, n));
+    if (n > 0 && (d_keys_in == nullptr || d_vals_in == nullptr)) return B200SORT_ERR_INVALID;
+    const bool i32_asc = key_type == B200SORT_KEY_I32 && descending == 0;
+    return radix_sort_pairs(static_cast<const int32_t *>(d_keys_in), static_cast<int32_t *>(d_keys_out),
+                            static_cast<int32_t *>(d_tmp_keys), d_vals_in, d_vals_out, d_tmp_vals, n, d_ws, ws_bytes,
+                            static_cast<cudaStream_t>(stream), i32_asc ? nullptr : &order);
+}
+
 int b200sort_radix_histogram_i32(const int32_t *d_keys, size_t n, uint32_t *d_hist, void *stream) {
     if (d_hist == nullptr || (n > 0 && d_keys == nullptr) || n > B200SORT_MAX_N) return B200SORT_ERR_INVALID;
     return radix_histogram(d_keys, n, d_hist, static_cast<cudaStream_t>(stream));

@@ -76,6 +76,39 @@ __host__ __device__ __forceinline__ uint32_t key_bits(int32_t k) {
     return static_cast<uint32_t>(k) ^ 0x80000000u;
 }
 
+// ---- key orders (b200sort_sort_keys) ------------------------------------------------------------
+// Every supported order of 32-bit keys is a bijection onto uint32 of the form
+//   image(k) = k ^ (k has its top bit set ? neg : pos)
+// and the keys are sorted by their images, unsigned ascending.  The same form with other masks maps an
+// image back to its key, or a key to a signed-comparable int32 (image ^ 0x80000000: the merge sort).
+struct SignXor {
+    uint32_t neg, pos;
+};
+__host__ __device__ __forceinline__ uint32_t sign_xor(uint32_t k, uint32_t neg, uint32_t pos) {
+    return k ^ ((k & 0x80000000u) ? neg : pos);
+}
+// The (neg, pos) masks of an order; false for an unknown key type.
+inline bool key_order(int key_type, int descending, SignXor *m) {
+    static const SignXor kOrders[3][2] = {
+        {{0x80000000u, 0x80000000u}, {0x7fffffffu, 0x7fffffffu}},   // int32   ascending / descending
+        {{0x00000000u, 0x00000000u}, {0xffffffffu, 0xffffffffu}},   // uint32
+        {{0xffffffffu, 0x80000000u}, {0x00000000u, 0x7fffffffu}},   // float32: IEEE-754 totalOrder on the bits
+    };
+    if (key_type < B200SORT_KEY_I32 || key_type > B200SORT_KEY_F32 || (descending != 0 && descending != 1)) return false;
+    *m = kOrders[key_type][descending];
+    return true;
+}
+// The masks that map an image back to its key.  Each order sends the keys with the top bit set to one half
+// of the images (top bit of the image = 1 ^ top bit of `neg`), so the inverse is keyed on the image's top bit.
+__host__ __device__ __forceinline__ SignXor image_inverse(SignXor m) {
+    return (m.neg & 0x80000000u) ? SignXor{m.pos, m.neg} : SignXor{m.neg, m.pos};
+}
+// The key whose image is 0xFFFFFFFF: last in every order, digit 255 in every pass (the radix tiles' padding).
+__host__ __device__ __forceinline__ uint32_t key_of_last_image(SignXor m) {
+    const SignXor inv = image_inverse(m);
+    return sign_xor(0xFFFFFFFFu, inv.neg, inv.pos);
+}
+
 __device__ __forceinline__ uint32_t lane_id() {
     uint32_t l;
     asm volatile("mov.u32 %0, %%laneid;" : "=r"(l));

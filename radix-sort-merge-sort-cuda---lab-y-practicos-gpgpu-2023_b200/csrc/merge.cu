@@ -147,9 +147,9 @@ __device__ __forceinline__ void warp_bitonic_merge_rounds(int32_t (&key)[K], uin
 // global merge pass less).  Full, 32-byte-aligned tiles are loaded and stored with 256-bit accesses
 // straight from / to the 16 consecutive keys a thread owns.
 // WARPNET: the rounds 16 -> 512 run as a bitonic network over the warp's registers.
-template <int THREADS, int WARPNET>
-__global__ void __launch_bounds__(THREADS)
-block_sort_kernel(const int32_t *in, int32_t *out, size_t n)
+// KEYS (block_sort_keys_kernel): every key is loaded as sign_xor(k, ld) and stored as sign_xor(k, st).
+template <int THREADS, int WARPNET, int KEYS>
+__device__ __forceinline__ void block_sort_body(const int32_t *in, int32_t *out, size_t n, SignXor ld, SignXor st)
 {
     constexpr int kTile = THREADS * kSortK;
     constexpr int kWords = (kTile + kSortK + 1) + ((kTile + kSortK + 1) >> 5) + 1;
@@ -165,13 +165,19 @@ block_sort_kernel(const int32_t *in, int32_t *out, size_t n)
         const int32_t *src = in + tile_base + (size_t)tid * kSortK;
 #pragma unroll
         for (int q = 0; q < kSortK / 8; ++q) ld_stream_v8(src + 8 * q, key + 8 * q);
+        if (KEYS) {
+#pragma unroll
+            for (int k = 0; k < kSortK; ++k) key[k] = (int32_t)sign_xor((uint32_t)key[k], ld.neg, ld.pos);
+        }
         if (tid == 0) s[pad(kTile)] = 0x7FFFFFFF;
     } else {
         // coalesced load; the tail is padded with INT_MAX, which sorts last
 #pragma unroll
         for (int j = 0; j < kSortK; ++j) {
             const uint32_t i = j * THREADS + tid;
-            s[pad(i)] = (i < valid) ? ld_stream(in + tile_base + i) : 0x7FFFFFFF;
+            s[pad(i)] = (i < valid) ? (KEYS ? (int32_t)sign_xor((uint32_t)ld_stream(in + tile_base + i), ld.neg, ld.pos)
+                                            : ld_stream(in + tile_base + i))
+                                    : 0x7FFFFFFF;
         }
         if (tid == 0) s[pad(kTile)] = 0x7FFFFFFF;
         __syncthreads();
@@ -196,6 +202,10 @@ block_sort_kernel(const int32_t *in, int32_t *out, size_t n)
         __syncthreads();
     }
 
+    if (KEYS) {
+#pragma unroll
+        for (int k = 0; k < kSortK; ++k) key[k] = (int32_t)sign_xor((uint32_t)key[k], st.neg, st.pos);
+    }
     if (direct) {
         int32_t *dst = out + tile_base + (size_t)tid * kSortK;
 #pragma unroll
@@ -210,6 +220,19 @@ block_sort_kernel(const int32_t *in, int32_t *out, size_t n)
         const uint32_t i = j * THREADS + tid;
         if (i < valid) st_stream(out + tile_base + i, s[pad(i)]);
     }
+}
+
+template <int THREADS, int WARPNET>
+__global__ void __launch_bounds__(THREADS)
+block_sort_kernel(const int32_t *in, int32_t *out, size_t n)
+{
+    block_sort_body<THREADS, WARPNET, 0>(in, out, n, SignXor{0, 0}, SignXor{0, 0});
+}
+template <int THREADS, int WARPNET>
+__global__ void __launch_bounds__(THREADS)
+block_sort_keys_kernel(const int32_t *in, int32_t *out, size_t n, SignXor ld, SignXor st)
+{
+    block_sort_body<THREADS, WARPNET, 1>(in, out, n, ld, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -348,9 +371,11 @@ __device__ __forceinline__ MergeTileGeom merge_tile_geom(const int32_t *in, size
     return g;
 }
 
-__global__ void __launch_bounds__(kSortThreads, 4)
-merge_pass_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
-                  const uint32_t *__restrict__ splits, size_t t_begin, size_t tiles /* = end of the range */)
+// KEYS (merge_pass_keys_kernel): every key is stored as sign_xor(k, st).
+template <int KEYS>
+__device__ __forceinline__ void
+merge_pass_body(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
+                const uint32_t *__restrict__ splits, size_t t_begin, size_t tiles, SignXor st)
 {
     __shared__ int32_t s[kSortSmemWords];
     const uint32_t tid = threadIdx.x;
@@ -404,12 +429,25 @@ merge_pass_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, siz
 #pragma unroll
         for (int j = 0; j < kSortK; ++j) {
             const uint32_t i = j * kSortThreads + tid;
-            if (i < total) st_stream(out + g0 + i, s[pad(i)]);
+            if (i < total) st_stream(out + g0 + i, KEYS ? (int32_t)sign_xor((uint32_t)s[pad(i)], st.neg, st.pos) : s[pad(i)]);
         }
         if (!more) break;
         t = t_next;
         __syncthreads();                                   // the staging area is reused
     }
+}
+
+__global__ void __launch_bounds__(kSortThreads, 4)
+merge_pass_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
+                  const uint32_t *__restrict__ splits, size_t t_begin, size_t tiles /* = end of the range */)
+{
+    merge_pass_body<0>(in, out, n, run, splits, t_begin, tiles, SignXor{0, 0});
+}
+__global__ void __launch_bounds__(kSortThreads, 4)
+merge_pass_keys_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
+                       const uint32_t *__restrict__ splits, size_t t_begin, size_t tiles, SignXor st)
+{
+    merge_pass_body<1>(in, out, n, run, splits, t_begin, tiles, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -490,11 +528,11 @@ __device__ __forceinline__ MergeTileGeom32 merge_tile_geom32(const int32_t *in, 
 }
 
 // MINB: CTAs per SM the register allocation is held to (4: 64 registers, 5: 48, 6: 40).
-template <int MINB>
-__global__ void __launch_bounds__(kSortThreads, MINB)
-merge_pass2_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
-                   int pair_shift, const uint32_t *__restrict__ splits, size_t t_begin,
-                   size_t tiles /* = end of the range */)
+// KEYS (merge_pass2_keys_kernel): every key is stored as sign_xor(k, st).
+template <int KEYS>
+__device__ __forceinline__ void
+merge_pass2_body(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run, int pair_shift,
+                 const uint32_t *__restrict__ splits, size_t t_begin, size_t tiles, SignXor st)
 {
     __shared__ int32_t s2[2][kPass2Words];
     const uint32_t tid = threadIdx.x;
@@ -554,6 +592,10 @@ merge_pass2_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, si
         const uint32_t ai = merge_path_gap(s, na, na + kGap, nb, diag);
         int32_t key[kSortK];
         serial_merge_sentinel<kSortK>(s, ai, na + kGap + (diag - ai), key);
+        if (KEYS) {
+#pragma unroll
+            for (int k = 0; k < kSortK; ++k) key[k] = (int32_t)sign_xor((uint32_t)key[k], st.neg, st.pos);
+        }
         int32_t *dst = out + g0 + first;
         if (total == (uint32_t)kSortTile && out_aligned) {
 #pragma unroll
@@ -567,6 +609,22 @@ merge_pass2_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, si
         t = t_next;
         buf ^= 1;
     }
+}
+
+template <int MINB>
+__global__ void __launch_bounds__(kSortThreads, MINB)
+merge_pass2_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
+                   int pair_shift, const uint32_t *__restrict__ splits, size_t t_begin,
+                   size_t tiles /* = end of the range */)
+{
+    merge_pass2_body<0>(in, out, n, run, pair_shift, splits, t_begin, tiles, SignXor{0, 0});
+}
+template <int MINB>
+__global__ void __launch_bounds__(kSortThreads, MINB)
+merge_pass2_keys_kernel(const int32_t *__restrict__ in, int32_t *__restrict__ out, size_t n, size_t run,
+                        int pair_shift, const uint32_t *__restrict__ splits, size_t t_begin, size_t tiles, SignXor st)
+{
+    merge_pass2_body<1>(in, out, n, run, pair_shift, splits, t_begin, tiles, st);
 }
 
 // ================================================================================================
@@ -640,7 +698,7 @@ int merge_partition(const int32_t *d_in, size_t n, size_t run, uint32_t *d_split
 }
 
 int merge_pass_range(const int32_t *d_in, int32_t *d_out, size_t n, size_t run, const uint32_t *d_splits,
-                     size_t tile_begin, size_t tile_end, cudaStream_t s) {
+                     size_t tile_begin, size_t tile_end, cudaStream_t s, const SignXor *st) {
     if (n == 0) return B200SORT_OK;
     if (run == 0 || run % kSortTile != 0) return B200SORT_ERR_INVALID;
     const size_t tiles = div_up(n, kSortTile);
@@ -655,6 +713,10 @@ int merge_pass_range(const int32_t *d_in, int32_t *d_out, size_t n, size_t run, 
     {
         int pair_shift = -1;                                   // 2 * run a power of two: shifts instead of divisions
         if ((run & (run - 1)) == 0) { pair_shift = 1; while (((size_t)1 << pair_shift) < 2 * run) ++pair_shift; }
+        if (st != nullptr)
+            merge_pass2_keys_kernel<4><<<grid, kSortThreads, 0, s>>>(d_in, d_out, n, run, pair_shift, d_splits, tile_begin,
+                                                                    tile_end, *st);
+        else
 #ifdef B200SORT_EXPERIMENTS
         if (per_sm == 5)      merge_pass2_kernel<5><<<grid, kSortThreads, 0, s>>>(d_in, d_out, n, run, pair_shift, d_splits, tile_begin, tile_end);
         else if (per_sm == 6) merge_pass2_kernel<6><<<grid, kSortThreads, 0, s>>>(d_in, d_out, n, run, pair_shift, d_splits, tile_begin, tile_end);
@@ -662,6 +724,8 @@ int merge_pass_range(const int32_t *d_in, int32_t *d_out, size_t n, size_t run, 
 #endif
         merge_pass2_kernel<4><<<grid, kSortThreads, 0, s>>>(d_in, d_out, n, run, pair_shift, d_splits, tile_begin, tile_end);
     }
+    else if (st != nullptr)
+        merge_pass_keys_kernel<<<grid, kSortThreads, 0, s>>>(d_in, d_out, n, run, d_splits, tile_begin, tile_end, *st);
     else
         merge_pass_kernel<<<grid, kSortThreads, 0, s>>>(d_in, d_out, n, run, d_splits, tile_begin, tile_end);
     B200_LAUNCH_CHECK();
@@ -673,8 +737,9 @@ int merge_pass(const int32_t *d_in, int32_t *d_out, size_t n, size_t run, const 
     return merge_pass_range(d_in, d_out, n, run, d_splits, 0, div_up(n, kSortTile), s);
 }
 
-int merge_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
-               size_t ws_bytes, cudaStream_t s, float *ms, bool lab_stages) {
+namespace {
+int merge_sort_impl(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
+                    size_t ws_bytes, cudaStream_t s, float *ms, bool lab_stages, const SignXor *order) {
     if (ms) ms[0] = ms[1] = ms[2] = 0.f;
     if (n == 0) return B200SORT_OK;
     if (n == 1) {
@@ -699,11 +764,27 @@ int merge_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, vo
         for (auto &e : ev) B200_CUDA_TRY(cudaEventCreate(&e));
         B200_CUDA_TRY(cudaEventRecord(ev[0], s));
     }
-    B200_TRY(merge_block_sort(d_in, src, n, s, lab_stages));
+    // order: the block sort maps every key to image ^ 0x80000000 (a signed-comparable int32), the passes sort those
+    // with the int32 kernels, and the last kernel maps them back: d_tmp and d_out are scratch until then
+    SignXor to_signed{}, to_key{}, identity{0u, 0u};
+    if (order != nullptr) {
+        const SignXor inv = image_inverse(*order);
+        to_signed = SignXor{order->neg ^ 0x80000000u, order->pos ^ 0x80000000u};
+        to_key = SignXor{inv.pos ^ 0x80000000u, inv.neg ^ 0x80000000u};     // keyed on the image's top bit = !(sign)
+    }
+    if (order != nullptr) {
+        block_sort_keys_kernel<2 * kSortThreads, 1><<<(unsigned)div_up(n, 2 * kSortTile), 2 * kSortThreads, 0, s>>>(
+            d_in, src, n, to_signed, passes == 0 ? to_key : identity);
+        B200_LAUNCH_CHECK();
+    } else {
+        B200_TRY(merge_block_sort(d_in, src, n, s, lab_stages));
+    }
     if (ms) B200_CUDA_TRY(cudaEventRecord(ev[1], s));
-    for (size_t run = first_run; run < n; run *= 2) {
+    int pass = 0;
+    for (size_t run = first_run; run < n; run *= 2, ++pass) {
         B200_TRY(merge_partition(src, n, run, splits, s));
-        B200_TRY(merge_pass(src, dst, n, run, splits, s));
+        B200_TRY(merge_pass_range(src, dst, n, run, splits, 0, div_up(n, kSortTile), s,
+                                  (order != nullptr && pass == passes - 1) ? &to_key : nullptr));
         int32_t *t = src; src = dst; dst = t;
     }
     if (ms) {
@@ -714,6 +795,19 @@ int merge_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, vo
         ms[2] = (float)passes;
     }
     return B200SORT_OK;
+}
+}  // namespace
+
+int merge_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
+               size_t ws_bytes, cudaStream_t s, float *ms, bool lab_stages) {
+    return merge_sort_impl(d_in, d_out, d_tmp, n, d_ws, ws_bytes, s, ms, lab_stages, nullptr);
+}
+
+int merge_sort_keys(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
+                    size_t ws_bytes, cudaStream_t s, SignXor order) {
+    // the generic kernels exist for the shipped shapes only (8192-key block sort, variants 0 and 1)
+    if (n > 1 && g_merge_variant.load() > 1) return B200SORT_ERR_INVALID;
+    return merge_sort_impl(d_in, d_out, d_tmp, n, d_ws, ws_bytes, s, nullptr, false, &order);
 }
 
 }  // namespace b200sort

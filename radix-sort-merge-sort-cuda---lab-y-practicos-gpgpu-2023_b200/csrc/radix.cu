@@ -21,7 +21,9 @@
 //   k0  radix_small_kernel (radix_small.cuh)  n <= 8192: all four passes in one CTA, one launch
 // This file is the host side: the shape table, workspace layout, launches.
 //
-// Signed order: digits are taken from key ^ 0x80000000 (only the top digit changes).
+// Signed order: digits are taken from key ^ 0x80000000 (only the top digit changes).  Any other key order
+// (b200sort_sort_keys): digits of the key's image k ^ (k < 0 ? key_neg : key_pos), by a second, generic instantiation
+// of the histogram, the small-array kernel and the shipped pass kernels (DESIGN section 4.2c).
 // Stability of every pass is what makes LSD correct: inside a tile the order is (warp, item,
 // lane) and keys are loaded warp-striped so that this is memory order.
 #include "radix.cuh"
@@ -59,6 +61,7 @@ struct Variant {
     size_t smem;
     OnesweepFn fn;
     OnesweepFn fn_devn = nullptr;   // the same shape reading the key count from the control block (radix_sort_devn)
+    OnesweepFn fn_key = nullptr;    // the same shape for any key order (RadixControl::key_*; b200sort_sort_keys)
 };
 
 #define B200_VARIANT(W, I, B, M, C)                                                                 \
@@ -96,7 +99,8 @@ struct Variant {
 const Variant kVariants[] = {
     // ---- the shipped shapes ------------------------------------------------------------------------------------
     { "tma3_16w_2x16_kRankAdd_tmem_keys_bulk_store_a_counts_b_resolves", kRankAdd, 0, 1, kT2Threads, kT2Tile, kT3SmemBytes,
-      radix_onesweep_tma3_kernel<0, 0, 0, 1>, radix_onesweep_tma3_kernel<0, 1, 0, 1> },   //  0: DEFAULT: persistent CTAs,
+      radix_onesweep_tma3_kernel<0, 0, 0, 1>, radix_onesweep_tma3_kernel<0, 1, 0, 1>,
+      radix_onesweep_tma3_kernel<0, 0, 0, 1, 1> },   //  0: DEFAULT: persistent CTAs,
                                                //     16384-key tiles, keys parked in tensor memory, positions from a second
                                                //     shared atomic, write-out by TMA bulk copies, one half of the CTA counts
                                                //     and publishes while the other writes out and resolves, the next tiles
@@ -104,15 +108,18 @@ const Variant kVariants[] = {
                                                //     (radix_sort_impl) arrays below 2^23 keys run shape 1.
     { "pipelined2_16w_ipt20_kRankAdd_pack1_late_ticket", kRankAdd, 0, 1, 512, Pipelined2Shape<20, 1>::kTile,
       Pipelined2Shape<20, 1>::kSmemBytes, radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1>,
-      radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 0, 0, 1> },   //  1: the ALTERNATE: 10240-key tiles,
+      radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 0, 0, 1>,
+      radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 0, 0, 0, 1> },   //  1: the ALTERNATE: 10240-key tiles,
                                                //     delayed two-level look-back, 16-bit counters (two warps per row),
                                                //     ticket drawn after the look-back, write-out by the load/store pipe
     { "pipelined2_16w_ipt20_kRankBallot_pack1_late_ticket", kRankBallot, 0, 1, 512, Pipelined2Shape<20, 1>::kTile,
       Pipelined2Shape<20, 1>::kSmemBytes, radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 1>,
-      radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 1, 0, 1> },   //  2: the documented-
+      radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 1, 0, 1>,
+      radix_onesweep_pipelined2_kernel<20, 0, 0, 1, 2, 0, 0, 1, 1, 0, 0, 1> },   //  2: the documented-
                                                //     behaviour fallback: shape 1 ranked by ballots
     { "tma3_16w_2x16_kRankAdd_tmem_keys_bulk_store_a_counts_b_resolves_any_size", kRankAdd, 0, 1, kT2Threads, kT2Tile,
-      kT3SmemBytes, radix_onesweep_tma3_kernel<0, 0, 0, 1>, radix_onesweep_tma3_kernel<0, 1, 0, 1> },   //  3: shape 0
+      kT3SmemBytes, radix_onesweep_tma3_kernel<0, 0, 0, 1>, radix_onesweep_tma3_kernel<0, 1, 0, 1>,
+      radix_onesweep_tma3_kernel<0, 0, 0, 1, 1> },   //  3: shape 0
                                                //     whatever the size
 #ifdef B200SORT_EXPERIMENTS
     // ---- every other shape measured in rounds 1-2 (profiles/r0*_onesweep_variants.md): make EXPERIMENTS=1 ----------
@@ -268,13 +275,14 @@ const bool g_small_env_on = [] { const char *e = getenv("B200SORT_RADIX_SMALL");
 std::atomic<int> g_small_enabled{g_small_env_on ? 1 : 0};
 // Function attributes are per device, so they are set before every launch instead of once per process
 // (the call costs well under a microsecond).
-int ensure_smem_attr(int v) {
-    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kVariants[v].fn),
+int ensure_smem_attr(int v, bool keys = false) {
+    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(keys ? kVariants[v].fn_key : kVariants[v].fn),
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVariants[v].smem));
     return B200SORT_OK;
 }
-int ensure_hist_attr() {
-    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_histogram_kernel),
+int ensure_hist_attr(bool keys = false) {
+    B200_CUDA_TRY(cudaFuncSetAttribute(keys ? reinterpret_cast<const void *>(radix_histogram_keys_kernel)
+                                            : reinterpret_cast<const void *>(radix_histogram_kernel),
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kHistSmemBytes));
     return B200SORT_OK;
 }
@@ -286,12 +294,14 @@ size_t status_rows(const Variant &var, size_t tiles) {
 
 int launch_onesweep(const Variant &var, size_t tiles, cudaStream_t s, const int32_t *in, int32_t *out,
                     int32_t *tmp, size_t n, int pass, RadixControl *ctl, uint32_t *cur, uint32_t *next,
-                    int follow_plan, bool devn = false) {
+                    int follow_plan, bool devn = false, bool keys = false) {
     if (devn && (var.fn_devn == nullptr || var.cluster != 0)) return B200SORT_ERR_INVALID;
+    if (keys && (var.fn_key == nullptr || var.cluster != 0)) return B200SORT_ERR_INVALID;
     if (var.cluster <= 0) {          // persistent: one CTA per resident slot, tiles by ticket
         const unsigned slots = (var.cluster == 0 ? 2u : (unsigned)(-var.cluster)) * kNumSMs;
         const unsigned grid = (unsigned)(tiles < slots ? tiles : slots);
-        (devn ? var.fn_devn : var.fn)<<<grid, var.threads, var.smem, s>>>(in, out, tmp, n, pass, ctl, cur, next, follow_plan);
+        (devn ? var.fn_devn : keys ? var.fn_key : var.fn)<<<grid, var.threads, var.smem, s>>>(in, out, tmp, n, pass, ctl, cur,
+                                                                                            next, follow_plan);
         B200_LAUNCH_CHECK();
         return B200SORT_OK;
     }
@@ -431,9 +441,10 @@ struct StepTimer {
 
 int radix_sort_impl(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
                     size_t ws_bytes, cudaStream_t s, float *ms, const uint32_t *d_n = nullptr,
-                    const uint32_t *d_hist = nullptr) {
+                    const uint32_t *d_hist = nullptr, const SignXor *order = nullptr) {
     // d_n != nullptr: n is an upper bound (grids, status rows), the kernels read the key count from *d_n;
-    // d_hist != nullptr (with d_n): the four digit histograms exist already, the histogram kernel is not run
+    // d_hist != nullptr (with d_n): the four digit histograms exist already, the histogram kernel is not run;
+    // order != nullptr (not with d_n): any key order, by the generic instantiations
     if (ms) for (int i = 0; i < 6; ++i) ms[i] = 0.f;
     if (n == 0) return B200SORT_OK;
     if (n == 1 && d_n == nullptr) {
@@ -447,20 +458,28 @@ int radix_sort_impl(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t 
     // k0: up to 8192 keys are sorted by one CTA in one launch (untimed calls only: the timed form reports
     // the pipeline's kernels).  Same lane-ordered atomic rank as the pass kernel, same gate.
     if (ms == nullptr && d_n == nullptr && n <= (size_t)kSmallTile && g_small_enabled.load() && atomic_order_ok()) {
-        B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_small_kernel),
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallSmemBytes));
-        radix_small_kernel<<<1, kSmallThreads, kSmallSmemBytes, s>>>(d_in, d_out, (uint32_t)n);
+        if (order != nullptr) {
+            B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_small_keys_kernel),
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallSmemBytes));
+            radix_small_keys_kernel<<<1, kSmallThreads, kSmallSmemBytes, s>>>(d_in, d_out, (uint32_t)n, *order);
+        } else {
+            B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_small_kernel),
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallSmemBytes));
+            radix_small_kernel<<<1, kSmallThreads, kSmallSmemBytes, s>>>(d_in, d_out, (uint32_t)n);
+        }
         B200_LAUNCH_CHECK();
         return B200SORT_OK;
     }
     int v = effective_variant();
     if (d_n != nullptr && kVariants[v].fn_devn == nullptr) v = atomic_order_ok() ? 0 : kFallbackVariant;
     if (v == 0 && n < kDefaultMinKeys) v = kSmallTileVariant;
-    B200_TRY(ensure_smem_attr(v));
+    const bool keys = order != nullptr;
+    if (keys && (d_n != nullptr || kVariants[v].fn_key == nullptr)) return B200SORT_ERR_INVALID;   // an experiment shape
+    B200_TRY(ensure_smem_attr(v, keys));
     if (d_n != nullptr)
         B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(kVariants[v].fn_devn),
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVariants[v].smem));
-    B200_TRY(ensure_hist_attr());
+    B200_TRY(ensure_hist_attr(keys));
     const Variant &var = kVariants[v];
     auto *ctl = static_cast<RadixControl *>(d_ws);
     const size_t tiles = div_up(n, (size_t)var.tile);
@@ -477,6 +496,10 @@ int radix_sort_impl(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t 
     if (d_hist != nullptr) {
         B200_CUDA_TRY(cudaMemsetAsync(status[0], 0, rows * kRadixBins * sizeof(uint32_t), s));
         radix_plan_kernel<<<1, kHistThreads, 0, s>>>(d_hist, d_n, ctl, (uint32_t)skip, in_place);
+    } else if (keys) {
+        radix_histogram_keys_kernel<<<hist_grid(n), kHistThreads, kHistSmemBytes, s>>>(d_in, n, ctl, status[0],
+                                                                                       rows * kRadixBins, (uint32_t)skip,
+                                                                                       in_place, *order);
     } else {
         radix_histogram_kernel<<<hist_grid(n), kHistThreads, kHistSmemBytes, s>>>(d_in, n, ctl, status[0], rows * kRadixBins,
                                                                      (uint32_t)skip, in_place, d_n);
@@ -486,7 +509,7 @@ int radix_sort_impl(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t 
     for (int pass = 0; pass < kRadixPasses; ++pass) {
         uint32_t *cur = status[pass & 1];
         uint32_t *next = (pass + 1 < kRadixPasses) ? status[(pass + 1) & 1] : nullptr;
-        B200_TRY(launch_onesweep(var, tiles, s, d_in, d_out, d_tmp, n, pass, ctl, cur, next, 1, d_n != nullptr));
+        B200_TRY(launch_onesweep(var, tiles, s, d_in, d_out, d_tmp, n, pass, ctl, cur, next, 1, d_n != nullptr, keys));
         B200_TRY(timer.mark());
     }
     if (skip) {
@@ -504,8 +527,8 @@ int radix_sort_impl(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t 
 }  // namespace
 
 int radix_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
-               size_t ws_bytes, cudaStream_t s) {
-    return radix_sort_impl(d_in, d_out, d_tmp, n, d_ws, ws_bytes, s, nullptr);
+               size_t ws_bytes, cudaStream_t s, const SignXor *order) {
+    return radix_sort_impl(d_in, d_out, d_tmp, n, d_ws, ws_bytes, s, nullptr, nullptr, nullptr, order);
 }
 
 int radix_sort_devn(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n_max, const uint32_t *d_n,
@@ -521,11 +544,11 @@ int radix_sort_devn(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t 
 // pass is (that is what makes LSD correct in the first place): equal keys keep their input order,
 // the A-before-B rule of SRM/lab.cu:163-170 carried through the whole sort.
 // Pairs per thread: 10 (default) or 12 (B200SORT_PAIRS_IPT=12, for A/B).
-template <int IPT, int SAFE>
+template <int IPT, int SAFE, int KEYS = 0>
 int launch_pairs_passes(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const int32_t *v_in, int32_t *v_out,
                         int32_t *v_tmp, size_t n, RadixControl *ctl, uint32_t *const *status, cudaStream_t s) {
     constexpr size_t smem = Pipelined2Shape<IPT, 1, 1>::kSmemBytes;
-    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_onesweep_pairs_kernel<IPT, SAFE>),
+    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_onesweep_pairs_kernel<IPT, SAFE, KEYS>),
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const size_t tiles = div_up(n, (size_t)Pipelined2Shape<IPT, 1, 1>::kTile);
     const unsigned slots = 2u * kNumSMs;
@@ -533,8 +556,8 @@ int launch_pairs_passes(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, con
     for (int pass = 0; pass < kRadixPasses; ++pass) {
         uint32_t *cur = status[pass & 1];
         uint32_t *next = (pass + 1 < kRadixPasses) ? status[(pass + 1) & 1] : nullptr;
-        radix_onesweep_pairs_kernel<IPT, SAFE><<<grid, 512, smem, s>>>(d_in, d_out, d_tmp, n, pass, ctl, cur, next, 1,
-                                                                v_in, v_out, v_tmp);
+        radix_onesweep_pairs_kernel<IPT, SAFE, KEYS><<<grid, 512, smem, s>>>(d_in, d_out, d_tmp, n, pass, ctl, cur, next, 1,
+                                                                      v_in, v_out, v_tmp);
         B200_LAUNCH_CHECK();
     }
     return B200SORT_OK;
@@ -550,7 +573,7 @@ int pairs_ipt() {
 size_t radix_pairs_tile() { return 512u * (size_t)(atomic_order_ok() ? pairs_ipt() : 10); }
 
 int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const int32_t *v_in, int32_t *v_out,
-                     int32_t *v_tmp, size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s) {
+                     int32_t *v_tmp, size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s, const SignXor *order) {
     if (n == 0) return B200SORT_OK;
     if (n == 1) {
         if (d_in != d_out) B200_CUDA_TRY(cudaMemcpyAsync(d_out, d_in, sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
@@ -561,7 +584,9 @@ int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const 
     B200_TRY(check_ws(d_ws, ws_bytes, n));
     if (n >= ((size_t)1 << 30) && !g_skip_enabled.load()) return B200SORT_ERR_INVALID;   // see radix_sort_impl
     const bool safe = !atomic_order_ok();                                  // then the ballot-ranked shape runs
-    B200_TRY(ensure_hist_attr());
+    const bool keys = order != nullptr;
+    if (keys && !safe && pairs_ipt() != 10) return B200SORT_ERR_INVALID;   // the generic pairs kernel has 5120-key tiles
+    B200_TRY(ensure_hist_attr(keys));
     auto *ctl = static_cast<RadixControl *>(d_ws);
     const size_t tiles = div_up(n, radix_pairs_tile());
     const size_t rows = tiles + div_up(tiles, (size_t)kLookGroup);
@@ -572,10 +597,17 @@ int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const 
     const uint32_t in_place = (d_in == d_out) ? 1u : 0u;
 
     B200_CUDA_TRY(cudaMemsetAsync(ctl, 0, kRadixZeroBytes, s));
-    radix_histogram_kernel<<<hist_grid(n), kHistThreads, kHistSmemBytes, s>>>(d_in, n, ctl, status[0], rows * kRadixBins,
-                                                                 (uint32_t)skip, in_place);
+    if (keys)
+        radix_histogram_keys_kernel<<<hist_grid(n), kHistThreads, kHistSmemBytes, s>>>(d_in, n, ctl, status[0],
+                                                                                       rows * kRadixBins, (uint32_t)skip,
+                                                                                       in_place, *order);
+    else
+        radix_histogram_kernel<<<hist_grid(n), kHistThreads, kHistSmemBytes, s>>>(d_in, n, ctl, status[0], rows * kRadixBins,
+                                                                     (uint32_t)skip, in_place);
     B200_LAUNCH_CHECK();
-    if (safe)                   B200_TRY((launch_pairs_passes<10, 1>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, ctl, status, s)));
+    if (keys && safe)           B200_TRY((launch_pairs_passes<10, 1, 1>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, ctl, status, s)));
+    else if (keys)              B200_TRY((launch_pairs_passes<10, 0, 1>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, ctl, status, s)));
+    else if (safe)              B200_TRY((launch_pairs_passes<10, 1>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, ctl, status, s)));
 #ifdef B200SORT_EXPERIMENTS
     else if (pairs_ipt() == 12) B200_TRY((launch_pairs_passes<12, 0>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, ctl, status, s)));
 #endif

@@ -24,7 +24,10 @@ struct RadixControl {
     uint32_t hot[kRadixPasses];                // 0, or 1 + the most frequent digit value of the pass if it
                                                // holds > 1/8 of the keys
     uint32_t n_dev;                            // number of keys, as the kernels use it (see radix_sort_devn)
-    uint32_t pad1[2];
+    uint32_t key_neg, key_pos;                 // the key order's masks (SignXor), written by the generic histogram
+                                               // kernel and read by the generic pass kernels; unused for int32 ascending
+    uint32_t key_pad;                          // the key whose image is 0xFFFFFFFF: pads the ragged last tile
+    uint32_t pad1[3];
 };
 constexpr uint32_t kSelIn = 1, kSelTmp = 2, kSelOut = 3;
 constexpr size_t kRadixZeroBytes    = offsetof(RadixControl, base);
@@ -41,12 +44,15 @@ int radix_histogram(const int32_t *d_keys, size_t n, uint32_t *d_hist, cudaStrea
 int radix_single_pass(const int32_t *d_in, int32_t *d_out, size_t n, int pass,
                       void *d_ws, size_t ws_bytes, cudaStream_t s);
 // d_in may equal d_out (in-place sort); otherwise d_in is left untouched.
+// order: nullptr = int32 ascending (the kernels specialised for it); else the key order's masks (key_order), served by
+// the generic instantiations.  B200SORT_ERR_INVALID if the selected shape has no generic instantiation.
 int radix_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
-               size_t ws_bytes, cudaStream_t s);
+               size_t ws_bytes, cudaStream_t s, const SignXor *order = nullptr);
 // Sort-by-key: (key, value) pairs ordered by key, stable.  Same workspace as radix_sort.  Either both of
 // d_in == d_out and v_in == v_out (in place) or neither.
 int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const int32_t *v_in, int32_t *v_out,
-                     int32_t *v_tmp, size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s);
+                     int32_t *v_tmp, size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s,
+                     const SignXor *order = nullptr);
 // The same sort with the key count taken from DEVICE memory (*d_n <= n_max, read by the kernels when they run):
 // lets a caller whose n is produced by an earlier kernel (the multi-GPU exchange) enqueue the sort without a
 // host synchronisation.  Grids, workspace and status rows are sized for n_max.

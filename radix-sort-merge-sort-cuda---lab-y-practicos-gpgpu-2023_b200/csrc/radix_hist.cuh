@@ -129,10 +129,12 @@ radix_plan_kernel(const uint32_t *__restrict__ d_hist, const uint32_t *d_n, Radi
     radix_finish_plan(ctl, (size_t)*d_n, skip_enabled, in_place, tid, s_warp_sums, s_skip, s_hot);
 }
 
-__global__ void __launch_bounds__(kHistThreads)
-radix_histogram_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl *ctl,
-                       uint32_t *status_to_zero, size_t status_words, uint32_t skip_enabled,
-                       uint32_t in_place, const uint32_t *d_n = nullptr)
+// KEYS = 1: any key order; the bytes of every key's image k ^ (k < 0 ? order.neg : order.pos) are counted, and the
+// order is left in the control block for the generic pass kernels.  0: int32 ascending.
+template <int KEYS>
+__device__ __forceinline__ void
+radix_histogram_body(const int32_t *__restrict__ keys, size_t n, RadixControl *ctl, uint32_t *status_to_zero,
+                     size_t status_words, uint32_t skip_enabled, uint32_t in_place, const uint32_t *d_n, SignXor order)
 {
     if (d_n != nullptr) n = *d_n;                       // key count produced on the device (<= the n the grid was sized for)
     extern __shared__ __align__(16) uint32_t sh[];
@@ -142,6 +144,13 @@ radix_histogram_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl 
     __shared__ uint32_t s_is_last;
 
     const uint32_t tid = threadIdx.x;
+    if (KEYS && blockIdx.x == 0 && tid == 0) {
+        ctl->key_neg = order.neg;
+        ctl->key_pos = order.pos;
+        ctl->key_pad = key_of_last_image(order);
+    }
+    // hist_flush flips the top byte of what it was given back: hand it image ^ 0x80000000
+    const uint32_t xneg = order.neg ^ 0x80000000u, xpos = order.pos ^ 0x80000000u;
     {
         uint4 *z = reinterpret_cast<uint4 *>(sh);
         for (uint32_t i = tid; i < kHistSmemWords / 4; i += kHistThreads) z[i] = make_uint4(0, 0, 0, 0);
@@ -158,6 +167,7 @@ radix_histogram_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl 
     __syncthreads();
 
     const uint32_t col = smem_u32(sh + (tid & 31));
+    auto add = [&](int32_t k) { hist_add(col, KEYS ? (int32_t)sign_xor((uint32_t)k, xneg, xpos) : k); };
 
     // Scalar head up to 16-byte alignment, 128-bit body, scalar tail.
     size_t head = ((16 - (reinterpret_cast<uintptr_t>(keys) & 15)) & 15) / 4;
@@ -187,15 +197,15 @@ radix_histogram_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl 
 #pragma unroll
         for (int u = 0; u < kHistUnroll; ++u) {
             if (ok[u]) {
-                hist_add(col, r[u].x); hist_add(col, r[u].y);
-                hist_add(col, r[u].z); hist_add(col, r[u].w);
+                add(r[u].x); add(r[u].y);
+                add(r[u].z); add(r[u].w);
             }
         }
         if (++iters == kHistFlushIters) { hist_flush(sh, ctl, tid); iters = 0; }
     }
     if (blockIdx.x == 0) {   // < 8 keys in total: cannot overflow anything
-        for (size_t i = tid; i < head; i += kHistThreads) hist_add(col, keys[i]);
-        for (size_t i = tail_start + tid; i < n; i += kHistThreads) hist_add(col, keys[i]);
+        for (size_t i = tid; i < head; i += kHistThreads) add(keys[i]);
+        for (size_t i = tail_start + tid; i < n; i += kHistThreads) add(keys[i]);
     }
     hist_flush(sh, ctl, tid);
 
@@ -211,5 +221,19 @@ radix_histogram_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl 
     radix_finish_plan(ctl, n, skip_enabled, in_place, tid, s_warp_sums, s_skip, s_hot);
 }
 
+__global__ void __launch_bounds__(kHistThreads)
+radix_histogram_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl *ctl,
+                       uint32_t *status_to_zero, size_t status_words, uint32_t skip_enabled,
+                       uint32_t in_place, const uint32_t *d_n = nullptr)
+{
+    radix_histogram_body<0>(keys, n, ctl, status_to_zero, status_words, skip_enabled, in_place, d_n,
+                            SignXor{0x80000000u, 0x80000000u});
+}
+__global__ void __launch_bounds__(kHistThreads)
+radix_histogram_keys_kernel(const int32_t *__restrict__ keys, size_t n, RadixControl *ctl, uint32_t *status_to_zero,
+                            size_t status_words, uint32_t skip_enabled, uint32_t in_place, SignXor order)
+{
+    radix_histogram_body<1>(keys, n, ctl, status_to_zero, status_words, skip_enabled, in_place, nullptr, order);
+}
 
 }  // namespace b200sort

@@ -378,7 +378,9 @@ struct Pipelined2Shape {
 // DEVN : the key count is read from the control block (written by the histogram kernel from a device pointer,
 //        radix_sort_devn) instead of the kernel argument.  A separate instantiation: as a run-time switch it cost
 //        the default kernel 64 bytes of spills and 4 % (0.696 -> 0.726 ms per pass).
-template <int IPT, int TIMING, int SPLIT, int PACK, int KV, int EG = 0, int OVL = 0, int LATE = 0, int SAFE = 0, int PFW = 0, int DEVN = 0>
+// KEYS = 1: any key order (RadixControl::key_neg / key_pos / key_pad); 0: int32 ascending.
+template <int IPT, int TIMING, int SPLIT, int PACK, int KV, int EG = 0, int OVL = 0, int LATE = 0, int SAFE = 0, int PFW = 0, int DEVN = 0,
+          int KEYS = 0>
 __device__ __forceinline__ void
 radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n,
                                int pass, RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next,
@@ -412,6 +414,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
         const uint32_t n32 = DEVN ? ctl->n_dev : (uint32_t)n;
         s_misc[20] = n32;
         s_misc[21] = (uint32_t)(((size_t)n32 + kTile - 1) / kTile);
+        if (KEYS && SAFE) s_misc[22] = flips_of(ctl->key_neg, ctl->key_pos, pass * kRadixBits);
     }
     __syncthreads();
     auto n_f = [&]() -> size_t { return DEVN ? (size_t)reinterpret_cast<volatile uint32_t *>(s_misc)[20] : n; };
@@ -439,6 +442,13 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
     }
     const int shift = pass * kRadixBits;
     const uint32_t flip = (pass == kRadixPasses - 1) ? 0x80u : 0u;
+    // the ballot-ranked shape (SAFE) already spills for int32: there the order's bytes are re-read from shared memory
+    // (s_misc[22]) at every use instead of taking a register
+    const uint32_t flips = (KEYS && !SAFE) ? flips_of(ctl->key_neg, ctl->key_pos, shift) : 0u;
+    auto dig = [&](int32_t k) -> uint32_t {
+        if (!KEYS) return digit_of(k, shift, flip);
+        return digit_of_image(k, shift, SAFE ? reinterpret_cast<volatile uint32_t *>(s_misc)[22] : flips);
+    };
     const uint32_t lt = lanemask_lt();
     const bool in_a = tid < kRadixBins;                       // warps 0..7 : thread = digit
     const bool in_b = !in_a;                                  // warps 8..15: thread - 256 = digit
@@ -471,7 +481,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
         } else {
 #pragma unroll
             for (int i = 0; i < IPT; ++i)
-                key[i] = (wofs + i * 32 < valid) ? ld_stream(src + i * 32) : 0x7FFFFFFF;
+                key[i] = (wofs + i * 32 < valid) ? ld_stream(src + i * 32) : (KEYS ? (int32_t)ctl->key_pad : 0x7FFFFFFF);
         }
         if (KV) {
             const int32_t *vsrc = vin + tile_base + wofs;
@@ -491,7 +501,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
             for (int j = 0; j < IPT; ++j) {
                 const uint32_t p = tid + j * kThreads;
                 const int32_t k = sk[p];
-                const size_t dst = (size_t)(uint32_t)(go[digit_of(k, shift, flip)] + p);
+                const size_t dst = (size_t)(uint32_t)(go[dig(k)] + p);
                 B200_CHECK_AT(2, dst < n_f());
                 st_stream(out + dst, k);
                 if (KV) st_stream(vout + dst, sv[p]);
@@ -502,7 +512,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
                 const uint32_t p = tid + j * kThreads;
                 if (p < valid) {
                     const int32_t k = sk[p];
-                    const size_t dst = (size_t)(uint32_t)(go[digit_of(k, shift, flip)] + p);
+                    const size_t dst = (size_t)(uint32_t)(go[dig(k)] + p);
                     B200_CHECK_AT(2, dst < n_f());
                     st_stream(out + dst, k);
                     if (KV) st_stream(vout + dst, sv[p]);
@@ -555,7 +565,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
                 if (last_of_group) st_relaxed_gpu(grow, kFlagIncl | ((gprev + inprev + p_total) & kValueMask));
             }
         }
-        // the run lies inside the array (the last tile's count of digit 255 includes its INT_MAX padding slots)
+        // the run lies inside the array (the last tile's count of digit 255 includes its padding slots)
         B200_CHECK_AT(3, (size_t)digit_base + inprev + gprev + (((size_t)pt + 1 == tiles_f()) ? 0u : p_total) <= n_f());
         s_gofs[buf * kRadixBins + bd] = digit_base + inprev + gprev - s_tstart[buf * kRadixBins + bd];
     };
@@ -639,7 +649,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
         // ---- rank: one shared-memory atomicAdd per key (lane-ordered; see the self-test) ----------
         uint32_t rank2[IPT / 2];
         {
-            const uint32_t d0 = digit_of(key[0], shift, flip);
+            const uint32_t d0 = dig(key[0]);
             const uint32_t agree = __ballot_sync(0xffffffffu, d0 == __shfl_sync(0xffffffffu, d0, 0));
             // hot digit of the pass (the histogram kernel found one value holding > 1/8 of the keys), else
             // a locally hot one (a quarter of the warp's first keys agree with lane 0's: sorted input)
@@ -648,7 +658,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
             if (SAFE) {
 #pragma unroll
                 for (int i = 0; i < IPT; ++i) {
-                    const uint32_t d = digit_of(key[i], shift, flip);
+                    const uint32_t d = dig(key[i]);
                     uint32_t peers = 0xffffffffu;                 // lanes of this instruction that hold my digit
 #pragma unroll
                     for (int bit = 0; bit < kRadixBits; ++bit) {
@@ -666,7 +676,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
             } else if (!hot) {
 #pragma unroll
                 for (int i = 0; i < IPT; ++i) {
-                    const uint32_t r = my_half(atomicAdd(wt + digit_of(key[i], shift, flip), 1u << sh));
+                    const uint32_t r = my_half(atomicAdd(wt + dig(key[i]), 1u << sh));
                     rank2[i / 2] = (i & 1) ? (rank2[i / 2] | (r << 16)) : r;
                 }
             } else {
@@ -674,7 +684,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
                 // lane); the others take the atomic as usual
 #pragma unroll
                 for (int i = 0; i < IPT; ++i) {
-                    const uint32_t d = digit_of(key[i], shift, flip);
+                    const uint32_t d = dig(key[i]);
                     const uint32_t hd = hot_word ? hot_word - 1u : __shfl_sync(0xffffffffu, d, 0);
                     const bool same = (d == hd);
                     const uint32_t sm = __ballot_sync(0xffffffffu, same);
@@ -828,7 +838,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
 #pragma unroll
             for (int i = 0; i < IPT; ++i) {
                 const uint32_t r = (i & 1) ? (rank2[i / 2] >> 16) : (rank2[i / 2] & 0xffffu);
-                const uint32_t pos = my_half(wt[digit_of(key[i], shift, flip)]) + r;
+                const uint32_t pos = my_half(wt[dig(key[i])]) + r;
                 B200_CHECK_AT(1, pos < (uint32_t)kTile);
                 sk[pos] = key[i];
                 if (KV) sv[pos] = val[KV ? i : 0];
@@ -890,24 +900,25 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
 }
 
 // MINB: CTAs per SM the register allocation is held to (3 with tiles of <= 6144 keys: 40 registers).
-template <int IPT, int TIMING = 0, int SPLIT = 0, int PACK = 0, int MINB = 2, int EG = 0, int OVL = 0, int LATE = 0, int SAFE = 0, int PFW = 0, int DEVN = 0>
+template <int IPT, int TIMING = 0, int SPLIT = 0, int PACK = 0, int MINB = 2, int EG = 0, int OVL = 0, int LATE = 0, int SAFE = 0, int PFW = 0, int DEVN = 0,
+          int KEYS = 0>
 __global__ void __launch_bounds__(512, MINB)
 radix_onesweep_pipelined2_kernel(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n,
                                  int pass, RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next,
                                  int follow_plan)
 {
-    radix_onesweep_pipelined2_body<IPT, TIMING, SPLIT, PACK, 0, EG, OVL, LATE, SAFE, PFW, DEVN>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur,
+    radix_onesweep_pipelined2_body<IPT, TIMING, SPLIT, PACK, 0, EG, OVL, LATE, SAFE, PFW, DEVN, KEYS>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur,
                                                                 status_next, follow_plan, nullptr, nullptr, nullptr);
 }
 
 // Sort-by-key: the same pass with a 32-bit value riding along with every key.
-template <int IPT, int SAFE = 0>
+template <int IPT, int SAFE = 0, int KEYS = 0>
 __global__ void __launch_bounds__(512, 2)
 radix_onesweep_pairs_kernel(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n,
                             int pass, RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next,
                             int follow_plan, const int32_t *in_vals, int32_t *out_vals, int32_t *tmp_vals)
 {
-    radix_onesweep_pipelined2_body<IPT, 0, 0, 1, 1, 0, 0, 1, SAFE>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur,
+    radix_onesweep_pipelined2_body<IPT, 0, 0, 1, 1, 0, 0, 1, SAFE, 0, 0, KEYS>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur,
                                                     status_next, follow_plan, in_vals, out_vals, tmp_vals);
 }
 

@@ -4,8 +4,9 @@
 // onesweep pipeline is seven launches of mostly launch latency.  Up to 8192 keys fit one CTA's shared
 // memory, so the four 8-bit passes run back to back in one kernel: rank with one shared-memory atomicAdd per
 // key on the warp's counters (the same lane-ordered rank as the pass kernel, same self-test gate), scan,
-// scatter into the other shared-memory buffer, next digit.  Slots past n hold INT_MAX: they are last in
-// tile order and carry the largest digit in every pass, so they stay behind the n real keys.
+// scatter into the other shared-memory buffer, next digit.  Slots past n hold INT_MAX (any other order: the key whose
+// image is 0xFFFFFFFF): they are last in tile order and carry the largest digit in every pass, so they stay behind the
+// n real keys.
 #pragma once
 #include "radix_pipelined.cuh"
 
@@ -17,8 +18,9 @@ constexpr int kSmallIpt = 16;
 constexpr int kSmallTile = kSmallThreads * kSmallIpt;          // 8192
 constexpr size_t kSmallSmemBytes = (size_t)2 * kSmallTile * 4 + (size_t)kSmallWarps * kRadixBins * 4 + 64;
 
-__global__ void __launch_bounds__(kSmallThreads, 1)
-radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
+// KEYS = 1: any key order, `order` = its masks; 0: int32 ascending.
+template <int KEYS>
+__device__ __forceinline__ void radix_small_body(const int32_t *in, int32_t *out, uint32_t n, SignXor order)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     int32_t  *s_buf   = reinterpret_cast<int32_t *>(smem_raw);                       // [2][kSmallTile]
@@ -29,7 +31,8 @@ radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
     uint32_t *wt = s_table + warp * kRadixBins;
     const uint32_t wofs = warp * (32 * kSmallIpt) + lane;
 
-    for (uint32_t i = tid; i < (uint32_t)kSmallTile; i += kSmallThreads) s_buf[i] = (i < n) ? in[i] : 0x7FFFFFFF;
+    const int32_t pad_key = KEYS ? (int32_t)key_of_last_image(order) : 0x7FFFFFFF;
+    for (uint32_t i = tid; i < (uint32_t)kSmallTile; i += kSmallThreads) s_buf[i] = (i < n) ? in[i] : pad_key;
     __syncthreads();
 
     int cur = 0;
@@ -37,6 +40,8 @@ radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
     for (int pass = 0; pass < kRadixPasses; ++pass) {
         const int shift = pass * kRadixBits;
         const uint32_t flip = (pass == kRadixPasses - 1) ? 0x80u : 0u;
+        const uint32_t flips = flips_of(order.neg, order.pos, shift);
+        auto dig = [&](int32_t k) -> uint32_t { return KEYS ? digit_of_image(k, shift, flips) : digit_of(k, shift, flip); };
         const int32_t *src = s_buf + cur * kSmallTile;
         int32_t *dst = s_buf + (cur ^ 1) * kSmallTile;
         for (int j = lane; j < kRadixBins; j += 32) wt[j] = 0;
@@ -46,7 +51,7 @@ radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
 #pragma unroll
         for (int i = 0; i < kSmallIpt; ++i) {
             key[i] = src[wofs + i * 32];                      // warp-striped: tile order = memory order
-            rank[i] = atomicAdd(wt + digit_of(key[i], shift, flip), 1u);
+            rank[i] = atomicAdd(wt + dig(key[i]), 1u);
         }
         __syncthreads();                                      // counts final, src fully read
         if (tid < kRadixBins) {
@@ -75,14 +80,25 @@ radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
         __syncthreads();                                      // positions final
 #pragma unroll
         for (int i = 0; i < kSmallIpt; ++i) {
-            B200_CHECK_AT(8, wt[digit_of(key[i], shift, flip)] + rank[i] < (uint32_t)kSmallTile);
-            dst[wt[digit_of(key[i], shift, flip)] + rank[i]] = key[i];
+            B200_CHECK_AT(8, wt[dig(key[i])] + rank[i] < (uint32_t)kSmallTile);
+            dst[wt[dig(key[i])] + rank[i]] = key[i];
         }
         __syncthreads();                                      // dst complete; the counters may be cleared
         cur ^= 1;
     }
     const int32_t *res = s_buf + cur * kSmallTile;
     for (uint32_t i = tid; i < n; i += kSmallThreads) out[i] = res[i];
+}
+
+__global__ void __launch_bounds__(kSmallThreads, 1)
+radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
+{
+    radix_small_body<0>(in, out, n, SignXor{0x80000000u, 0x80000000u});
+}
+__global__ void __launch_bounds__(kSmallThreads, 1)
+radix_small_keys_kernel(const int32_t *in, int32_t *out, uint32_t n, SignXor order)
+{
+    radix_small_body<1>(in, out, n, order);
 }
 
 }  // namespace b200sort

@@ -72,7 +72,8 @@ __device__ __forceinline__ uint32_t sum_window(const uint32_t (&w)[ROWS], uint32
     return acc;
 }
 
-template <int TIMING, int DEVN = 0, int INSTEP = 0, int ACOUNT = 0>
+// KEYS = 1: any key order (RadixControl::key_neg / key_pos / key_pad); 0: int32 ascending.
+template <int TIMING, int DEVN = 0, int INSTEP = 0, int ACOUNT = 0, int KEYS = 0>
 __device__ __forceinline__ void
 radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n, int pass,
                          RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next, int follow_plan)
@@ -113,6 +114,8 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
     }
     const int shift = pass * kRadixBits;
     const uint32_t flip = (pass == kRadixPasses - 1) ? 0x80u : 0u;
+    const uint32_t flips = KEYS ? flips_of(ctl->key_neg, ctl->key_pos, shift) : 0u;
+    auto dig = [&](int32_t k) -> uint32_t { return KEYS ? digit_of_image(k, shift, flips) : digit_of(k, shift, flip); };
     const uint32_t lt = lanemask_lt();
     const bool in_a = tid < kRadixBins;                          // warps 0..7 : thread = digit
     const uint32_t bd = tid - kRadixBins;                        // warps 8..15: thread - 256 = digit
@@ -163,7 +166,8 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
             for (int i = 0; i < kT2Batch; ++i) k[i] = ld_stream(src + i * 32);
         } else {
 #pragma unroll
-            for (int i = 0; i < kT2Batch; ++i) k[i] = (o + i * 32 < valid) ? ld_stream(src + i * 32) : 0x7FFFFFFF;
+            for (int i = 0; i < kT2Batch; ++i)
+                k[i] = (o + i * 32 < valid) ? ld_stream(src + i * 32) : (KEYS ? (int32_t)ctl->key_pad : 0x7FFFFFFF);
         }
     };
     auto load_batch = [&](uint32_t t, int batch, int32_t (&k)[kT2Batch]) { load_batch_of(t, warp, batch, k); };
@@ -172,7 +176,7 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
     // found one value holding > 1/8 of the keys, or a quarter of the warp's first keys agree with lane 0's) is handled
     // with one ballot and ONE atomic per instruction, so skewed / sorted inputs do not serialise on one address.
     auto sweep = [&](const int32_t (&k)[kT2Batch], uint32_t *wt, bool count_only) {
-        const uint32_t d0 = digit_of(k[0], shift, flip);
+        const uint32_t d0 = dig(k[0]);
         const uint32_t agree = __ballot_sync(0xffffffffu, d0 == __shfl_sync(0xffffffffu, d0, 0));
         const uint32_t hot_word = follow_plan ? ctl->hot[pass] : 0u;
         const bool hot = hot_word != 0 || __popc(agree) >= 8;
@@ -187,7 +191,7 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
             uint32_t pos[kT2Batch];
 #pragma unroll
             for (int i = 0; i < kT2Batch; ++i) {
-                uint32_t d = digit_of(k[i], shift, flip);
+                uint32_t d = dig(k[i]);
                 if (count_only && i >= 2 * kT3Group && i % kT3Group == 0) d += pos[i - kT3Group - 1] >> 31;
                 pos[i] = atomicAdd(wt + d, 1u << sh);
                 if (!count_only && i >= kT3Group && i % kT3Group == kT3Group - 1) {
@@ -210,7 +214,7 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
         } else {
 #pragma unroll
             for (int i = 0; i < kT2Batch; ++i) {
-                const uint32_t d = digit_of(k[i], shift, flip);
+                const uint32_t d = dig(k[i]);
                 const uint32_t hd = hot_word ? hot_word - 1u : __shfl_sync(0xffffffffu, d, 0);
                 const bool same = (d == hd);
                 const uint32_t sm = __ballot_sync(0xffffffffu, same);
@@ -409,8 +413,8 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
                 const uint32_t start = (pw >> 16) + (g & 3u);
 #pragma unroll
                 for (int w = 0; w < kRows; ++w) atomicAdd(&tab_prev[w * kRadixBins + bd], start * 0x10001u);
-                // slots past n (last tile only) carry INT_MAX: digit 255, counted behind every real key; they are
-                // staged but never written
+                // slots past n (last tile only) carry INT_MAX (KEYS: key_pad, whose image is 0xFFFFFFFF): digit 255,
+                // counted behind every real key; they are staged but never written
                 uint32_t cw = p_total;
                 if (last_tile && bd == kRadixBins - 1) cw -= (uint32_t)(tiles_f() * (size_t)kTile - n_f());
                 s_rg[pb * kRadixBins + bd] = make_uint2(start | (cw << 16), g);
@@ -592,12 +596,12 @@ radix_onesweep_tma3_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_b
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "n"(kT2TmemCols) : "memory");
 }
 
-template <int TIMING, int DEVN = 0, int INSTEP = 0, int ACOUNT = 0>
+template <int TIMING, int DEVN = 0, int INSTEP = 0, int ACOUNT = 0, int KEYS = 0>
 __global__ void __launch_bounds__(kT2Threads, 2)
 radix_onesweep_tma3_kernel(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n, int pass,
                            RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next, int follow_plan)
 {
-    radix_onesweep_tma3_body<TIMING, DEVN, INSTEP, ACOUNT>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur, status_next, follow_plan);
+    radix_onesweep_tma3_body<TIMING, DEVN, INSTEP, ACOUNT, KEYS>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur, status_next, follow_plan);
 }
 
 }  // namespace b200sort
