@@ -147,6 +147,39 @@ int    b200sort_radix_pairs_keys(int key_type, int descending, const void *d_key
                                  void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
                                  size_t n, void *d_ws, size_t ws_bytes, void *stream);
 
+/* ---- segmented sort: many independent segments of one array in one call ---------------------------
+ * Segment i is keys[d_offsets[i] .. d_offsets[i+1]), for i < num_segments.  d_offsets is a DEVICE array of
+ * num_segments + 1 int32 with d_offsets[0] = 0, d_offsets[num_segments] = n, non-decreasing; empty segments allowed.
+ * Each segment comes out sorted in the order (key_type, descending) of b200sort_sort_keys; keys never cross segments.
+ * The host never reads d_offsets: a call is stream-ordered, enqueues the same kernels whatever the number of segments
+ * (no host loop over segments, no host synchronisation), and can be captured in a CUDA graph once
+ * b200sort_device_check() has run on the device.  Malformed offsets (decreasing, negative, past n) give an undefined
+ * order but never an access out of bounds: every segment is clamped to [0, n] on the device, and the checked build
+ * counts what the clamps caught at check site 15.
+ * Segments are routed by length to size classes (b200sort_segmented_class_max): copies for length 0-1, a warp per
+ * segment, a CTA per segment sorted in shared memory (two capacities), and above that a segmented onesweep whose tiles
+ * never straddle a segment.  Like the 1-D radix sort, the ranking kernels rely on lane-ordered shared-memory atomics
+ * only after the self-test of b200sort_radix_i32 has passed on the device; otherwise, or with B200SORT_RANK_SAFE=1,
+ * their ballot-ranked forms run.  b200sort_radix_set_variant and b200sort_radix_set_skip select shapes and policies
+ * of the 1-D sort: the segmented sort ignores both.
+ * d_in may equal d_out; otherwise d_in is only read.  d_tmp: n keys of scratch.  Workspace:
+ * b200sort_segmented_workspace_bytes(n, num_segments) bytes, 256-byte aligned, sized from (n, num_segments) alone.
+ * Unknown key_type, descending not 0/1, NULL data pointers, n or num_segments > B200SORT_MAX_N, NULL d_offsets with
+ * num_segments > 0 -> B200SORT_ERR_INVALID; missing, small or misaligned workspace -> B200SORT_ERR_WORKSPACE; all
+ * checked before any device work.  n == 0 returns B200SORT_OK without touching the device. */
+size_t b200sort_segmented_workspace_bytes(size_t n, size_t num_segments);
+int    b200sort_segmented_sort_keys(int key_type, int descending, const void *d_in, void *d_out, void *d_tmp, size_t n,
+                                    const int32_t *d_offsets, size_t num_segments,
+                                    void *d_ws, size_t ws_bytes, void *stream);
+/* Stable within each segment (equal keys keep their input order); in place iff d_keys_in == d_keys_out and
+ * d_vals_in == d_vals_out, a mix of the two -> B200SORT_ERR_INVALID. */
+int    b200sort_segmented_pairs_keys(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                     void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                     size_t n, const int32_t *d_offsets, size_t num_segments,
+                                     void *d_ws, size_t ws_bytes, void *stream);
+/* Largest segment length served by size class c (0, 1, ...); 0 past the last class (the onesweep class, unbounded). */
+size_t b200sort_segmented_class_max(int c);
+
 /* ---- stages, exposed for unit tests and per-kernel timing -------------------------------------- */
 
 /* d_hist[p*256+d] (uint32) = number of keys whose digit p of (key ^ 0x80000000) equals d.

@@ -42,6 +42,18 @@
 
 namespace b200sort {
 
+// k0 (radix_small.cuh): int32 ascending and any other key order
+__global__ void __launch_bounds__(kSmallThreads, 1)
+radix_small_kernel(const int32_t *in, int32_t *out, uint32_t n)
+{
+    radix_small_body<0>(in, out, n, SignXor{0x80000000u, 0x80000000u});
+}
+__global__ void __launch_bounds__(kSmallThreads, 1)
+radix_small_keys_kernel(const int32_t *in, int32_t *out, uint32_t n, SignXor order)
+{
+    radix_small_body<1>(in, out, n, order);
+}
+
 // ================================================================================================
 // host side
 // ================================================================================================

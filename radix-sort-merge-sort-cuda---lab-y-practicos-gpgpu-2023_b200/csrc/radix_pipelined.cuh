@@ -23,9 +23,6 @@ constexpr uint32_t kPPPoison = 0xFFFFFFFFu;
 constexpr int kPPWindow = 8;                         // status rows in flight per chain thread
 enum { kBarW = 1, kBarA = 2, kBarTotals = 3, kBarTstart = 5, kBarGofs = 7 };   // +buffer for the last three
 
-__device__ __forceinline__ void bar_sync(int id, int count) {
-    asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(count) : "memory");
-}
 __device__ __forceinline__ void bar_arrive(int id, int count) {
     asm volatile("bar.arrive %0, %1;" :: "r"(id), "r"(count) : "memory");
 }

@@ -1,6 +1,7 @@
 // radix_tile.cuh -- k2: one onesweep pass, one tile per CTA; shared look-back helpers (included by radix.cu).
 #pragma once
 #include "radix.cuh"
+#include "radix_digit.cuh"
 
 #include <cooperative_groups.h>
 
@@ -11,9 +12,6 @@ namespace b200sort {
 // ================================================================================================
 // k2: one onesweep pass
 // ================================================================================================
-constexpr uint32_t kFlagLocal = 1u << 30;   // this tile's own digit count
-constexpr uint32_t kFlagIncl  = 2u << 30;   // inclusive count over tiles 0..this
-constexpr uint32_t kValueMask = (1u << 30) - 1;
 
 // How a warp finds, for each of its 32 current keys, the lanes holding the same digit:
 //   kRankMatch   __match_any_sync (one MATCH instruction; runs on the ADU pipe)
@@ -34,20 +32,6 @@ struct OnesweepShape {
         + (size_t)kRadixBins * 4 * 4                   // global offset, tile total, tile start, chain prefix
         + 64;                                          // warp sums, tile id
 };
-
-// digit of `key` for the pass with this shift; `flip` is 0x80 for the top digit (signed order)
-__device__ __forceinline__ uint32_t digit_of(int32_t key, int shift, uint32_t flip) {
-    return ((static_cast<uint32_t>(key) >> shift) & (kRadixBins - 1)) ^ flip;
-}
-// The generic pass kernels (KEYS = 1): the digit of the key's image key ^ (key < 0 ? key_neg : key_pos).  `flips`
-// (flips_of) holds this pass's byte of key_pos in byte 0 and of key_neg in byte 1, so the order costs one register,
-// as `flip` does, and two instructions more per digit: the sign as a byte selector, and the byte permute.
-__device__ __forceinline__ uint32_t flips_of(uint32_t key_neg, uint32_t key_pos, int shift) {
-    return ((key_pos >> shift) & (kRadixBins - 1)) | (((key_neg >> shift) & (kRadixBins - 1)) << 8);
-}
-__device__ __forceinline__ uint32_t digit_of_image(int32_t key, int shift, uint32_t flips) {
-    return ((static_cast<uint32_t>(key) >> shift) ^ __byte_perm(flips, 0u, static_cast<uint32_t>(key) >> 31)) & (kRadixBins - 1);
-}
 
 // ---- two-level look-back ---------------------------------------------------------------------------
 // Measured with the phase probe (tools/phase_timing.py): with one level the look-back takes 4.7 us of

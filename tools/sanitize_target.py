@@ -81,6 +81,17 @@ top = (everything.view(np.uint32) ^ np.uint32(0x80000000)) >> np.uint32(32 - bit
 dest = owner[top.astype(np.int64)]
 for r in range(world):
     same(np.sort(bufs[r].cpu().numpy()[:int(recv[r])]), np.sort(everything[dest == r]), f"dist partition: destination {r}")
+# segmented sort: every size class at once (empty, one-key, warp, both CTA capacities, onesweep), keys and pairs
+import key_orders as ko  # noqa: E402
+from test_segmented_gpu import ragged_offsets, seg_keys, seg_pairs, seg_sort_keys, seg_sort_pairs  # noqa: E402
+seg_offs = ragged_offsets(5, total_segments=2000, big=1)
+seg_n = int(seg_offs[-1])
+seg_k = (datagen.uniform_u32(seg_n, 11) % np.uint32(1000)).astype(np.float32)
+same(seg_keys(seg_k, seg_offs, ko.KEY_F32, 1, False), ko.bits(seg_sort_keys(seg_k, seg_offs, ko.KEY_F32, 1)),
+     f"segmented keys n={seg_n}, {seg_offs.size - 1} segments")
+seg_gk, seg_gv = seg_pairs(seg_k, np.arange(seg_n, dtype=np.int32), seg_offs, ko.KEY_F32, 0, True)
+seg_wk, seg_wv = seg_sort_pairs(seg_k, np.arange(seg_n, dtype=np.int32), seg_offs, ko.KEY_F32, 0)
+same(seg_gk, ko.bits(seg_wk), "segmented pairs: keys"); same(seg_gv, seg_wv, "segmented pairs: values (stable)")
 # host operator
 h = datagen.lab_rand(4096, 100, seed=1)
 wh = oracle.order_array(h)
