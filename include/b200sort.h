@@ -25,6 +25,9 @@
  *   b200sort_lab_i32            SRM/lab.cu:303-402 the assignment's staged pipeline kept as a third
  *                               algorithm (warp-tile split -> rank merge -> merge path)
  *   b200sort_dist_*             no reference counterpart (north_star (c)): one-box multi-GPU sort
+ *   b200sort_sort_keys64 / b200sort_radix_pairs_keys64
+ *                               no reference counterpart: int64, uint64 and float64 keys (8 radix passes),
+ *                               keys only or with an int32 value
  *
  * The C++ symbols order_array(int*,int) / order_with_trust(int*,int) that SRM/main.cpp and
  * SRM/performanceTest.cpp link against are exported by the same library (csrc/lab_shim.cu) with
@@ -146,6 +149,43 @@ int    b200sort_sort_keys(int algo, int key_type, int descending, const void *d_
 int    b200sort_radix_pairs_keys(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
                                  void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
                                  size_t n, void *d_ws, size_t ws_bytes, void *stream);
+
+/* ---- 64-bit keys: int64, uint64 and float64 on the radix path -------------------------------------------
+ * Keys are 8-byte words; key_type says how they compare:
+ *   B200SORT_KEY_I64  signed integers, numeric order;
+ *   B200SORT_KEY_U64  unsigned integers, numeric order;
+ *   B200SORT_KEY_F64  IEEE-754 binary64 in totalOrder on the bit pattern, as B200SORT_KEY_F32:
+ *                     -NaN (any payload) < -inf < negatives < -0.0 < +0.0 < positives < +inf < +NaN, NaNs of one
+ *                     sign ordered by payload.  Bits are never changed.  This is NOT the order of torch.sort /
+ *                     np.sort, which treat -0.0 == +0.0 and put every NaN last.
+ * The 32-bit entry points (b200sort_sort_keys, b200sort_radix_pairs_keys, the segmented sort) reject these key types,
+ * and these entry points reject B200SORT_KEY_I32..F32.  descending = 1 is the reverse order; sort-by-key is STABLE in
+ * both directions (without NaN or -0.0 it equals torch.sort(stable=True, descending=...)).  Internally every order is
+ * image(k) = k ^ (bit 63 of k set ? M_neg : M_pos) sorted as uint64: 8 stable passes of 8-bit digits, of which
+ * those where one digit value holds every key are skipped on the device (b200sort_radix_set_skip applies; the
+ * variant switch b200sort_radix_set_variant does not).  DESIGN section 4.2e.
+ * Like the other radix sorts the passes rank with lane-ordered shared-memory atomics only after the self-test of
+ * b200sort_radix_i32 has passed on the device; otherwise, or with B200SORT_RANK_SAFE=1, their ballot-ranked form runs.
+ * A call enqueues one memset and the same ten kernels for every n >= 2 and every distribution, never synchronises and
+ * never reads device results on the host, so it can be captured in a CUDA graph once b200sort_device_check() has run.
+ * Arrays of up to 8192 keys pay that whole sequence too: there is no one-CTA path for 64-bit keys.
+ * d_in may equal d_out (in place); otherwise d_in is only read.  d_tmp: n keys of scratch.  Workspace:
+ * b200sort_keys64_workspace_bytes(n) bytes, 256-byte aligned, sized from n alone.
+ * Key type outside B200SORT_KEY_I64..F64, descending not 0/1, n > B200SORT_MAX_N, NULL data pointers with n > 0, key
+ * pointers not 8-byte aligned -> B200SORT_ERR_INVALID; missing, small or misaligned workspace ->
+ * B200SORT_ERR_WORKSPACE; all checked before any device work.  n == 0, and n == 1 in place, return B200SORT_OK
+ * without touching the device.  With b200sort_radix_set_skip(0), n = 2^30 -> B200SORT_ERR_INVALID. */
+#define B200SORT_KEY_I64            3
+#define B200SORT_KEY_U64            4
+#define B200SORT_KEY_F64            5
+size_t b200sort_keys64_workspace_bytes(size_t n);
+int    b200sort_sort_keys64(int key_type, int descending, const void *d_in, void *d_out, void *d_tmp, size_t n,
+                            void *d_ws, size_t ws_bytes, void *stream);
+/* Stable sort of (64-bit key, int32 value) pairs by key.  In place iff d_keys_in == d_keys_out and
+ * d_vals_in == d_vals_out; a mix of the two -> B200SORT_ERR_INVALID.  Same workspace as b200sort_sort_keys64. */
+int    b200sort_radix_pairs_keys64(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                   void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                   size_t n, void *d_ws, size_t ws_bytes, void *stream);
 
 /* ---- segmented sort: many independent segments of one array in one call ---------------------------
  * Segment i is keys[d_offsets[i] .. d_offsets[i+1]), for i < num_segments.  d_offsets is a DEVICE array of

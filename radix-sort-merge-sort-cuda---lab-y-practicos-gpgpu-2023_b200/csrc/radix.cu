@@ -370,6 +370,7 @@ int radix_set_variant(int v) {
     return B200SORT_OK;
 }
 void radix_set_skip(int enabled) { g_skip_enabled.store(enabled ? 1 : 0); }
+int radix_skip_enabled() { return g_skip_enabled.load(); }
 size_t radix_current_tile() { return (size_t)kVariants[g_variant.load()].tile; }
 const char *radix_effective_variant_name() { return kVariants[effective_variant()].name; }
 

@@ -1,5 +1,6 @@
 // radix_digit.cuh -- what every radix kernel shares about digits and tile-status words: the digit of a key in a
-// pass, the {flag:2, count:30} status words of the decoupled look-back, a named barrier (radix.cu, segmented.cu).
+// pass, the {flag:2, count:30} status words of the decoupled look-back, a named barrier and the 256-digit scan
+// (radix.cu, segmented.cu, radix64.cu).
 #pragma once
 #include "radix.cuh"
 
@@ -25,6 +26,23 @@ __device__ __forceinline__ uint32_t digit_of_image(int32_t key, int shift, uint3
 
 __device__ __forceinline__ void bar_sync(int id, int count) {
     asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(count) : "memory");
+}
+
+// Exclusive scan of one value per thread over threads 0..255 (named barrier 1); `sums` holds 8 words.
+__device__ __forceinline__ uint32_t scan256(uint32_t v, uint32_t *sums) {
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= (uint32_t)o) x += y;
+    }
+    if (lane == 31) sums[warp] = x;
+    bar_sync(1, kRadixBins);
+    uint32_t add = 0;
+#pragma unroll
+    for (int w = 0; w < kRadixBins / 32; ++w) add += (w < (int)warp) ? sums[w] : 0u;
+    return x - v + add;
 }
 
 }  // namespace b200sort

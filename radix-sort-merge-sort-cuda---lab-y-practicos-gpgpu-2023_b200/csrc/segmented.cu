@@ -113,23 +113,6 @@ seg_classify_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t
     }
 }
 
-// Exclusive scan of one value per thread over threads 0..255 (named barrier 1); `sums` holds 8 words.
-__device__ __forceinline__ uint32_t scan256(uint32_t v, uint32_t *sums) {
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= (uint32_t)o) x += y;
-    }
-    if (lane == 31) sums[warp] = x;
-    bar_sync(1, kRadixBins);
-    uint32_t add = 0;
-#pragma unroll
-    for (int w = 0; w < kRadixBins / 32; ++w) add += (w < (int)warp) ? sums[w] : 0u;
-    return x - v + add;
-}
-
 // ---- s1 -------------------------------------------------------------------------------------------------------------
 constexpr int kPlanThreads = 1024;
 __global__ void __launch_bounds__(kPlanThreads)

@@ -92,6 +92,15 @@ same(seg_keys(seg_k, seg_offs, ko.KEY_F32, 1, False), ko.bits(seg_sort_keys(seg_
 seg_gk, seg_gv = seg_pairs(seg_k, np.arange(seg_n, dtype=np.int32), seg_offs, ko.KEY_F32, 0, True)
 seg_wk, seg_wv = seg_sort_pairs(seg_k, np.arange(seg_n, dtype=np.int32), seg_offs, ko.KEY_F32, 0)
 same(seg_gk, ko.bits(seg_wk), "segmented pairs: keys"); same(seg_gv, seg_wv, "segmented pairs: values (stable)")
+# 64-bit keys: keys only and pairs, a ragged last tile, every pass executed and a skipped half
+import key_orders64 as ko64  # noqa: E402
+from test_keys64_gpu import low_entropy, random_keys, sort64_keys, sort64_pairs  # noqa: E402
+k64 = random_keys(n + 123, ko64.KEY_F64, 12)
+same(sort64_keys(k64, ko64.KEY_F64, 1, False), ko64.bits(ko64.sort_keys(k64, ko64.KEY_F64, 1)), "64-bit keys n=2^16+123 float64 desc")
+k64 = low_entropy("below_2_32", n + 45).view(np.int64)
+k64_gk, k64_gv = sort64_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 0, True)
+k64_wk, k64_wv = ko64.sort_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 0)
+same(k64_gk, ko64.bits(k64_wk), "64-bit pairs: keys (4 passes skipped)"); same(k64_gv, k64_wv, "64-bit pairs: values (stable)")
 # host operator
 h = datagen.lab_rand(4096, 100, seed=1)
 wh = oracle.order_array(h)
@@ -109,6 +118,11 @@ if L.b200sort_debug_checked_build():
     for dist_name in ("zipf16", "and3", "edge_mix"):
         k = datagen.make(dist_name, (1 << 23) + 77, 10)
         same(gpu_sort(k, ALGO_RADIX), oracle.radix_sort(k), f"radix default n=2^23+77 {dist_name}")
+    k64 = random_keys((1 << 22) + 77, ko64.KEY_I64, 13)
+    same(sort64_keys(k64, ko64.KEY_I64, 0, True), ko64.bits(ko64.sort_keys(k64, ko64.KEY_I64, 0)), "64-bit keys n=2^22+77 int64")
+    k64_gk, k64_gv = sort64_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 1, False)
+    k64_wk, k64_wv = ko64.sort_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 1)
+    same(k64_gk, ko64.bits(k64_wk), "64-bit pairs n=2^22+77: keys"); same(k64_gv, k64_wv, "64-bit pairs: values")
     sites = (ctypes.c_ulonglong * 16)()
     fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
     print('per check site:', list(sites), flush=True)
