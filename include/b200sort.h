@@ -341,15 +341,18 @@ int b200sort_dist_partition_i32(const int32_t *d_keys, size_t n, int bits, int w
  * (d_all_hist, world x 2^bits uint64 in DEVICE memory) and leaves its result in a device record d_plan
  * (B200SORT_DIST_PLAN_BYTES, 8-byte aligned): recv_count[16], send_count[16], dst_offset[16] (uint64 each), then
  * uint32 m = the number of keys this rank will own, uint32 error = 1 if some rank would receive more than `cap`
- * keys (then the partition kernel writes nothing), 8 bytes of padding, then uint32 top_hist[256] = the histogram
- * of the top byte (of key ^ 0x80000000) of the keys this rank will own, which follows from the bin counts.  Same
- * boundaries as b200sort_dist_plan, bit for bit.
+ * keys (then the partition kernel writes nothing), 8 bytes of padding, then uint32 top_hist[256] = for bits >= 8 the
+ * histogram of the top byte (of key ^ 0x80000000) of the keys this rank will own, which follows from the bin counts;
+ * for bits < 8 all zero, because a bin is then coarser than a byte.  Same boundaries as b200sort_dist_plan, bit for
+ * bit.
  * b200sort_dist_partition_planned_i32 takes its offsets from that record, and b200sort_radix_copy_devn_i32 sorts
  * what arrived with the key count read from device memory (d_n = the record's m; n_max sizes grids and workspace),
  * so a whole distributed sort is enqueued without the host ever reading a count.
- * d_src_hist (may be NULL; uint32[world][4][256], overwritten): the partition kernel also counts, per destination,
- * the 8-bit digit histograms 0..2 of the keys it sends there (of key ^ 0x80000000, as b200sort_radix_histogram_i32;
- * row 3, the top byte, stays zero: take it from the plan record's top_hist).
+ * d_src_hist (may be NULL; uint32[world][4][256]; needs bits >= 8, else B200SORT_ERR_INVALID before any device work):
+ * the partition kernel also counts, per destination, the 8-bit digit histograms 0..2 of the keys it sends there (of
+ * key ^ 0x80000000, as b200sort_radix_histogram_i32; row 3, the top byte, stays zero: take it from the plan record's
+ * top_hist).  d_src_hist is overwritten by every call, n == 0 included, and holds zeros when the plan's error flag is
+ * set.
  * Summed over the source ranks (a reduce-scatter, which doubles as the barrier after the exchange) row r is the
  * histogram of exactly what rank r received; passed as d_hist (may be NULL) to b200sort_radix_copy_devn_i32 it lets
  * the local sort skip its own histogram kernel. */

@@ -386,9 +386,15 @@ static int partition_launch(const int32_t *d_keys, size_t n, int bits, int world
     if (bits < B200SORT_DIST_BITS_MIN || bits > B200SORT_DIST_BITS_MAX || world < 1 || world > kDistMaxWorld ||
         h_dst_base == nullptr || (h_dst_offset == nullptr && d_plan == nullptr) || d_bin_owner == nullptr)
         return B200SORT_ERR_INVALID;
+    // Below 8 bits a bin spans more than one top-byte value, so the plan record cannot give row 3 (top_hist stays zero)
+    // and source histograms would hand the local sort a wrong top-byte row.
+    if (d_src_hist != nullptr && bits < 8) return B200SORT_ERR_INVALID;
     if (d_ws == nullptr || ws_bytes < 256) return B200SORT_ERR_WORKSPACE;
     for (int r = 0; r < world; ++r)       // 128-bit stores / bulk copies into the destinations
         if (reinterpret_cast<uintptr_t>(h_dst_base[r]) & 15) return B200SORT_ERR_INVALID;
+    // every call overwrites the source histograms, n == 0 included: a rank that sends nothing contributes zeros
+    if (d_src_hist != nullptr)
+        B200_CUDA_TRY(cudaMemsetAsync(d_src_hist, 0, (size_t)world * 1024 * sizeof(unsigned int), s));
     if (n == 0) return B200SORT_OK;
     DistPartitionArgs args;
     std::memset(&args, 0, sizeof args);
@@ -396,7 +402,6 @@ static int partition_launch(const int32_t *d_keys, size_t n, int bits, int world
     args.plan = d_plan;
     args.src_hist = d_src_hist;
     if (d_src_hist != nullptr) {                       // histograms ride along: the bulk-copy shape only
-        B200_CUDA_TRY(cudaMemsetAsync(d_src_hist, 0, (size_t)world * 1024 * sizeof(unsigned int), s));
         B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(dist_partition_kernel<512, 2, 1, 1>),
                                            cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)partition_smem(B200SORT_DIST_BITS_MAX, 512, kDistMaxWorld)));
