@@ -28,6 +28,9 @@
  *   b200sort_sort_keys64 / b200sort_radix_pairs_keys64
  *                               no reference counterpart: int64, uint64 and float64 keys (8 radix passes),
  *                               keys only or with an int32 value
+ *   b200sort_sort_keys16 / b200sort_radix_pairs_keys16
+ *                               no reference counterpart: int16, uint16, float16 and bfloat16 keys (a counting
+ *                               sort for keys only, 2 radix passes with an int32 value)
  *
  * The C++ symbols order_array(int*,int) / order_with_trust(int*,int) that SRM/main.cpp and
  * SRM/performanceTest.cpp link against are exported by the same library (csrc/lab_shim.cu) with
@@ -184,6 +187,50 @@ int    b200sort_sort_keys64(int key_type, int descending, const void *d_in, void
 /* Stable sort of (64-bit key, int32 value) pairs by key.  In place iff d_keys_in == d_keys_out and
  * d_vals_in == d_vals_out; a mix of the two -> B200SORT_ERR_INVALID.  Same workspace as b200sort_sort_keys64. */
 int    b200sort_radix_pairs_keys64(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                   void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                   size_t n, void *d_ws, size_t ws_bytes, void *stream);
+
+/* ---- 16-bit keys: int16, uint16, float16 and bfloat16 ------------------------------------------------------
+ * Keys are 2-byte words; key_type says how they compare:
+ *   B200SORT_KEY_I16   signed integers, numeric order;
+ *   B200SORT_KEY_U16   unsigned integers, numeric order;
+ *   B200SORT_KEY_F16   IEEE-754 binary16, and
+ *   B200SORT_KEY_BF16  bfloat16 (the top half of a binary32), both in totalOrder on the bit pattern, as
+ *                      B200SORT_KEY_F32: -NaN (any payload) < -inf < negatives < -0.0 < +0.0 < positives < +inf <
+ *                      +NaN, NaNs of one sign ordered by payload.  Bits are never changed.  This is NOT the order of
+ *                      torch.sort / np.sort, which treat -0.0 == +0.0 and put every NaN last.
+ * F16 and BF16 share one order; both names exist so that callers can name their dtype.  The 32-bit, segmented and
+ * 64-bit entry points reject these key types, and these entry points reject B200SORT_KEY_I32..F64.  descending = 1
+ * is the reverse order.  Every order is image(k) = k ^ (bit 15 of k set ? M_neg : M_pos) sorted as uint16.
+ * The output holds the input's bit patterns, permuted.  DESIGN section 4.2f.
+ *
+ * b200sort_sort_keys16 sorts by counting: one read of the keys counts each of the 65536 bit patterns, the counts are
+ * scanned in image order, and every pattern is written `count` times.  It ranks nothing, so it needs neither the
+ * lane-order self-test of b200sort_radix_i32 nor its ballot-ranked fallback, has no scratch buffer and no 2^30 limit.
+ * b200sort_radix_pairs_keys16 is a STABLE sort in both directions (without NaN or -0.0 it equals
+ * torch.sort(stable=True, descending=...)): after the same count, two radix passes of 8-bit digits of the image, of
+ * which one where a single digit value holds every key is skipped on the device (b200sort_radix_set_skip applies).
+ * Its passes rank like the other radix sorts: lane-ordered shared-memory atomics after the self-test has passed on
+ * the device, otherwise, or with B200SORT_RANK_SAFE=1, the ballot-ranked form.  b200sort_radix_set_variant applies to
+ * neither.  A call enqueues one memset and the same kernels for every n >= 2 and every distribution (3 for keys, 5
+ * for pairs), never synchronises and never reads device results on the host, so it can be captured in a CUDA graph
+ * (pairs once b200sort_device_check() has run).
+ * Key pointers need only 2-byte alignment.  d_in may equal d_out (in place); otherwise d_in is only read.
+ * Workspace: b200sort_keys16_workspace_bytes(n) bytes, 256-byte aligned, sized from n alone, for keys and pairs.
+ * Key type outside B200SORT_KEY_I16..BF16, descending not 0/1, n > B200SORT_MAX_N, NULL data pointers with n > 0, key
+ * pointers not 2-byte aligned -> B200SORT_ERR_INVALID; missing, small or misaligned workspace ->
+ * B200SORT_ERR_WORKSPACE; all checked before any device work.  n == 0, and n == 1 in place, return B200SORT_OK
+ * without touching the device.  Pairs with b200sort_radix_set_skip(0) and n = 2^30 -> B200SORT_ERR_INVALID. */
+#define B200SORT_KEY_I16            6
+#define B200SORT_KEY_U16            7
+#define B200SORT_KEY_F16            8
+#define B200SORT_KEY_BF16           9
+size_t b200sort_keys16_workspace_bytes(size_t n);
+int    b200sort_sort_keys16(int key_type, int descending, const void *d_in, void *d_out, size_t n, void *d_ws,
+                            size_t ws_bytes, void *stream);
+/* Stable sort of (16-bit key, int32 value) pairs by key.  d_tmp_keys, d_tmp_vals: n keys and n values of scratch.
+ * In place iff d_keys_in == d_keys_out and d_vals_in == d_vals_out; a mix of the two -> B200SORT_ERR_INVALID. */
+int    b200sort_radix_pairs_keys16(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
                                    void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
                                    size_t n, void *d_ws, size_t ws_bytes, void *stream);
 

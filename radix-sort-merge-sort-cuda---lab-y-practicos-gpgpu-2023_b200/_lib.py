@@ -49,6 +49,9 @@ SIGNATURES = {
     "b200sort_keys64_workspace_bytes": (_sz, [_sz]),
     "b200sort_sort_keys64": (_i, [_i, _i, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_radix_pairs_keys64": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_keys16_workspace_bytes": (_sz, [_sz]),
+    "b200sort_sort_keys16": (_i, [_i, _i, _vp, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_radix_pairs_keys16": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_segmented_workspace_bytes": (_sz, [_sz, _sz]),
     "b200sort_segmented_sort_keys": (_i, [_i, _i, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_segmented_pairs_keys": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),

@@ -4,6 +4,7 @@
 #include "dist.cuh"
 #include "merge.cuh"
 #include "radix.cuh"
+#include "radix16.cuh"
 #include "radix64.cuh"
 #include "segmented.cuh"
 
@@ -505,6 +506,40 @@ int b200sort_radix_pairs_keys64(int key_type, int descending, const void *d_keys
                         static_cast<cudaStream_t>(stream), order);
 }
 
+// Argument checks of the 16-bit entry points that come before the workspace, in the order and with the statuses of
+// the 64-bit ones; key pointers need 2-byte alignment.  d_tmp (pairs only) may be NULL for keys only.
+static int check_keys16_args(int key_type, int descending, SignXor16 *order, size_t n, const void *in, const void *out,
+                             const void *tmp, bool need_tmp) {
+    if (!key_order16(key_type, descending, order)) return B200SORT_ERR_INVALID;
+    if (n > B200SORT_MAX_N) return B200SORT_ERR_INVALID;
+    if (n > 0 && (in == nullptr || out == nullptr || (need_tmp && tmp == nullptr))) return B200SORT_ERR_INVALID;
+    if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(tmp)) & 1) != 0)
+        return B200SORT_ERR_INVALID;
+    return B200SORT_OK;
+}
+
+size_t b200sort_keys16_workspace_bytes(size_t n) { return radix16_workspace_bytes(n); }
+
+int b200sort_sort_keys16(int key_type, int descending, const void *d_in, void *d_out, size_t n, void *d_ws,
+                         size_t ws_bytes, void *stream) {
+    SignXor16 order;
+    B200_TRY(check_keys16_args(key_type, descending, &order, n, d_in, d_out, nullptr, false));
+    return radix16_sort(static_cast<const uint16_t *>(d_in), static_cast<uint16_t *>(d_out), nullptr, nullptr, nullptr,
+                        nullptr, n, d_ws, ws_bytes, static_cast<cudaStream_t>(stream), order);
+}
+
+int b200sort_radix_pairs_keys16(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals, size_t n,
+                                void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor16 order;
+    B200_TRY(check_keys16_args(key_type, descending, &order, n, d_keys_in, d_keys_out, d_tmp_keys, true));
+    if (n > 0 && (d_vals_in == nullptr || d_vals_out == nullptr || d_tmp_vals == nullptr)) return B200SORT_ERR_INVALID;
+    if ((d_keys_in == d_keys_out) != (d_vals_in == d_vals_out)) return B200SORT_ERR_INVALID;   // one plan for both
+    return radix16_sort(static_cast<const uint16_t *>(d_keys_in), static_cast<uint16_t *>(d_keys_out),
+                        static_cast<uint16_t *>(d_tmp_keys), d_vals_in, d_vals_out, d_tmp_vals, n, d_ws, ws_bytes,
+                        static_cast<cudaStream_t>(stream), order);
+}
+
 // Argument checks of the segmented entry points, in the order and with the statuses of b200sort_sort_keys.
 static int check_segmented_args(size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws, size_t ws_bytes) {
     if (num_segments > B200SORT_MAX_N || (num_segments > 0 && d_offsets == nullptr)) return B200SORT_ERR_INVALID;
@@ -602,13 +637,13 @@ int b200sort_debug_checked_build(void) {
 }
 unsigned long long b200sort_debug_check_failures(void) {
     return radix_check_failures(nullptr) + dist_check_failures(nullptr) + segmented_check_failures(nullptr) +
-           radix64_check_failures(nullptr);
+           radix64_check_failures(nullptr) + radix16_check_failures(nullptr);
 }
 unsigned long long b200sort_debug_check_failures_by_site(unsigned long long *per_site /* [16], overwritten */) {
     if (per_site == nullptr) return 0;
     for (int i = 0; i < 16; ++i) per_site[i] = 0;
     return radix_check_failures(per_site) + dist_check_failures(per_site) + segmented_check_failures(per_site) +
-           radix64_check_failures(per_site);
+           radix64_check_failures(per_site) + radix16_check_failures(per_site);
 }
 const char *b200sort_radix_effective_variant_name(void) { return radix_effective_variant_name(); }
 int b200sort_radix_set_skip(int enabled) { radix_set_skip(enabled); return B200SORT_OK; }

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """What compute-sanitizer runs (tools/sanitize.sh): every kernel family once at smoke sizes, each result checked
-against the oracle.  `python tools/sanitize_target.py [big]` -- `big` adds one 2^20-key radix sort."""
+against the oracle.  `python tools/sanitize_target.py [big | keys16]` -- `big` adds one 2^20-key radix sort; `keys16` runs only the
+16-bit sorts."""
 import ctypes
 import os
 import sys
@@ -26,6 +27,35 @@ n = 1 << 16
 def same(a, b, what):
     assert a.tobytes() == b.tobytes(), what
     print("  ok", what, flush=True)
+
+
+def keys16_runs(full_size):
+    """16-bit keys: the counting sort and the pairs passes, keys off a 16-byte boundary, a skipped pass."""
+    import key_orders16 as ko16
+    from test_keys16_gpu import check_both, low_entropy, random_keys
+    sizes = (n + 123, (1 << 22) + 77) if full_size else (n + 123,)
+    for m in sizes:
+        check_both(random_keys(m, ko16.KEY_BF16, 14), ko16.KEY_BF16, 1, f"16-bit keys and pairs n={m} bfloat16 desc",
+                   offs_k=(6, 2), offs_p=(6, 2, 14))
+        check_both(low_entropy("constant_high_byte", m).view(np.int16), ko16.KEY_I16, 0,
+                   f"16-bit n={m} int16, pass 1 skipped")
+        print("  ok 16-bit keys and pairs n =", m, flush=True)
+
+
+def report_checked():
+    sites = (ctypes.c_ulonglong * 16)()
+    fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
+    print('per check site:', list(sites), flush=True)
+    print(f"CHECKED BUILD: {fails} violated kernel invariants (staged positions, destination indices, bulk-copy alignment)", flush=True)
+    assert fails == 0
+
+
+if len(sys.argv) > 1 and sys.argv[1] == "keys16":      # only the 16-bit sorts, at smoke and full size
+    keys16_runs(True)
+    if L.b200sort_debug_checked_build():
+        report_checked()
+    print("SANITIZE TARGET PASSED", flush=True)
+    sys.exit(0)
 
 
 keys = datagen.uniform(n, 3)
@@ -101,6 +131,7 @@ k64 = low_entropy("below_2_32", n + 45).view(np.int64)
 k64_gk, k64_gv = sort64_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 0, True)
 k64_wk, k64_wv = ko64.sort_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 0)
 same(k64_gk, ko64.bits(k64_wk), "64-bit pairs: keys (4 passes skipped)"); same(k64_gv, k64_wv, "64-bit pairs: values (stable)")
+keys16_runs(False)
 # host operator
 h = datagen.lab_rand(4096, 100, seed=1)
 wh = oracle.order_array(h)
@@ -123,9 +154,6 @@ if L.b200sort_debug_checked_build():
     k64_gk, k64_gv = sort64_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 1, False)
     k64_wk, k64_wv = ko64.sort_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 1)
     same(k64_gk, ko64.bits(k64_wk), "64-bit pairs n=2^22+77: keys"); same(k64_gv, k64_wv, "64-bit pairs: values")
-    sites = (ctypes.c_ulonglong * 16)()
-    fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
-    print('per check site:', list(sites), flush=True)
-    print(f"CHECKED BUILD: {fails} violated kernel invariants (staged positions, destination indices, bulk-copy alignment)", flush=True)
-    assert fails == 0
+    keys16_runs(True)
+    report_checked()
 print("SANITIZE TARGET PASSED", flush=True)
