@@ -31,6 +31,9 @@
  *   b200sort_sort_keys16 / b200sort_radix_pairs_keys16
  *                               no reference counterpart: int16, uint16, float16 and bfloat16 keys (a counting
  *                               sort for keys only, 2 radix passes with an int32 value)
+ *   b200sort_segmented_sort_keys16 / b200sort_segmented_pairs_keys16
+ *                               no reference counterpart: every segment (row) of 16-bit keys sorted on its own
+ *                               in one call, keys only or with an int32 value
  *
  * The C++ symbols order_array(int*,int) / order_with_trust(int*,int) that SRM/main.cpp and
  * SRM/performanceTest.cpp link against are exported by the same library (csrc/lab_shim.cu) with
@@ -266,6 +269,44 @@ int    b200sort_segmented_pairs_keys(int key_type, int descending, const void *d
                                      void *d_ws, size_t ws_bytes, void *stream);
 /* Largest segment length served by size class c (0, 1, ...); 0 past the last class (the onesweep class, unbounded). */
 size_t b200sort_segmented_class_max(int c);
+
+/* ---- segmented sort of 16-bit keys: int16, uint16, float16 and bfloat16 -----------------------------------
+ * The segmented sort above on the 2-byte keys of b200sort_sort_keys16: segment i = keys[d_offsets[i] ..
+ * d_offsets[i+1]) comes out sorted in the order (key_type, descending) of b200sort_sort_keys16, image(k) = k ^ (bit 15
+ * set ? M_neg : M_pos) sorted as uint16 (float16 and bfloat16: IEEE-754 totalOrder on the bits; bits are never
+ * changed).  Only B200SORT_KEY_I16..BF16 are accepted; the 32-bit segmented entry points keep rejecting them.
+ * Pairs are STABLE within each segment in both directions: without NaN and -0.0, rows sorted by
+ * b200sort_segmented_pairs_keys16 with values 0..L-1 equal torch.sort(x, dim=-1, stable=True, descending=...) in
+ * values and indices.
+ * d_offsets follows the rules of b200sort_segmented_sort_keys: a DEVICE array of num_segments + 1 int32 the host
+ * never reads, segments clamped to [0, n] on the device, malformed offsets giving an undefined order but no access
+ * out of bounds (the checked build counts the clamps at check site 15).
+ * A call enqueues one memset and the same eight kernels whatever the number of segments and the data, never
+ * synchronises, and can be captured in a CUDA graph once b200sort_device_check() has run.  Size classes
+ * (b200sort_segmented16_class_max): copies for length 0-1, a warp per segment, a CTA per segment sorted in shared
+ * memory by two 8-bit passes (two capacities), and above that a segmented onesweep of two passes whose tiles never
+ * straddle a segment.  The ranking kernels use lane-ordered shared-memory atomics only after the self-test of
+ * b200sort_radix_i32 has passed on the device; otherwise, or with B200SORT_RANK_SAFE=1, their ballot-ranked forms run.
+ * b200sort_radix_set_variant and b200sort_radix_set_skip are ignored.  DESIGN section 4.2g.
+ * Key pointers need only 2-byte alignment: segments may begin anywhere.  d_in may equal d_out; otherwise d_in is only
+ * read.  d_tmp: n keys of scratch.  Workspace: b200sort_segmented16_workspace_bytes(n, num_segments) bytes, 256-byte
+ * aligned, sized from (n, num_segments) alone.
+ * Key type outside B200SORT_KEY_I16..BF16, descending not 0/1, NULL data pointers, odd key pointers, n or
+ * num_segments > B200SORT_MAX_N, NULL d_offsets with num_segments > 0 -> B200SORT_ERR_INVALID; missing, small or
+ * misaligned workspace -> B200SORT_ERR_WORKSPACE; all checked before any device work, in the order of the 32-bit
+ * segmented entry points.  n == 0 returns B200SORT_OK without touching the device. */
+size_t b200sort_segmented16_workspace_bytes(size_t n, size_t num_segments);
+/* Largest segment length served by size class c of the 16-bit segmented sort; 0 past the last bounded class. */
+size_t b200sort_segmented16_class_max(int c);
+int    b200sort_segmented_sort_keys16(int key_type, int descending, const void *d_in, void *d_out, void *d_tmp,
+                                      size_t n, const int32_t *d_offsets, size_t num_segments,
+                                      void *d_ws, size_t ws_bytes, void *stream);
+/* Stable within each segment; in place iff d_keys_in == d_keys_out and d_vals_in == d_vals_out, a mix of the two ->
+ * B200SORT_ERR_INVALID. */
+int    b200sort_segmented_pairs_keys16(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                       void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                       size_t n, const int32_t *d_offsets, size_t num_segments,
+                                       void *d_ws, size_t ws_bytes, void *stream);
 
 /* ---- stages, exposed for unit tests and per-kernel timing -------------------------------------- */
 

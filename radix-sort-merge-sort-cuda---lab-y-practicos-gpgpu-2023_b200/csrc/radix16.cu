@@ -51,14 +51,6 @@ struct R16Control {
 constexpr size_t kR16ZeroBytes = offsetof(R16Control, incl);
 constexpr size_t kR16ControlBytes = (sizeof(R16Control) + 255) / 256 * 256;
 
-__host__ __device__ __forceinline__ uint32_t image16(uint32_t k, SignXor16 o) {
-    return k ^ ((k & 0x8000u) ? o.neg : o.pos);
-}
-// The masks that map an image back to its key (common.cuh's image_inverse on 16-bit words).
-__host__ __device__ __forceinline__ SignXor16 inverse16(SignXor16 o) {
-    return (o.neg & 0x8000u) ? SignXor16{o.pos, o.neg} : SignXor16{o.neg, o.pos};
-}
-
 // ---- r0 -------------------------------------------------------------------------------------------------------------
 // 65536 32-bit counters would need 256 KiB, more than a CTA can have.  Image j counts in half (j & 1) of shared word
 // j >> 1.  A counter that wraps past 0xFFFF is repaired in ctl->over from the atomic's return value: +65536 for the

@@ -23,6 +23,14 @@ inline bool key_order16(int key_type, int descending, SignXor16 *m) {
     return true;
 }
 
+__host__ __device__ __forceinline__ uint32_t image16(uint32_t k, SignXor16 o) {
+    return k ^ ((k & 0x8000u) ? o.neg : o.pos);
+}
+// The masks that map an image back to its key (common.cuh's image_inverse on 16-bit words).
+__host__ __device__ __forceinline__ SignXor16 inverse16(SignXor16 o) {
+    return (o.neg & 0x8000u) ? SignXor16{o.pos, o.neg} : SignXor16{o.neg, o.pos};
+}
+
 size_t radix16_workspace_bytes(size_t n);
 // d_in may equal d_out.  v_in == nullptr sorts keys only, by counting (d_tmp unused); otherwise the pairs are sorted
 // stably by two radix passes, in place iff d_in == d_out (then v_in must equal v_out).  The caller has checked the

@@ -17,13 +17,13 @@ KEY_F16 = 8
 KEY_BF16 = 9
 
 
-def _key_type(torch, x) -> int:
+def _key_type(torch, x, others: str = "32-bit keys: b200sort.sort; 64-bit keys: b200sort.sort64") -> int:
     types = {torch.int16: KEY_I16, torch.uint16: KEY_U16, torch.float16: KEY_F16, torch.bfloat16: KEY_BF16}
     if not isinstance(x, torch.Tensor):
         raise TypeError(f"expected a torch.Tensor, got {type(x).__name__}")
     if x.dtype not in types:
         raise TypeError(f"keys must be torch.int16, torch.uint16, torch.float16 or torch.bfloat16, got {x.dtype} "
-                        f"(32-bit keys: b200sort.sort; 64-bit keys: b200sort.sort64)")
+                        f"({others})")
     return types[x.dtype]
 
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """What compute-sanitizer runs (tools/sanitize.sh): every kernel family once at smoke sizes, each result checked
-against the oracle.  `python tools/sanitize_target.py [big | keys16]` -- `big` adds one 2^20-key radix sort; `keys16` runs only the
-16-bit sorts."""
+against the oracle.  `python tools/sanitize_target.py [big | keys16 | segmented16]` -- `big` adds one 2^20-key radix sort; `keys16` runs
+only the 16-bit sorts, `segmented16` only the segmented sort of 16-bit keys."""
 import ctypes
 import os
 import sys
@@ -42,6 +42,21 @@ def keys16_runs(full_size):
         print("  ok 16-bit keys and pairs n =", m, flush=True)
 
 
+def segmented16_runs():
+    """Segmented 16-bit keys: a ragged mix covering every size class, bfloat16 descending, keys and pairs."""
+    import key_orders16 as ko16
+    from test_segmented16_gpu import check_pairs, mixed_keys, ragged_offsets, seg_keys, seg_sort_keys
+    offs = ragged_offsets(5, total_segments=2000, big=1)
+    m = int(offs[-1])
+    k = mixed_keys(m, ko16.KEY_BF16, 11)
+    same(seg_keys(k, offs, ko16.KEY_BF16, 1, False), ko16.bits(seg_sort_keys(k, offs, ko16.KEY_BF16, 1)),
+         f"segmented 16-bit keys n={m}, {offs.size - 1} segments, bfloat16 desc")
+    check_pairs(k, offs, ko16.KEY_BF16, 1, False, "segmented 16-bit pairs")
+    check_pairs((k.view(np.uint16) % np.uint16(50)).view(np.int16), offs, ko16.KEY_I16, 0, True,
+                "segmented 16-bit pairs in place, many ties")
+    print("  ok segmented 16-bit pairs (stable)", flush=True)
+
+
 def report_checked():
     sites = (ctypes.c_ulonglong * 16)()
     fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
@@ -52,6 +67,14 @@ def report_checked():
 
 if len(sys.argv) > 1 and sys.argv[1] == "keys16":      # only the 16-bit sorts, at smoke and full size
     keys16_runs(True)
+    if L.b200sort_debug_checked_build():
+        report_checked()
+    print("SANITIZE TARGET PASSED", flush=True)
+    sys.exit(0)
+
+
+if len(sys.argv) > 1 and sys.argv[1] == "segmented16":  # only the segmented sort of 16-bit keys
+    segmented16_runs()
     if L.b200sort_debug_checked_build():
         report_checked()
     print("SANITIZE TARGET PASSED", flush=True)
@@ -132,6 +155,7 @@ k64_gk, k64_gv = sort64_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY
 k64_wk, k64_wv = ko64.sort_pairs(k64, np.arange(k64.size, dtype=np.int32), ko64.KEY_I64, 0)
 same(k64_gk, ko64.bits(k64_wk), "64-bit pairs: keys (4 passes skipped)"); same(k64_gv, k64_wv, "64-bit pairs: values (stable)")
 keys16_runs(False)
+segmented16_runs()
 # host operator
 h = datagen.lab_rand(4096, 100, seed=1)
 wh = oracle.order_array(h)
