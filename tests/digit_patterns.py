@@ -1,5 +1,6 @@
-"""Key generators that steer the radix sorts' device-side pass plan, and canary-guarded buffer layouts (test
-infrastructure only, numpy only).
+"""Key generators that steer the radix sorts' device-side pass plan, canary-guarded buffer layouts, and the guarded
+device buffers and never-cleared workspace the GPU tests build from them (test infrastructure only; numpy, and torch
+only inside DevBuf and Workspace).
 
 The histogram kernel of every 1-D radix sort skips a pass when one digit value holds all n keys, picks the buffer
 each executed pass reads and writes from the number of executed passes, and flags a pass as hot when one digit value
@@ -146,31 +147,88 @@ def canary(words: int, salt: int = 0) -> np.ndarray:
 
 
 class Guarded:
-    """Layout of a buffer of 32-bit words that holds n items of `itemsize` bytes starting `word_offset` words past a
-    16-byte boundary, with at least `guard_words` words on each side.  Whatever allocates the buffer (a 16-byte
-    aligned numpy array or device tensor of `total` words) fills it with `self.fill` and puts the array at word
-    `self.start`; `check` asserts that every word outside the array still holds its canary."""
+    """Layout of a buffer of words that holds n items of `itemsize` bytes starting `word_offset` words past a
+    16-byte boundary, with at least `guard_words` words on each side.  A word is 32 bits for items of 4 and 8 bytes
+    and 16 bits for items of 2 bytes (2-byte keys may begin 2, 6 or 14 bytes past a boundary: word offsets 1, 3, 7).
+    Whatever allocates the buffer (a 16-byte aligned numpy array or device tensor of `total` words of `self.dtype`)
+    fills it with `self.fill` and puts the array at word `self.start`; `check` asserts that every word outside the
+    array still holds its canary."""
 
     def __init__(self, n: int, word_offset: int, guard_words: int = 16, itemsize: int = 4, salt: int = 0):
-        assert guard_words % 4 == 0 and itemsize % 4 == 0
+        assert itemsize in (2, 4, 8)
+        self.word = min(itemsize, 4)                                   # bytes per word
+        self.dtype = np.uint16 if self.word == 2 else np.uint32
+        line = 16 // self.word                                         # words per 16 bytes
+        assert guard_words % line == 0 and 0 <= word_offset < line
         self.n, self.word_offset, self.itemsize = n, word_offset, itemsize
         self.start = guard_words + word_offset
-        self.end = self.start + n * itemsize // 4
-        self.total = (self.end + guard_words + 3) // 4 * 4
-        self.fill = canary(self.total, salt)
+        self.end = self.start + n * itemsize // self.word
+        self.total = (self.end + guard_words + line - 1) // line * line
+        self.fill = canary(self.total, salt).astype(self.dtype)      # 16-bit: i * odd stays distinct below 2^16 words
 
     def check(self, words: np.ndarray, what: str = "") -> None:
-        words = np.ascontiguousarray(words).view(np.uint32)
+        words = np.ascontiguousarray(words).view(self.dtype)
         assert words.size == self.total, (words.size, self.total)
         for side, lo, hi in (("before", 0, self.start), ("after", self.end, self.total)):
             bad = np.flatnonzero(words[lo:hi] != self.fill[lo:hi])
             if bad.size:
                 k = lo + int(bad[0])
                 where = k - self.start if side == "before" else k - self.end
+                w = 2 + 2 * self.word
                 raise AssertionError(f"{what}: guard word {side} the array changed ({bad.size} words), first at "
                                      f"word {where:+d} from the array's {'start' if side == 'before' else 'end'}: "
-                                     f"{int(words[k]):#010x}, canary {int(self.fill[k]):#010x}")
+                                     f"{int(words[k]):#0{w}x}, canary {int(self.fill[k]):#0{w}x}")
 
 
 def guarded(n: int, word_offset: int, guard_words: int = 16, itemsize: int = 4, salt: int = 0) -> Guarded:
     return Guarded(n, word_offset, guard_words, itemsize, salt)
+
+
+# ---- device buffers of the GPU tests (torch is imported only when one is made) ---------------------------------------
+class DevBuf:
+    """n items of `itemsize` bytes at `word_offset` words past a 16-byte boundary inside a canary-filled device buffer
+    (Guarded)."""
+
+    def __init__(self, n: int, word_offset: int, itemsize: int, salt: int):
+        import torch
+        self.g = guarded(n, word_offset, itemsize=itemsize, salt=salt)
+        self.t = torch.empty(self.g.total, dtype=torch.int16 if self.g.word == 2 else torch.int32, device="cuda")
+        assert self.t.data_ptr() % 16 == 0
+        self.ptr = self.t.data_ptr() + self.g.word * self.g.start
+
+    def load(self, words=None):
+        """Canaries everywhere, `words` (any dtype of the item size) in the array if given."""
+        import torch
+        full = self.g.fill.copy()
+        if words is not None:
+            full[self.g.start:self.g.end] = np.ascontiguousarray(words).view(self.g.dtype)
+        self.t.copy_(torch.from_numpy(full.view(np.int16 if self.g.word == 2 else np.int32)))
+        return self
+
+    def read(self, what: str) -> np.ndarray:
+        """The array's words (uint32, or uint16 for 2-byte items), after checking every guard word."""
+        full = self.t.cpu().numpy().view(self.g.dtype)
+        self.g.check(full, what)
+        return full[self.g.start:self.g.end].copy()
+
+
+class Workspace:
+    """One workspace of `cap` bytes (256-byte aligned) for a whole test module, filled with 0xFF bytes once and never
+    cleared: every call finds what the calls before it (other sizes, other paths, other plans) left there.
+    guard(nbytes) is the stretch of GUARD bytes just past one call's ws_bytes, which that call must not change;
+    check_tail asserts that the bytes past the last such stretch still hold 0xFF."""
+    GUARD = 1024
+
+    def __init__(self, cap: int):
+        import torch
+        self.cap = cap + self.GUARD
+        self.t = torch.full((self.cap + 256 + self.GUARD,), 0xFF, dtype=torch.uint8, device="cuda")
+        self.lo = (-self.t.data_ptr()) % 256
+        self.ptr = self.t.data_ptr() + self.lo
+
+    def guard(self, nbytes: int):
+        return self.t[self.lo + nbytes:self.lo + nbytes + self.GUARD]
+
+    def check_tail(self):
+        tail = self.t[self.lo + self.cap:].cpu().numpy()
+        assert bool((tail == 0xFF).all()), "workspace written past every call's ws_bytes"

@@ -105,11 +105,16 @@ def test_locally_hot_runs_without_a_globally_hot_digit():
                 assert not bool((runs[:, 1, :] == runs[:, 1, :1]).all())      # the odd runs do not
 
 
-@pytest.mark.parametrize("word_offset,itemsize", [(0, 4), (1, 4), (2, 4), (3, 4), (0, 8), (2, 8)])
+# 2-byte items: 16-bit words, 2, 6 and 14 bytes past a 16-byte boundary
+@pytest.mark.parametrize("word_offset,itemsize", [(0, 4), (1, 4), (2, 4), (3, 4), (0, 8), (2, 8),
+                                                  (0, 2), (1, 2), (3, 2), (7, 2)])
 def test_guard_catches_a_changed_word_on_either_side(word_offset, itemsize):
-    n = 1000
+    n = 1001
     g = dp.guarded(n, word_offset, itemsize=itemsize)
-    assert g.start % 4 == word_offset and (g.end - g.start) * 4 == n * itemsize and g.total % 4 == 0
+    word = min(itemsize, 4)
+    assert g.fill.dtype.itemsize == word
+    assert (g.start * word) % 16 == word_offset * word and (g.end - g.start) * word == n * itemsize
+    assert (g.total * word) % 16 == 0
     assert g.total - g.end >= 16 and g.start >= 16
     buf = g.fill.copy()
     buf[g.start:g.end] = 0                                                     # the array itself may change
@@ -119,5 +124,16 @@ def test_guard_catches_a_changed_word_on_either_side(word_offset, itemsize):
         bad[k] ^= 1
         with pytest.raises(AssertionError, match=f"guard word {side}"):
             g.check(bad, "test")
+        if word == 2:                                                          # a byte of the word next to the array
+            raw = buf.copy().view(np.uint8)
+            raw[2 * k + 1] ^= 0x80
+            with pytest.raises(AssertionError, match=f"guard word {side}"):
+                g.check(raw, "test")
     assert len(np.unique(g.fill)) == g.total                                   # no two canary words alike
-    assert dp.guarded(n, word_offset, salt=1).fill.tobytes() != g.fill.tobytes()
+    assert dp.guarded(n, word_offset, itemsize=itemsize, salt=1).fill.tobytes() != g.fill.tobytes()
+
+
+def test_guard_rejects_offsets_past_a_16_byte_boundary():
+    for word_offset, itemsize in ((4, 4), (4, 8), (8, 2), (-1, 2)):
+        with pytest.raises(AssertionError):
+            dp.guarded(100, word_offset, itemsize=itemsize)

@@ -59,75 +59,26 @@ def plan_config(variant: int = 0, skip: int = 1):
         L.b200sort_radix_set_skip(1)
 
 
-# ---- guarded device buffers and the shared workspace --------------------------------------------------------------
-class DevBuf:
-    """n items of `itemsize` bytes at `word_offset` words past a 16-byte boundary inside a canary-filled device buffer
-    (digit_patterns.Guarded)."""
-
-    def __init__(self, n: int, word_offset: int, itemsize: int, salt: int):
-        import torch
-        self.g = dp.guarded(n, word_offset, itemsize=itemsize, salt=salt)
-        self.t = torch.empty(self.g.total, dtype=torch.int32, device="cuda")
-        assert self.t.data_ptr() % 16 == 0
-        self.ptr = self.t.data_ptr() + 4 * self.g.start
-
-    def load(self, words=None):
-        """Canaries everywhere, `words` (any 4- or 8-byte dtype) in the array if given."""
-        import torch
-        full = self.g.fill.copy()
-        if words is not None:
-            full[self.g.start:self.g.end] = np.ascontiguousarray(words).view(np.uint32)
-        self.t.copy_(torch.from_numpy(full.view(np.int32)))
-        return self
-
-    def read(self, what: str) -> np.ndarray:
-        """The array's words (uint32), after checking every guard word."""
-        full = self.t.cpu().numpy().view(np.uint32)
-        self.g.check(full, what)
-        return full[self.g.start:self.g.end].copy()
-
-
+# ---- guarded device buffers and the shared workspace (digit_patterns.DevBuf, digit_patterns.Workspace) -----------
 _bufs = {}
 
 
-def _buf(role: str, n: int, word_offset: int, itemsize: int = 4) -> DevBuf:
+def _buf(role: str, n: int, word_offset: int, itemsize: int = 4) -> dp.DevBuf:
     key = (role, n, word_offset, itemsize)
     if key not in _bufs:
-        _bufs[key] = DevBuf(n, word_offset, itemsize, salt=len(_bufs) + 1)
+        _bufs[key] = dp.DevBuf(n, word_offset, itemsize, salt=len(_bufs) + 1)
     return _bufs[key]
-
-
-class Workspace:
-    """One workspace for the module, filled with 0xFF bytes once and never cleared: every call finds what the calls
-    before it (other sizes, other paths, other plans) left there.  The bytes just past each call's ws_bytes must not
-    change."""
-    GUARD = 1024
-
-    def __init__(self):
-        import torch
-        L = lib()
-        cap = max(L.b200sort_workspace_bytes(N_BIG, ALGO_RADIX), L.b200sort_workspace_bytes(N_BIG, ALGO_MERGE),
-                  L.b200sort_keys64_workspace_bytes(N64_BIG))
-        self.cap = cap + self.GUARD
-        self.t = torch.full((self.cap + 256 + self.GUARD,), 0xFF, dtype=torch.uint8, device="cuda")
-        self.lo = (-self.t.data_ptr()) % 256
-        self.ptr = self.t.data_ptr() + self.lo
-
-    def guard(self, nbytes: int):
-        return self.t[self.lo + nbytes:self.lo + nbytes + self.GUARD]
-
-    def check_tail(self):
-        tail = self.t[self.lo + self.cap:].cpu().numpy()
-        assert bool((tail == 0xFF).all()), "workspace written past every call's ws_bytes"
 
 
 _ws = None
 
 
-def workspace() -> Workspace:
+def workspace() -> dp.Workspace:
     global _ws
     if _ws is None:
-        _ws = Workspace()
+        L = lib()
+        _ws = dp.Workspace(max(L.b200sort_workspace_bytes(N_BIG, ALGO_RADIX), L.b200sort_workspace_bytes(N_BIG, ALGO_MERGE),
+                               L.b200sort_keys64_workspace_bytes(N64_BIG)))
     return _ws
 
 
