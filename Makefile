@@ -20,7 +20,7 @@ endif
 REFROOT ?= /root/reference
 SRM     := $(REFROOT)/Sord Radix y Merge
 
-SRCS := $(CSRC)/radix.cu $(CSRC)/merge.cu $(CSRC)/dist.cu $(CSRC)/segmented.cu $(CSRC)/radix64.cu $(CSRC)/radix16.cu $(CSRC)/segmented16.cu $(CSRC)/api.cu $(CSRC)/lab_shim.cu
+SRCS := $(CSRC)/radix.cu $(CSRC)/merge.cu $(CSRC)/dist.cu $(CSRC)/segmented.cu $(CSRC)/radix64.cu $(CSRC)/radix16.cu $(CSRC)/segmented16.cu $(CSRC)/segmented64.cu $(CSRC)/api.cu $(CSRC)/lab_shim.cu
 HDRS := $(wildcard $(CSRC)/*.cuh) include/b200sort.h include/lab.h include/utils.h
 OBJS := $(patsubst $(CSRC)/%.cu,build/obj/%.o,$(SRCS))
 LIB  := $(PKG)/libb200sort.so

@@ -34,6 +34,10 @@
  *   b200sort_segmented_sort_keys16 / b200sort_segmented_pairs_keys16
  *                               no reference counterpart: every segment (row) of 16-bit keys sorted on its own
  *                               in one call, keys only or with an int32 value
+ *   b200sort_segmented_sort_keys64 / b200sort_segmented_pairs_keys64
+ *                               no reference counterpart: every segment (row) of 64-bit keys sorted on its own
+ *                               in one call, keys only or with an int32 value, skipping the digit passes that no
+ *                               segment needs
  *
  * The C++ symbols order_array(int*,int) / order_with_trust(int*,int) that SRM/main.cpp and
  * SRM/performanceTest.cpp link against are exported by the same library (csrc/lab_shim.cu) with
@@ -304,6 +308,49 @@ int    b200sort_segmented_sort_keys16(int key_type, int descending, const void *
 /* Stable within each segment; in place iff d_keys_in == d_keys_out and d_vals_in == d_vals_out, a mix of the two ->
  * B200SORT_ERR_INVALID. */
 int    b200sort_segmented_pairs_keys16(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                       void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                       size_t n, const int32_t *d_offsets, size_t num_segments,
+                                       void *d_ws, size_t ws_bytes, void *stream);
+
+/* ---- segmented sort of 64-bit keys: int64, uint64 and float64 -------------------------------------------
+ * The segmented sort above on the 8-byte keys of b200sort_sort_keys64: segment i = keys[d_offsets[i] ..
+ * d_offsets[i+1]) comes out sorted in the order (key_type, descending) of b200sort_sort_keys64, image(k) = k ^ (bit 63
+ * set ? M_neg : M_pos) sorted as uint64 (float64: IEEE-754 totalOrder on the bits; bits are never changed).  Only
+ * B200SORT_KEY_I64..F64 are accepted; the 32-bit and 16-bit segmented entry points keep rejecting them.
+ * Pairs are STABLE within each segment in both directions: without NaN and -0.0, rows sorted by
+ * b200sort_segmented_pairs_keys64 with values 0..L-1 equal torch.sort(x, dim=-1, stable=True, descending=...) in
+ * values and indices.
+ * d_offsets follows the rules of b200sort_segmented_sort_keys: a DEVICE array of num_segments + 1 int32 the host
+ * never reads, segments clamped to [0, n] on the device, malformed offsets giving an undefined order but no access
+ * out of bounds (the checked build counts the clamps at check site 15).
+ * Size classes (b200sort_segmented64_class_max): copies for length 0-1, a warp per segment, a CTA per segment sorted
+ * in shared memory by 8-bit passes (two capacities), and above that a segmented onesweep of 8 passes whose tiles never
+ * straddle a segment.  Passes are skipped on the device: a CTA-class segment skips every pass in which all its keys
+ * share the digit, and the onesweep class skips pass p when that holds in each of its segments (one large segment
+ * whose keys differ in digit p makes pass p run for all of them).  Rows of int64 ids below 2^32 thus run at most 4
+ * of the 8 passes.  A call still enqueues one memset and the same fifteen kernels whatever the number of segments
+ * and the data, never synchronises, and can be captured in a CUDA graph once b200sort_device_check() has run.  The
+ * ranking kernels use lane-ordered shared-memory atomics only after the self-test of b200sort_radix_i32 has passed on
+ * the device; otherwise, or with B200SORT_RANK_SAFE=1, their ballot-ranked forms run.  b200sort_radix_set_variant
+ * and b200sort_radix_set_skip are ignored: skipping is always on.  DESIGN section 4.2h.
+ * Any n up to B200SORT_MAX_N = 2^30 is accepted: a digit count reaches 2^30 only when one segment holds all 2^30 keys
+ * and every one of them has that digit, and then that pass is skipped.
+ * Key pointers need 8-byte alignment.  d_in may equal d_out; otherwise d_in is only read.  d_tmp: n keys of scratch.
+ * Workspace: b200sort_segmented64_workspace_bytes(n, num_segments) bytes, 256-byte aligned, sized from
+ * (n, num_segments) alone.
+ * Key type outside B200SORT_KEY_I64..F64, descending not 0/1, NULL data pointers, key pointers not 8-byte aligned, n
+ * or num_segments > B200SORT_MAX_N, NULL d_offsets with num_segments > 0 -> B200SORT_ERR_INVALID; missing, small or
+ * misaligned workspace -> B200SORT_ERR_WORKSPACE; all checked before any device work, in the order of the 32-bit
+ * segmented entry points.  n == 0 returns B200SORT_OK without touching the device. */
+size_t b200sort_segmented64_workspace_bytes(size_t n, size_t num_segments);
+/* Largest segment length served by size class c of the 64-bit segmented sort; 0 past the last bounded class. */
+size_t b200sort_segmented64_class_max(int c);
+int    b200sort_segmented_sort_keys64(int key_type, int descending, const void *d_in, void *d_out, void *d_tmp,
+                                      size_t n, const int32_t *d_offsets, size_t num_segments,
+                                      void *d_ws, size_t ws_bytes, void *stream);
+/* Stable within each segment; in place iff d_keys_in == d_keys_out and d_vals_in == d_vals_out, a mix of the two ->
+ * B200SORT_ERR_INVALID. */
+int    b200sort_segmented_pairs_keys64(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
                                        void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
                                        size_t n, const int32_t *d_offsets, size_t num_segments,
                                        void *d_ws, size_t ws_bytes, void *stream);

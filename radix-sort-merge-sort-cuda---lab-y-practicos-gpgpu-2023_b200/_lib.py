@@ -60,6 +60,10 @@ SIGNATURES = {
     "b200sort_segmented16_class_max": (_sz, [_i]),
     "b200sort_segmented_sort_keys16": (_i, [_i, _i, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_segmented_pairs_keys16": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_segmented64_workspace_bytes": (_sz, [_sz, _sz]),
+    "b200sort_segmented64_class_max": (_sz, [_i]),
+    "b200sort_segmented_sort_keys64": (_i, [_i, _i, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_segmented_pairs_keys64": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_radix_histogram_i32": (_i, [_vp, _sz, _vp, _vp]),
     "b200sort_radix_pass_i32": (_i, [_vp, _vp, _sz, _i, _vp, _sz, _vp]),
     "b200sort_block_sort_tile": (_sz, []),

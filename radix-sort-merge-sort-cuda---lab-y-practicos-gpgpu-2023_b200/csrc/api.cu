@@ -8,6 +8,7 @@
 #include "radix64.cuh"
 #include "segmented.cuh"
 #include "segmented16.cuh"
+#include "segmented64.cuh"
 
 #include <atomic>
 #include <cstdio>
@@ -642,6 +643,60 @@ int b200sort_segmented_pairs_keys16(int key_type, int descending, const void *d_
                             num_segments, d_ws, static_cast<cudaStream_t>(stream), order);
 }
 
+// Argument checks of the 64-bit segmented entry points before the workspace: those of b200sort_segmented_sort_keys in
+// its order and with its statuses, on the 64-bit key types, plus the 8-byte alignment of the key pointers.
+static int check_segmented64_keys(int key_type, int descending, SignXor64 *order, size_t n, const void *in,
+                                  const void *out, const void *tmp) {
+    if (!key_order64(key_type, descending, order)) return B200SORT_ERR_INVALID;
+    B200_TRY(check_sort_args(out, tmp, n));
+    if (n > 0 && (in == nullptr || out == nullptr)) return B200SORT_ERR_INVALID;        // n == 1 writes d_out too
+    if (((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(tmp)) & 7) != 0)
+        return B200SORT_ERR_INVALID;
+    return B200SORT_OK;
+}
+
+static int check_segmented64_args(size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws, size_t ws_bytes) {
+    if (num_segments > B200SORT_MAX_N || (num_segments > 0 && d_offsets == nullptr)) return B200SORT_ERR_INVALID;
+    if (n == 0) return B200SORT_OK;
+    if (d_ws == nullptr || (reinterpret_cast<uintptr_t>(d_ws) & 255) != 0 ||
+        ws_bytes < segmented64_workspace_bytes(n, num_segments))
+        return B200SORT_ERR_WORKSPACE;
+    return B200SORT_OK;
+}
+
+size_t b200sort_segmented64_workspace_bytes(size_t n, size_t num_segments) {
+    return segmented64_workspace_bytes(n, num_segments);
+}
+size_t b200sort_segmented64_class_max(int c) { return segmented64_class_max(c); }
+
+int b200sort_segmented_sort_keys64(int key_type, int descending, const void *d_in, void *d_out, void *d_tmp, size_t n,
+                                   const int32_t *d_offsets, size_t num_segments, void *d_ws, size_t ws_bytes,
+                                   void *stream) {
+    SignXor64 order;
+    B200_TRY(check_segmented64_keys(key_type, descending, &order, n, d_in, d_out, d_tmp));
+    B200_TRY(check_segmented64_args(n, d_offsets, num_segments, d_ws, ws_bytes));
+    if (n == 0) return B200SORT_OK;
+    return segmented64_sort(static_cast<const uint64_t *>(d_in), static_cast<uint64_t *>(d_out),
+                            static_cast<uint64_t *>(d_tmp), nullptr, nullptr, nullptr, n, d_offsets, num_segments, d_ws,
+                            static_cast<cudaStream_t>(stream), order);
+}
+
+int b200sort_segmented_pairs_keys64(int key_type, int descending, const void *d_keys_in, const int32_t *d_vals_in,
+                                    void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
+                                    size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws,
+                                    size_t ws_bytes, void *stream) {
+    SignXor64 order;
+    B200_TRY(check_segmented64_keys(key_type, descending, &order, n, d_keys_in, d_keys_out, d_tmp_keys));
+    B200_TRY(check_sort_args(d_vals_out, d_tmp_vals, n));
+    if (n > 0 && (d_vals_in == nullptr || d_vals_out == nullptr)) return B200SORT_ERR_INVALID;
+    if ((d_keys_in == d_keys_out) != (d_vals_in == d_vals_out)) return B200SORT_ERR_INVALID;
+    B200_TRY(check_segmented64_args(n, d_offsets, num_segments, d_ws, ws_bytes));
+    if (n == 0) return B200SORT_OK;
+    return segmented64_sort(static_cast<const uint64_t *>(d_keys_in), static_cast<uint64_t *>(d_keys_out),
+                            static_cast<uint64_t *>(d_tmp_keys), d_vals_in, d_vals_out, d_tmp_vals, n, d_offsets,
+                            num_segments, d_ws, static_cast<cudaStream_t>(stream), order);
+}
+
 int b200sort_radix_histogram_i32(const int32_t *d_keys, size_t n, uint32_t *d_hist, void *stream) {
     if (d_hist == nullptr || (n > 0 && d_keys == nullptr) || n > B200SORT_MAX_N) return B200SORT_ERR_INVALID;
     return radix_histogram(d_keys, n, d_hist, static_cast<cudaStream_t>(stream));
@@ -692,13 +747,15 @@ int b200sort_debug_checked_build(void) {
 }
 unsigned long long b200sort_debug_check_failures(void) {
     return radix_check_failures(nullptr) + dist_check_failures(nullptr) + segmented_check_failures(nullptr) +
-           radix64_check_failures(nullptr) + radix16_check_failures(nullptr) + segmented16_check_failures(nullptr);
+           radix64_check_failures(nullptr) + radix16_check_failures(nullptr) + segmented16_check_failures(nullptr) +
+           segmented64_check_failures(nullptr);
 }
 unsigned long long b200sort_debug_check_failures_by_site(unsigned long long *per_site /* [16], overwritten */) {
     if (per_site == nullptr) return 0;
     for (int i = 0; i < 16; ++i) per_site[i] = 0;
     return radix_check_failures(per_site) + dist_check_failures(per_site) + segmented_check_failures(per_site) +
-           radix64_check_failures(per_site) + radix16_check_failures(per_site) + segmented16_check_failures(per_site);
+           radix64_check_failures(per_site) + radix16_check_failures(per_site) + segmented16_check_failures(per_site) +
+           segmented64_check_failures(per_site);
 }
 const char *b200sort_radix_effective_variant_name(void) { return radix_effective_variant_name(); }
 int b200sort_radix_set_skip(int enabled) { radix_set_skip(enabled); return B200SORT_OK; }

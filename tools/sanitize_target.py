@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """What compute-sanitizer runs (tools/sanitize.sh): every kernel family once at smoke sizes, each result checked
 against the oracle.  `python tools/sanitize_target.py [big | keys16 | segmented16]` -- `big` adds one 2^20-key radix sort; `keys16` runs
-only the 16-bit sorts, `segmented16` only the segmented sort of 16-bit keys."""
+only the 16-bit sorts, `segmented16` only the segmented sort of 16-bit keys,
+`segmented64` only the segmented sort of 64-bit keys."""
 import ctypes
 import os
 import sys
@@ -57,6 +58,22 @@ def segmented16_runs():
     print("  ok segmented 16-bit pairs (stable)", flush=True)
 
 
+def segmented64_runs():
+    """Segmented 64-bit keys: a ragged mix covering every size class, every order, keys and pairs, copied and in place,
+    with executed and skipped passes."""
+    import key_orders64 as ko64
+    from test_segmented64_gpu import check_all, every_class_layout, random_keys, varying_bytes
+    offs = ragged_offsets(5, total_segments=2000, big=1)
+    m = int(offs[-1])
+    for kt, desc in ko64.ORDERS:
+        check_all(random_keys(m, kt, 11 + kt + desc), offs, kt, desc, f"segmented 64-bit n={m} {kt},{desc}")
+        print(f"  ok segmented 64-bit keys and pairs n={m}, {offs.size - 1} segments, order {kt},{desc}", flush=True)
+    offs = every_class_layout(6)
+    for mask in (0x00, 0x0F, 0xF0, 0x5A, 0x81, 0xFF):
+        check_all(varying_bytes(int(offs[-1]), mask, mask).view(np.int64), offs, ko64.KEY_I64, 0, f"mask {mask:#x}")
+    print("  ok segmented 64-bit skipped-pass patterns", flush=True)
+
+
 def report_checked():
     sites = (ctypes.c_ulonglong * 16)()
     fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
@@ -73,6 +90,13 @@ if len(sys.argv) > 1 and sys.argv[1] == "keys16":      # only the 16-bit sorts, 
     sys.exit(0)
 
 
+if len(sys.argv) > 1 and sys.argv[1] == "segmented64":  # only the segmented sort of 64-bit keys
+    from test_segmented_gpu import ragged_offsets  # noqa: E402
+    segmented64_runs()
+    if L.b200sort_debug_checked_build():
+        report_checked()
+    print("SANITIZE TARGET PASSED", flush=True)
+    sys.exit(0)
 if len(sys.argv) > 1 and sys.argv[1] == "segmented16":  # only the segmented sort of 16-bit keys
     segmented16_runs()
     if L.b200sort_debug_checked_build():
