@@ -38,6 +38,9 @@
  *                               no reference counterpart: every segment (row) of 64-bit keys sorted on its own
  *                               in one call, keys only or with an int32 value, skipping the digit passes that no
  *                               segment needs
+ *   b200sort_radix_sort_indices_keys / b200sort_segmented_sort_indices_keys
+ *                               no reference counterpart: 32-bit keys sorted with their int64 positions (the
+ *                               values and indices of torch.sort), 1-D or segmented, with no index input
  *
  * The C++ symbols order_array(int*,int) / order_with_trust(int*,int) that SRM/main.cpp and
  * SRM/performanceTest.cpp link against are exported by the same library (csrc/lab_shim.cu) with
@@ -273,6 +276,37 @@ int    b200sort_segmented_pairs_keys(int key_type, int descending, const void *d
                                      void *d_ws, size_t ws_bytes, void *stream);
 /* Largest segment length served by size class c (0, 1, ...); 0 past the last class (the onesweep class, unbounded). */
 size_t b200sort_segmented_class_max(int c);
+
+/* ---- sort with indices: 32-bit keys and their int64 positions -------------------------------------------
+ * The keys of B200SORT_KEY_I32..F32 sorted in the order (key_type, descending) of b200sort_sort_keys, and beside them
+ * d_idx_out[i] = the position that d_keys_out[i] held in its segment of the input, as int64 (the index dtype of
+ * torch.sort, torch.gather and friends).  The result is the STABLE sort of (key, position) pairs in both directions:
+ * without NaN and -0.0 it equals torch.sort(x, stable=True, descending=...) in values and indices, byte for byte, and
+ * for rows torch.sort(x, dim=-1, stable=True, descending=...).  There is no index input: the first pass makes the
+ * positions as it loads the keys, they travel as int32 (d_tmp_idx: n int32 of scratch; passes may also use d_idx_out's
+ * 8n bytes as int32 scratch) and the pass that stores them for the last time writes them as int64.  Which pass that
+ * is depends on the passes skipped, which only the device knows; a final kernel covers a sort in which no pass ran
+ * (the indices are then 0..n-1) and an in-place sort whose last pass landed in scratch.  DESIGN section 4.2i.
+ * d_keys_in may equal d_keys_out (in place); otherwise d_keys_in is only read.  d_tmp_keys: n keys of scratch.
+ * Workspaces are those of the pairs sorts: b200sort_workspace_bytes(n, B200SORT_ALGO_RADIX) for the 1-D form (n >= 2),
+ * b200sort_segmented_workspace_bytes(n, num_segments) for the segmented form (n >= 1).
+ * Key type outside B200SORT_KEY_I32..F32, descending not 0/1, n or num_segments > B200SORT_MAX_N, NULL pointers with
+ * n > 0 (d_offsets: with num_segments > 0), d_idx_out not 8-byte aligned -> B200SORT_ERR_INVALID; missing, small or
+ * misaligned workspace -> B200SORT_ERR_WORKSPACE; all checked before any device work.  n == 0 returns B200SORT_OK
+ * without touching the device; the 1-D form sorts n == 1 with a memset of d_idx_out (and a copy of the key when out of
+ * place).  The 1-D form follows b200sort_radix_pairs_keys: the generic pass kernels, the same self-test gate and
+ * ballot-ranked fallback, skipped passes (b200sort_radix_set_skip applies, and with skipping off n = 2^30 ->
+ * B200SORT_ERR_INVALID).  The segmented form follows b200sort_segmented_pairs_keys: offsets as there, clamped on the
+ * device.  A call enqueues the same kernels for every n >= 2 and every distribution (1-D: one memset and six kernels,
+ * five with skipping off; segmented: those of b200sort_segmented_pairs_keys), never synchronises and never reads
+ * device results on the host, so it can be captured in a CUDA graph once b200sort_device_check() has run. */
+int    b200sort_radix_sort_indices_keys(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                        int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                        void *d_ws, size_t ws_bytes, void *stream);
+int    b200sort_segmented_sort_indices_keys(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                            int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                            const int32_t *d_offsets, size_t num_segments,
+                                            void *d_ws, size_t ws_bytes, void *stream);
 
 /* ---- segmented sort of 16-bit keys: int16, uint16, float16 and bfloat16 -----------------------------------
  * The segmented sort above on the 2-byte keys of b200sort_sort_keys16: segment i = keys[d_offsets[i] ..

@@ -473,6 +473,29 @@ int b200sort_radix_pairs_keys(int key_type, int descending, const void *d_keys_i
                             static_cast<cudaStream_t>(stream), i32_asc ? nullptr : &order);
 }
 
+// Argument checks of the sort with indices that come before the workspace, in the order and with the statuses of
+// b200sort_radix_pairs_keys, every pointer required with n > 0, plus the 8-byte alignment of the index output.
+static int check_indices_args(int key_type, int descending, SignXor *order, size_t n, const void *keys_in,
+                              const void *keys_out, const int64_t *idx_out, const void *tmp_keys, const int32_t *tmp_idx) {
+    if (!key_order(key_type, descending, order)) return B200SORT_ERR_INVALID;
+    if (n > B200SORT_MAX_N) return B200SORT_ERR_INVALID;
+    if (n > 0 && (keys_in == nullptr || keys_out == nullptr || idx_out == nullptr || tmp_keys == nullptr ||
+                  tmp_idx == nullptr))
+        return B200SORT_ERR_INVALID;
+    if ((reinterpret_cast<uintptr_t>(idx_out) & 7) != 0) return B200SORT_ERR_INVALID;
+    return B200SORT_OK;
+}
+
+int b200sort_radix_sort_indices_keys(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                     int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                     void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor order;
+    B200_TRY(check_indices_args(key_type, descending, &order, n, d_keys_in, d_keys_out, d_idx_out, d_tmp_keys, d_tmp_idx));
+    return radix_sort_indices(static_cast<const int32_t *>(d_keys_in), static_cast<int32_t *>(d_keys_out),
+                              static_cast<int32_t *>(d_tmp_keys), d_idx_out, d_tmp_idx, n, d_ws, ws_bytes,
+                              static_cast<cudaStream_t>(stream), order);
+}
+
 // Argument checks of the 64-bit entry points that come before the workspace, in the order and with the statuses of
 // b200sort_sort_keys, plus the 8-byte alignment of the key pointers.
 static int check_keys64_args(int key_type, int descending, SignXor64 *order, size_t n, const void *in, const void *out,
@@ -587,6 +610,19 @@ int b200sort_segmented_pairs_keys(int key_type, int descending, const void *d_ke
     return segmented_sort(static_cast<const int32_t *>(d_keys_in), static_cast<int32_t *>(d_keys_out),
                           static_cast<int32_t *>(d_tmp_keys), d_vals_in, d_vals_out, d_tmp_vals, n, d_offsets,
                           num_segments, d_ws, static_cast<cudaStream_t>(stream), order);
+}
+
+int b200sort_segmented_sort_indices_keys(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                         int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                         const int32_t *d_offsets, size_t num_segments,
+                                         void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor order;
+    B200_TRY(check_indices_args(key_type, descending, &order, n, d_keys_in, d_keys_out, d_idx_out, d_tmp_keys, d_tmp_idx));
+    B200_TRY(check_segmented_args(n, d_offsets, num_segments, d_ws, ws_bytes));
+    if (n == 0) return B200SORT_OK;
+    return segmented_sort_indices(static_cast<const int32_t *>(d_keys_in), static_cast<int32_t *>(d_keys_out),
+                                  static_cast<int32_t *>(d_tmp_keys), d_idx_out, d_tmp_idx, n, d_offsets, num_segments,
+                                  d_ws, static_cast<cudaStream_t>(stream), order);
 }
 
 // Argument checks of the 16-bit segmented entry points before the workspace: those of b200sort_segmented_sort_keys in

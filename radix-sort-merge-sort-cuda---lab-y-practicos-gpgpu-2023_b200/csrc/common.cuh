@@ -135,6 +135,9 @@ __device__ __forceinline__ int32_t ld_stream(const int32_t *p) {
 __device__ __forceinline__ void st_stream(int32_t *p, int32_t v) {
     asm volatile("st.global.L1::no_allocate.s32 [%0], %1;" :: "l"(p), "r"(v) : "memory");
 }
+__device__ __forceinline__ void st_stream_s64(int64_t *p, int64_t v) {
+    asm volatile("st.global.L1::no_allocate.s64 [%0], %1;" :: "l"(p), "l"(v) : "memory");
+}
 
 // Tile-status words of the decoupled look-back are single 32-bit words read and written at GPU
 // scope with relaxed ordering: flag and value travel together, so no fence is needed.

@@ -636,6 +636,66 @@ int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const 
     return B200SORT_OK;
 }
 
+// ---- sort with indices ------------------------------------------------------------------------------------------
+// The generic pairs pipeline with the values made on the device: histogram, four passes, one final kernel.  The
+// indices never travel as an input, and travel as int64 only when they are stored for the last time.
+template <int SAFE>
+int launch_indices_passes(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, int32_t *idx_out32, int32_t *tmp_idx,
+                          size_t n, RadixControl *ctl, uint32_t *const *status, cudaStream_t s) {
+    constexpr size_t smem = Pipelined2Shape<10, 1, 1>::kSmemBytes;
+    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(radix_onesweep_indices_kernel<10, SAFE>),
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t tiles = div_up(n, (size_t)Pipelined2Shape<10, 1, 1>::kTile);
+    const unsigned slots = 2u * kNumSMs;
+    const unsigned grid = (unsigned)(tiles < slots ? tiles : slots);
+    for (int pass = 0; pass < kRadixPasses; ++pass) {
+        uint32_t *cur = status[pass & 1];
+        uint32_t *next = (pass + 1 < kRadixPasses) ? status[(pass + 1) & 1] : nullptr;
+        radix_onesweep_indices_kernel<10, SAFE><<<grid, 512, smem, s>>>(d_in, d_out, d_tmp, n, pass, ctl, cur, next, 1,
+                                                                       idx_out32, tmp_idx);
+        B200_LAUNCH_CHECK();
+    }
+    return B200SORT_OK;
+}
+
+int radix_sort_indices(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx, size_t n,
+                       void *d_ws, size_t ws_bytes, cudaStream_t s, const SignXor &order) {
+    if (n == 0) return B200SORT_OK;
+    if (n == 1) {
+        if (d_in != d_out) B200_CUDA_TRY(cudaMemcpyAsync(d_out, d_in, sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+        B200_CUDA_TRY(cudaMemsetAsync(idx_out, 0, sizeof(int64_t), s));
+        return B200SORT_OK;
+    }
+    B200_TRY(check_ws(d_ws, ws_bytes, n));
+    if (n >= ((size_t)1 << 30) && !g_skip_enabled.load()) return B200SORT_ERR_INVALID;   // see radix_sort_impl
+    const bool safe = !atomic_order_ok();
+    B200_TRY(ensure_hist_attr(true));
+    auto *ctl = static_cast<RadixControl *>(d_ws);
+    const size_t tiles = div_up(n, (size_t)Pipelined2Shape<10, 1, 1>::kTile);
+    const size_t rows = tiles + div_up(tiles, (size_t)kLookGroup);
+    uint32_t *status[2];
+    status[0] = reinterpret_cast<uint32_t *>(static_cast<unsigned char *>(d_ws) + kRadixControlBytes);
+    status[1] = status[0] + rows * kRadixBins;
+    const int skip = g_skip_enabled.load();
+    const uint32_t in_place = (d_in == d_out) ? 1u : 0u;
+    auto *idx32 = reinterpret_cast<int32_t *>(idx_out);
+
+    B200_CUDA_TRY(cudaMemsetAsync(ctl, 0, kRadixZeroBytes, s));
+    radix_histogram_keys_kernel<<<hist_grid(n), kHistThreads, kHistSmemBytes, s>>>(d_in, n, ctl, status[0], rows * kRadixBins,
+                                                                                   (uint32_t)skip, in_place, order);
+    B200_LAUNCH_CHECK();
+    if (safe) B200_TRY(launch_indices_passes<1>(d_in, d_out, d_tmp, idx32, tmp_idx, n, ctl, status, s));
+    else      B200_TRY(launch_indices_passes<0>(d_in, d_out, d_tmp, idx32, tmp_idx, n, ctl, status, s));
+    if (skip) {
+        // With skipping off all four passes run, and the fourth stores the int64 indices into out.
+        const size_t blocks = div_up(n, 256);
+        const unsigned g2 = (unsigned)(blocks < (size_t)kNumSMs * 8 ? blocks : (size_t)kNumSMs * 8);
+        radix_final_indices_kernel<<<g2, 256, 0, s>>>(d_in, d_out, d_tmp, idx_out, tmp_idx, n, ctl);
+        B200_LAUNCH_CHECK();
+    }
+    return B200SORT_OK;
+}
+
 int radix_sort_timed(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, void *d_ws,
                      size_t ws_bytes, cudaStream_t s, float *ms) {
     return radix_sort_impl(d_in, d_out, d_tmp, n, d_ws, ws_bytes, s, ms);

@@ -53,6 +53,11 @@ int radix_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, size_t n, vo
 int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const int32_t *v_in, int32_t *v_out,
                      int32_t *v_tmp, size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s,
                      const SignXor *order = nullptr);
+// Sort with indices: keys in any order of `order`, stable, and idx_out[i] = the input position of out[i], as int64.
+// No index input: the passes make the positions and widen them when they store them for the last time (the pass
+// body's IDX flag).  tmp_idx holds n int32.  d_in may equal d_out.  Same workspace as radix_sort.
+int radix_sort_indices(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx, size_t n,
+                       void *d_ws, size_t ws_bytes, cudaStream_t s, const SignXor &order);
 // The same sort with the key count taken from DEVICE memory (*d_n <= n_max, read by the kernels when they run):
 // lets a caller whose n is produced by an earlier kernel (the multi-GPU exchange) enqueue the sort without a
 // host synchronisation.  Grids, workspace and status rows are sized for n_max.

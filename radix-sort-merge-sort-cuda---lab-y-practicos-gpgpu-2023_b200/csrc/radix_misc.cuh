@@ -29,6 +29,29 @@ radix_final_copy_kernel(const int32_t *in_buf, int32_t *out_buf, const int32_t *
     }
 }
 
+// The final step of the sort with indices (radix_sort_indices), in place of the final copy.  Keys: the final copy's
+// plan.  Indices, which only the executed passes wrote:
+//   no pass executed (one bin held every key in every pass): the sort is the identity, the indices are 0..n-1;
+//   the last executed pass landed in tmp (in place, an odd number of passes): widen tmp_idx -> out_idx;
+//   else the last executed pass stored them as int64 already.
+__global__ void __launch_bounds__(256)
+radix_final_indices_kernel(const int32_t *in_buf, int32_t *out_buf, const int32_t *tmp_buf, int64_t *out_idx,
+                           const int32_t *tmp_idx, size_t n, const RadixControl *ctl)
+{
+    const uint32_t sel = ctl->final_copy;
+    uint32_t executed = 0;
+    for (int p = 0; p < kRadixPasses; ++p) executed += ctl->skip[p] ? 0u : 1u;
+    if (sel == 0 && executed != 0) return;
+    const int32_t *src = (sel == kSelIn) ? in_buf : tmp_buf;
+    const bool copy_keys = sel != 0 && src != out_buf;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    B200_CHECK((reinterpret_cast<uintptr_t>(out_idx) & 7) == 0);
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        if (copy_keys) out_buf[i] = src[i];
+        out_idx[i] = executed == 0 ? (int64_t)i : (int64_t)tmp_idx[i];
+    }
+}
+
 // Self-test behind kRankAdd: that mode is stable only if same-address shared-memory atomics issued by one
 // warp instruction are resolved in lane order.  PTX does not promise that; every B200 tried does it
 // (tools/atomic_order_probe.cu: 245 M same-address pairs, 0 violations).  The library checks it once per

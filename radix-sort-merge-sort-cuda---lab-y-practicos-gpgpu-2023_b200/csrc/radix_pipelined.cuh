@@ -376,8 +376,11 @@ struct Pipelined2Shape {
 //        radix_sort_devn) instead of the kernel argument.  A separate instantiation: as a run-time switch it cost
 //        the default kernel 64 bytes of spills and 4 % (0.696 -> 0.726 ms per pass).
 // KEYS = 1: any key order (RadixControl::key_neg / key_pos / key_pad); 0: int32 ascending.
+// IDX  = 1 (with KV): the values are the keys' positions in the input (b200sort_radix_sort_indices_keys).  The pass that
+//        reads the input makes them instead of loading them; the last executed pass, when it writes out, stores them as
+//        int64 into out_vals; every other pass moves them as int32 (in out_vals' first 4n bytes when it writes out).
 template <int IPT, int TIMING, int SPLIT, int PACK, int KV, int EG = 0, int OVL = 0, int LATE = 0, int SAFE = 0, int PFW = 0, int DEVN = 0,
-          int KEYS = 0>
+          int KEYS = 0, int IDX = 0>
 __device__ __forceinline__ void
 radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n,
                                int pass, RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next,
@@ -391,6 +394,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
     static_assert(kTile + 64 < 65536, "PACK keeps 16-bit positions");
     static_assert(!(OVL && SPLIT), "OVL restructures the unsplit resolve");
     static_assert(!PFW || (!SPLIT && !OVL && !EG), "the prefetched look-back is written for the unsplit resolve");
+    static_assert(!IDX || KV, "the indices ride as values");
 
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint32_t *s_table  = reinterpret_cast<uint32_t *>(smem_raw);                      // [kRows][256]
@@ -412,10 +416,18 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
         s_misc[20] = n32;
         s_misc[21] = (uint32_t)(((size_t)n32 + kTile - 1) / kTile);
         if (KEYS && SAFE) s_misc[22] = flips_of(ctl->key_neg, ctl->key_pos, pass * kRadixBits);
+        if constexpr (IDX != 0) {
+            // bit 0: this pass reads the input, so it makes the indices; bit 1: it is the last pass the plan executes
+            // and it writes out, so it stores them as int64.  Only the device knows the plan.
+            uint32_t last = 1;
+            for (int q = pass + 1; q < kRadixPasses; ++q) last &= ctl->skip[q];
+            s_misc[23] = (ctl->src_sel[pass] == kSelIn ? 1u : 0u) | ((last && ctl->dst_sel[pass] == kSelOut) ? 2u : 0u);
+        }
     }
     __syncthreads();
     auto n_f = [&]() -> size_t { return DEVN ? (size_t)reinterpret_cast<volatile uint32_t *>(s_misc)[20] : n; };
     auto tiles_f = [&]() -> size_t { return (size_t)reinterpret_cast<volatile uint32_t *>(s_misc)[21]; };
+    auto idx_mode = [&]() -> uint32_t { return reinterpret_cast<volatile uint32_t *>(s_misc)[23]; };
 
     const int32_t *in = in_buf;
     int32_t *out = out_buf;
@@ -480,12 +492,30 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
             for (int i = 0; i < IPT; ++i)
                 key[i] = (wofs + i * 32 < valid) ? ld_stream(src + i * 32) : (KEYS ? (int32_t)ctl->key_pad : 0x7FFFFFFF);
         }
+        if constexpr (IDX != 0) {
+            if (idx_mode() & 1u) {
+#pragma unroll
+                for (int i = 0; i < IPT; ++i) val[i] = (int32_t)(tile_base + wofs + i * 32);
+                return;
+            }
+        }
         if (KV) {
             const int32_t *vsrc = vin + tile_base + wofs;
 #pragma unroll
             for (int i = 0; i < (KV ? IPT : 0); ++i)
                 val[i] = (wofs + i * 32 < valid) ? ld_stream(vsrc + i * 32) : 0;
         }
+    };
+    auto store_val = [&](size_t dst, int32_t v) {
+        if constexpr (IDX != 0) {
+            if (idx_mode() & 2u) {
+                int64_t *wide = reinterpret_cast<int64_t *>(vout);
+                B200_CHECK((reinterpret_cast<uintptr_t>(wide) & 7) == 0);
+                st_stream_s64(wide + dst, (int64_t)v);
+                return;
+            }
+        }
+        if (KV) st_stream(vout + dst, v);
     };
     auto write_tile = [&](uint32_t t, int buf) {
         const size_t tile_base = (size_t)t * kTile;
@@ -501,7 +531,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
                 const size_t dst = (size_t)(uint32_t)(go[dig(k)] + p);
                 B200_CHECK_AT(2, dst < n_f());
                 st_stream(out + dst, k);
-                if (KV) st_stream(vout + dst, sv[p]);
+                store_val(dst, sv[p]);
             }
         } else {
 #pragma unroll
@@ -512,7 +542,7 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
                     const size_t dst = (size_t)(uint32_t)(go[dig(k)] + p);
                     B200_CHECK_AT(2, dst < n_f());
                     st_stream(out + dst, k);
-                    if (KV) st_stream(vout + dst, sv[p]);
+                    store_val(dst, sv[p]);
                 }
             }
         }
@@ -816,7 +846,8 @@ radix_onesweep_pipelined2_body(const int32_t *in_buf, int32_t *out_buf, int32_t 
                     const uint32_t bytes = (uint32_t)((left < (size_t)kTile * 4 ? left : (size_t)kTile * 4) & ~(size_t)15);
                     if (bytes > 0) {
                         bulk_prefetch_l2(reinterpret_cast<const void *>(reinterpret_cast<uintptr_t>(in + t_far * kTile) & ~(uintptr_t)15), bytes);
-                        if (KV) bulk_prefetch_l2(reinterpret_cast<const void *>(reinterpret_cast<uintptr_t>(vin + t_far * kTile) & ~(uintptr_t)15), bytes);
+                        if (KV && !(IDX && (idx_mode() & 1u)))    // made indices have nothing to prefetch
+                            bulk_prefetch_l2(reinterpret_cast<const void *>(reinterpret_cast<uintptr_t>(vin + t_far * kTile) & ~(uintptr_t)15), bytes);
                     }
                 }
             }
@@ -917,6 +948,18 @@ radix_onesweep_pairs_kernel(const int32_t *in_buf, int32_t *out_buf, int32_t *tm
 {
     radix_onesweep_pipelined2_body<IPT, 0, 0, 1, 1, 0, 0, 1, SAFE, 0, 0, KEYS>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur,
                                                     status_next, follow_plan, in_vals, out_vals, tmp_vals);
+}
+
+// Sort with indices: the generic pairs pass whose values are the keys' input positions (IDX above).  out_idx is the
+// int64 index output viewed as int32; tmp_idx holds n int32.
+template <int IPT, int SAFE = 0>
+__global__ void __launch_bounds__(512, 2)
+radix_onesweep_indices_kernel(const int32_t *in_buf, int32_t *out_buf, int32_t *tmp_buf, size_t n,
+                              int pass, RadixControl *ctl, uint32_t *status_cur, uint32_t *status_next,
+                              int follow_plan, int32_t *out_idx, int32_t *tmp_idx)
+{
+    radix_onesweep_pipelined2_body<IPT, 0, 0, 1, 1, 0, 0, 1, SAFE, 0, 0, 1, 1>(in_buf, out_buf, tmp_buf, n, pass, ctl, status_cur,
+                                                    status_next, follow_plan, nullptr, out_idx, tmp_idx);
 }
 
 }  // namespace b200sort

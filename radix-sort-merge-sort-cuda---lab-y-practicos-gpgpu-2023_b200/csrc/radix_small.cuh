@@ -25,7 +25,8 @@ constexpr size_t small_smem_bytes(int threads, int ipt, int vals) {
 }
 
 // KEYS = 1: any key order, `order` = its masks; 0: int32 ascending.  THREADS >= 256 (the digit scan).
-// VALS = 1: vin[i] moves with in[i] (stable).  SAFE = 1: ranks from ballots instead of lane-ordered atomics.
+// VALS = 1: vin[i] moves with in[i] (stable); 2: the values are the positions 0..n-1, made here (vin is not read), and
+// vout is an int64 output viewed as int32.  SAFE = 1: ranks from ballots instead of lane-ordered atomics.
 // SKIP_PAD = 1: the slots past n are neither ranked nor moved.  They would stay last anyway, but ranking them sends
 // every padded lane of a warp to the same counter (digit 255) in every pass: with a short segment in a large tile
 // that contended atomicAdd is most of the work.
@@ -48,7 +49,9 @@ __device__ __forceinline__ void radix_small_body(const int32_t *in, int32_t *out
 
     const int32_t pad_key = KEYS ? (int32_t)key_of_last_image(order) : 0x7FFFFFFF;
     for (uint32_t i = tid; i < (uint32_t)kTile; i += THREADS) s_buf[i] = (i < n) ? in[i] : pad_key;
-    if constexpr (VALS != 0)
+    if constexpr (VALS == 2)
+        for (uint32_t i = tid; i < n; i += THREADS) s_vbuf[i] = (int32_t)i;
+    else if constexpr (VALS != 0)
         for (uint32_t i = tid; i < n; i += THREADS) s_vbuf[i] = vin[i];
     __syncthreads();
 
@@ -127,7 +130,12 @@ __device__ __forceinline__ void radix_small_body(const int32_t *in, int32_t *out
     }
     const int32_t *res = s_buf + cur * kTile;
     for (uint32_t i = tid; i < n; i += THREADS) out[i] = res[i];
-    if constexpr (VALS != 0) {
+    if constexpr (VALS == 2) {
+        const int32_t *vres = s_vbuf + cur * kTile;
+        int64_t *wide = reinterpret_cast<int64_t *>(vout);
+        B200_CHECK((reinterpret_cast<uintptr_t>(wide) & 7) == 0);
+        for (uint32_t i = tid; i < n; i += THREADS) wide[i] = vres[i];
+    } else if constexpr (VALS != 0) {
         const int32_t *vres = s_vbuf + cur * kTile;
         for (uint32_t i = tid; i < n; i += THREADS) vout[i] = vres[i];
     }

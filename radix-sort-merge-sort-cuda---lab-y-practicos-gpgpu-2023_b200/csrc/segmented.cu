@@ -10,6 +10,9 @@
 //   s4  seg_warp_kernel         class 1: a warp per segment
 //   s5  seg_small_kernel x2     classes 2 and 3: a CTA per segment, radix_small_body
 //
+// VALS: 0 keys only, 1 a 32-bit value beside every key, kValsIdx the key's position in its segment (sort with
+// indices): made where the key is first loaded and stored as int64 into vout where it is stored for the last time.
+//
 // The onesweep passes and the small-segment CTAs rank with lane-ordered shared-memory atomics like the 1-D kernels,
 // behind the same self-test (radix_atomic_order_ok); SAFE = 1 is their ballot-ranked form.
 #include "segmented.cuh"
@@ -30,6 +33,7 @@ size_t segmented_class_max(int c) {
     }
 }
 
+constexpr int kValsIdx = 2;
 constexpr int kSegWarps = kSegThreads / 32;
 constexpr int kWarpSegMax = (int)kSegMax1;            // 128
 constexpr int kWarpSegIpt = kWarpSegMax / 32;
@@ -80,9 +84,10 @@ __device__ __forceinline__ uint32_t seg_image(int32_t k, SignXor order) {
 }
 
 // ---- s0 -------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-seg_classify_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
-                    const int32_t *offsets, uint32_t num_segments, SegControl *ctl, SegLists lists, uint32_t *hist)
+template <int IDX>
+__device__ __forceinline__ void
+seg_classify_body(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
+                  const int32_t *offsets, uint32_t num_segments, SegControl *ctl, SegLists lists, uint32_t *hist)
 {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < num_segments; i += gridDim.x * blockDim.x) {
         const int32_t o0 = offsets[i], o1 = offsets[i + 1];
@@ -90,7 +95,14 @@ seg_classify_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t
         const uint32_t e = o1 < (int32_t)b ? b : ((uint32_t)o1 > n ? n : (uint32_t)o1);
         const uint32_t len = e - b;
         if (len == 1 && in != out) out[b] = in[b];
-        if (len == 1 && vin != nullptr && vin != vout) vout[b] = vin[b];
+        if constexpr (IDX != 0) {
+            if (len == 1) {
+                B200_CHECK((reinterpret_cast<uintptr_t>(vout) & 7) == 0);
+                reinterpret_cast<int64_t *>(vout)[b] = 0;
+            }
+        } else if (len == 1 && vin != nullptr && vin != vout) {
+            vout[b] = vin[b];
+        }
         // class c - 1; 4 = nothing to sort.  One atomicAdd per class and warp: with millions of short segments,
         // one per segment serialises on the four counters.
         const int c = len <= kSegMax0 ? 4 : len <= kSegMax1 ? 0 : len <= kSegMax2 ? 1 : len <= kSegMax3 ? 2 : 3;
@@ -111,6 +123,19 @@ seg_classify_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t
             for (int w = 0; w < kRadixPasses * kRadixBins / 4; ++w) h[w] = make_uint4(0, 0, 0, 0);
         }
     }
+}
+__global__ void __launch_bounds__(256)
+seg_classify_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
+                    const int32_t *offsets, uint32_t num_segments, SegControl *ctl, SegLists lists, uint32_t *hist)
+{
+    seg_classify_body<0>(in, out, vin, vout, n, offsets, num_segments, ctl, lists, hist);
+}
+// Sort with indices: a segment of one key gets index 0 (vout is the int64 index output viewed as int32).
+__global__ void __launch_bounds__(256)
+seg_classify_indices_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
+                            const int32_t *offsets, uint32_t num_segments, SegControl *ctl, SegLists lists, uint32_t *hist)
+{
+    seg_classify_body<1>(in, out, vin, vout, n, offsets, num_segments, ctl, lists, hist);
 }
 
 // ---- s1 -------------------------------------------------------------------------------------------------------------
@@ -219,6 +244,9 @@ struct SegPassSmem {
 // tiles OF ITS SEGMENT until an inclusive count, and writes key i of digit d to
 //   segment begin + segment base[d] + (keys of digit d in earlier tiles of the segment) + tile-local rank.
 // Buffers: pass 0 reads in, passes 0 and 2 write tmp, 1 and 3 write out: four passes land in out.
+// VALS = kValsIdx: pass 0 makes the indices, pass 3 stores them as int64 into vout, and pass 1 leaves them as int32 in
+// the first half of the segment's own int64 range of vout (vout[2 * begin + pos]).  So no pass writes into another
+// segment's part of the index output, which the other kernels of the call fill in any order.
 template <int VALS, int SAFE>
 __global__ void __launch_bounds__(kSegThreads, 2)
 seg_onesweep_kernel(const int32_t *in, int32_t *out, int32_t *tmp, const int32_t *vin, int32_t *vout, int32_t *vtmp,
@@ -267,7 +295,13 @@ seg_onesweep_kernel(const int32_t *in, int32_t *out, int32_t *tmp, const int32_t
         for (int i = 0; i < kSegIpt; ++i) {
             const uint32_t at = wofs + i * 32;                // warp-striped: tile order = memory order
             key[i] = at < valid ? src[begin + start + at] : pad_key;
-            if constexpr (VALS != 0) val[i] = at < valid ? vsrc[begin + start + at] : 0;
+            if constexpr (VALS == kValsIdx) {
+                if (pass == 0) val[i] = (int32_t)(start + at);
+                else if (pass & 1) val[i] = at < valid ? vtmp[begin + start + at] : 0;
+                else val[i] = at < valid ? vout[2 * (size_t)begin + start + at] : 0;
+            } else if constexpr (VALS != 0) {
+                val[i] = at < valid ? vsrc[begin + start + at] : 0;
+            }
         }
 #pragma unroll
         for (int i = 0; i < kSegIpt; ++i) {
@@ -329,7 +363,18 @@ seg_onesweep_kernel(const int32_t *in, int32_t *out, int32_t *tmp, const int32_t
             B200_CHECK_AT(15, pos < len);
             if (pos < len) {                                   // only malformed offsets fail this
                 dst[begin + pos] = kk;
-                if constexpr (VALS != 0) vdst[begin + pos] = sm.vals[i];
+                if constexpr (VALS == kValsIdx) {
+                    if (pass == kRadixPasses - 1) {
+                        B200_CHECK((reinterpret_cast<uintptr_t>(vout) & 7) == 0);
+                        reinterpret_cast<int64_t *>(vout)[begin + pos] = sm.vals[i];
+                    } else if (pass & 1) {
+                        vout[2 * (size_t)begin + pos] = sm.vals[i];
+                    } else {
+                        vtmp[begin + pos] = sm.vals[i];
+                    }
+                } else if constexpr (VALS != 0) {
+                    vdst[begin + pos] = sm.vals[i];
+                }
             }
         }
         __syncthreads();                                       // shared memory free for the next tile
@@ -357,7 +402,8 @@ seg_warp_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *vo
         for (int q = 0; q < kWarpSegIpt; ++q) {
             const uint32_t i = lane + 32 * q;
             key[q] = i < len ? in[seg.x + i] : 0;
-            if constexpr (VALS != 0) val[q] = i < len ? vin[seg.x + i] : 0;
+            if constexpr (VALS == kValsIdx) val[q] = (int32_t)i;
+            else if constexpr (VALS != 0) val[q] = i < len ? vin[seg.x + i] : 0;
             img[q] = seg_image(key[q], order);
             pos[q] = 0;
             if (i < len) img_s[i] = img[q];
@@ -372,7 +418,13 @@ seg_warp_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *vo
         for (int q = 0; q < kWarpSegIpt; ++q) {
             if (lane + 32 * q < len) {
                 out[seg.x + pos[q]] = key[q];
-                if constexpr (VALS != 0) vout[seg.x + pos[q]] = val[q];
+                if constexpr (VALS == kValsIdx) {
+                    B200_CHECK_AT(15, pos[q] < len);
+                    B200_CHECK((reinterpret_cast<uintptr_t>(vout) & 7) == 0);
+                    reinterpret_cast<int64_t *>(vout)[seg.x + pos[q]] = val[q];
+                } else if constexpr (VALS != 0) {
+                    vout[seg.x + pos[q]] = val[q];
+                }
             }
         }
         __syncwarp();                                          // img_s free for the warp's next segment
@@ -388,8 +440,12 @@ seg_small_kernel(const int32_t *in, int32_t *out, const int32_t *vin, int32_t *v
     const uint32_t count = ctl->count[c] < cap ? ctl->count[c] : cap;
     for (uint32_t s = blockIdx.x; s < count; s += gridDim.x) {
         const uint2 seg = list[s];
-        radix_small_body<1, THREADS, IPT, VALS, SAFE, 1>(in + seg.x, out + seg.x, seg.y - seg.x, order,
-                                                      VALS ? vin + seg.x : nullptr, VALS ? vout + seg.x : nullptr);
+        if constexpr (VALS == kValsIdx)
+            radix_small_body<1, THREADS, IPT, VALS, SAFE, 1>(in + seg.x, out + seg.x, seg.y - seg.x, order, nullptr,
+                                                          reinterpret_cast<int32_t *>(reinterpret_cast<int64_t *>(vout) + seg.x));
+        else
+            radix_small_body<1, THREADS, IPT, VALS, SAFE, 1>(in + seg.x, out + seg.x, seg.y - seg.x, order,
+                                                          VALS ? vin + seg.x : nullptr, VALS ? vout + seg.x : nullptr);
         __syncthreads();                                       // shared memory free for the next segment
     }
 }
@@ -429,7 +485,7 @@ int seg_sort_impl(const int32_t *in, int32_t *out, int32_t *tmp, const int32_t *
     const uint32_t cap_large = (uint32_t)L.cap[3];
 
     B200_CUDA_TRY(cudaMemsetAsync(ctl, 0, sizeof(SegControl), s));
-    seg_classify_kernel<<<grid_of(div_up(S, 256), (size_t)kNumSMs * 8), 256, 0, s>>>(
+    (VALS == kValsIdx ? seg_classify_indices_kernel : seg_classify_kernel)<<<grid_of(div_up(S, 256), (size_t)kNumSMs * 8), 256, 0, s>>>(
         in, out, vin, vout, (uint32_t)n, offsets, (uint32_t)S, ctl, lists, hist);
     B200_LAUNCH_CHECK();
     seg_tile_plan_kernel<<<1, kPlanThreads, 0, s>>>(ctl, lists.list[3], cap_large, prefix, (uint32_t)L.rows);
@@ -467,6 +523,16 @@ int segmented_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const in
                     : seg_sort_impl<0, 0>(d_in, d_out, d_tmp, nullptr, nullptr, nullptr, n, d_offsets, num_segments, d_ws, s, order);
     return safe ? seg_sort_impl<1, 1>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, d_offsets, num_segments, d_ws, s, order)
                 : seg_sort_impl<1, 0>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, d_offsets, num_segments, d_ws, s, order);
+}
+
+int segmented_sort_indices(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx,
+                           size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws, cudaStream_t s,
+                           SignXor order) {
+    if (num_segments == 0) return B200SORT_OK;
+    auto *idx32 = reinterpret_cast<int32_t *>(idx_out);
+    return radix_atomic_order_ok()
+               ? seg_sort_impl<kValsIdx, 0>(d_in, d_out, d_tmp, nullptr, idx32, tmp_idx, n, d_offsets, num_segments, d_ws, s, order)
+               : seg_sort_impl<kValsIdx, 1>(d_in, d_out, d_tmp, nullptr, idx32, tmp_idx, n, d_offsets, num_segments, d_ws, s, order);
 }
 
 unsigned long long segmented_check_failures(unsigned long long *per_site) { return tu_check_failures(per_site); }

@@ -23,6 +23,11 @@ size_t segmented_workspace_bytes(size_t n, size_t num_segments);
 int segmented_sort(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const int32_t *v_in, int32_t *v_out,
                    int32_t *v_tmp, size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws,
                    cudaStream_t s, SignXor order);
+// Sort with indices: idx_out[i] = position of out[i] inside its segment, as int64 (no index input).  tmp_idx holds n
+// int32.  Checked by the caller like segmented_sort.
+int segmented_sort_indices(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx,
+                           size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws, cudaStream_t s,
+                           SignXor order);
 unsigned long long segmented_check_failures(unsigned long long *per_site);
 
 }  // namespace b200sort

@@ -1,5 +1,5 @@
 """Sorting torch tensors of int32, uint32 or float32 keys, ascending or descending (b200sort_sort_keys,
-b200sort_radix_pairs_keys in include/b200sort.h).
+b200sort_radix_pairs_keys, b200sort_radix_sort_indices_keys in include/b200sort.h).
 
 float32 keys are ordered by IEEE-754 totalOrder on their bit patterns:
 -NaN < -inf < negatives < -0.0 < +0.0 < positives < +inf < +NaN, NaNs of one sign by payload.  That is not what
@@ -70,12 +70,8 @@ def sort_by_key(keys, values, *, descending: bool = False):
 
     ``keys``: 1-D CUDA tensor of int32, uint32 or float32; ``values``: int32 of the same length on the same device.
     Equal keys keep their input order in both directions, so a descending result is not the reverse of the
-    ascending one.  The inputs are left untouched.  argsort::
-
-        order = sort_by_key(x, torch.arange(n, dtype=torch.int32, device=x.device))[1]
-
-    On inputs without NaN and -0.0 this equals ``torch.sort(x, stable=True, descending=descending)``, values and
-    indices; float32 keys otherwise follow IEEE-754 totalOrder (see the module docstring).
+    ascending one.  The inputs are left untouched.  For the sorted keys with their int64 positions (what
+    ``torch.sort`` returns) call ``sort_with_indices``: it makes the positions on the device instead of reading them.
     """
     import torch
 
@@ -102,3 +98,32 @@ def sort_by_key(keys, values, *, descending: bool = False):
                                               k_out.data_ptr(), v_out.data_ptr(), k_tmp.data_ptr(), v_tmp.data_ptr(),
                                               n, ws_ptr, ws_bytes, stream))
     return k_out, v_out
+
+
+def sort_with_indices(x, *, descending: bool = False):
+    """``(values, indices)``: ``x`` sorted, and the int64 position in ``x`` of every value.
+
+    ``x``: 1-D contiguous CUDA tensor of int32, uint32 or float32; it is left untouched.  The sort is STABLE in both
+    directions (equal keys keep their input order), so on inputs without NaN and -0.0 the result equals
+    ``torch.sort(x, stable=True, descending=descending)``, values and indices, dtype for dtype; float32 keys otherwise
+    follow IEEE-754 totalOrder (see the module docstring).  No index array is read: the radix passes make the
+    positions and store them as int64 the last time they move.  Runs on ``torch.cuda.current_stream(x.device)``.
+    """
+    import torch
+
+    key_type = _key_type(torch, x)
+    _check_layout(x, "keys")
+    n = x.numel()
+    values = torch.empty_like(x)
+    indices = torch.empty(n, dtype=torch.int64, device=x.device)
+    if n == 0:
+        return values, indices
+    with torch.cuda.device(x.device):
+        k_tmp = torch.empty_like(x)
+        i_tmp = torch.empty(n, dtype=torch.int32, device=x.device)
+        ws, ws_ptr, ws_bytes = _workspace(torch, n, ALGO_RADIX, x.device)
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        check(lib().b200sort_radix_sort_indices_keys(key_type, int(bool(descending)), x.data_ptr(), values.data_ptr(),
+                                                     indices.data_ptr(), k_tmp.data_ptr(), i_tmp.data_ptr(), n,
+                                                     ws_ptr, ws_bytes, stream))
+    return values, indices

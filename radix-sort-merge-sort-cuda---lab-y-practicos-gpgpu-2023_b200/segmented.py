@@ -1,5 +1,5 @@
 """Sorting many independent segments of a torch tensor in one call (b200sort_segmented_sort_keys,
-b200sort_segmented_pairs_keys in include/b200sort.h).
+b200sort_segmented_pairs_keys, b200sort_segmented_sort_indices_keys in include/b200sort.h).
 
 Keys are int32, uint32 or float32, in the orders of ``b200sort.sort`` (float32: IEEE-754 totalOrder on the bit
 patterns, see ``keys.py``).  The number of kernel launches does not depend on the number of segments.
@@ -76,12 +76,8 @@ def segmented_sort_by_key(keys, values, offsets=None, *, descending: bool = Fals
     """``(sorted keys, values in the same order)``: a STABLE sort by key of every segment of (key, value) pairs.
 
     ``values``: int32 of ``keys``' shape on the same device.  Segments as in ``segmented_sort``.  Equal keys keep
-    their input order in both directions.  argsort of every row of a ``(B, L)`` tensor ``x``::
-
-        values = torch.arange(L, dtype=torch.int32, device=x.device).repeat(B).view(B, L)
-        indices = segmented_sort_by_key(x, values, descending=True)[1]
-
-    Without NaN and -0.0 this equals ``torch.sort(x, dim=-1, stable=True, descending=...)``, values and indices.
+    their input order in both directions.  For every row's sorted keys with their int64 column indices (what
+    ``torch.sort(x, dim=-1)`` returns) call ``segmented_sort_with_indices``: it makes the indices on the device.
     """
     import torch
 
@@ -106,3 +102,34 @@ def segmented_sort_by_key(keys, values, offsets=None, *, descending: bool = Fals
                                                   k_out.data_ptr(), v_out.data_ptr(), k_tmp.data_ptr(), v_tmp.data_ptr(),
                                                   n, offs.data_ptr(), segments, ws_ptr, ws_bytes, stream))
     return k_out, v_out
+
+
+def segmented_sort_with_indices(keys, offsets=None, *, descending: bool = False):
+    """``(values, indices)``: every segment of ``keys`` sorted on its own, and the int64 position of every value
+    inside its segment.
+
+    Segments as in ``segmented_sort``: the rows of a 2-D contiguous ``keys``, or the ``offsets`` ranges of a 1-D one.
+    ``indices`` has ``keys``' shape; for rows it holds column indices, for offsets ``i - offsets[s]``.  ``keys`` is
+    left untouched.  The sort is STABLE in both directions, so without NaN and -0.0 rows give exactly
+    ``torch.sort(keys, dim=-1, stable=True, descending=descending)``, values and indices, dtype for dtype.  No index
+    array is read: the kernels make the positions and store them as int64 the last time they move.  Runs on
+    ``torch.cuda.current_stream(keys.device)``.
+    """
+    import torch
+
+    key_type = _key_type(torch, keys)
+    n, offs, segments = _segments(torch, keys, offsets)
+    values = torch.empty_like(keys)
+    indices = torch.empty(keys.shape, dtype=torch.int64, device=keys.device)
+    if n == 0:
+        return values, indices
+    with torch.cuda.device(keys.device):
+        k_tmp = torch.empty_like(keys)
+        i_tmp = torch.empty(n, dtype=torch.int32, device=keys.device)
+        ws, ws_ptr, ws_bytes = _workspace(torch, n, segments, keys.device)
+        stream = torch.cuda.current_stream(keys.device).cuda_stream
+        check(lib().b200sort_segmented_sort_indices_keys(key_type, int(bool(descending)), keys.data_ptr(),
+                                                         values.data_ptr(), indices.data_ptr(), k_tmp.data_ptr(),
+                                                         i_tmp.data_ptr(), n, offs.data_ptr(), segments, ws_ptr,
+                                                         ws_bytes, stream))
+    return values, indices

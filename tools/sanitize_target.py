@@ -2,7 +2,7 @@
 """What compute-sanitizer runs (tools/sanitize.sh): every kernel family once at smoke sizes, each result checked
 against the oracle.  `python tools/sanitize_target.py [big | keys16 | segmented16]` -- `big` adds one 2^20-key radix sort; `keys16` runs
 only the 16-bit sorts, `segmented16` only the segmented sort of 16-bit keys,
-`segmented64` only the segmented sort of 64-bit keys."""
+`segmented64` only the segmented sort of 64-bit keys, `indices` only the sorts with int64 indices."""
 import ctypes
 import os
 import sys
@@ -74,6 +74,26 @@ def segmented64_runs():
     print("  ok segmented 64-bit skipped-pass patterns", flush=True)
 
 
+def indices_runs():
+    """Sort with indices: 1-D in every order and every pass plan, in place and copied, and the segmented form on a
+    ragged mix covering every size class."""
+    import digit_patterns as dp
+    import key_orders as ko
+    from test_sort_indices_gpu import check_1d, check_seg, dup_keys, ragged_offsets
+    for kt, desc in ko.ORDERS:
+        for in_place in (False, True):
+            check_1d(dup_keys((1 << 20) + 7, kt, kt + desc), kt, desc, in_place, "1-D")
+    for m in range(16):
+        S = {p for p in range(4) if m >> p & 1}
+        for in_place in (False, True):
+            check_1d(dp.with_constant_digits(70001, S, (ko.KEY_U32, m & 1), m), ko.KEY_U32, m & 1, in_place, "plan")
+    print("  ok 1-D sort with indices, every order and pass plan", flush=True)
+    offs = ragged_offsets(5, total_segments=2000, big=1)
+    for kt, desc in ko.ORDERS:
+        check_seg(dup_keys(int(offs[-1]), kt, desc), offs, kt, desc, desc == 1, "segmented")
+    print(f"  ok segmented sort with indices, n={int(offs[-1])}, {offs.size - 1} segments, every order", flush=True)
+
+
 def report_checked():
     sites = (ctypes.c_ulonglong * 16)()
     fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
@@ -93,6 +113,12 @@ if len(sys.argv) > 1 and sys.argv[1] == "keys16":      # only the 16-bit sorts, 
 if len(sys.argv) > 1 and sys.argv[1] == "segmented64":  # only the segmented sort of 64-bit keys
     from test_segmented_gpu import ragged_offsets  # noqa: E402
     segmented64_runs()
+    if L.b200sort_debug_checked_build():
+        report_checked()
+    print("SANITIZE TARGET PASSED", flush=True)
+    sys.exit(0)
+if len(sys.argv) > 1 and sys.argv[1] == "indices":      # only the sorts with int64 indices
+    indices_runs()
     if L.b200sort_debug_checked_build():
         report_checked()
     print("SANITIZE TARGET PASSED", flush=True)
