@@ -41,6 +41,8 @@
  *   b200sort_radix_sort_indices_keys / b200sort_segmented_sort_indices_keys
  *                               no reference counterpart: 32-bit keys sorted with their int64 positions (the
  *                               values and indices of torch.sort), 1-D or segmented, with no index input
+ *   b200sort_radix_sort_indices_keys16 / b200sort_segmented_sort_indices_keys16
+ *                               no reference counterpart: the same for 16-bit keys
  *
  * The C++ symbols order_array(int*,int) / order_with_trust(int*,int) that SRM/main.cpp and
  * SRM/performanceTest.cpp link against are exported by the same library (csrc/lab_shim.cu) with
@@ -345,6 +347,39 @@ int    b200sort_segmented_pairs_keys16(int key_type, int descending, const void 
                                        void *d_keys_out, int32_t *d_vals_out, void *d_tmp_keys, int32_t *d_tmp_vals,
                                        size_t n, const int32_t *d_offsets, size_t num_segments,
                                        void *d_ws, size_t ws_bytes, void *stream);
+
+/* ---- sort with indices: 16-bit keys and their int64 positions -------------------------------------------
+ * The keys of B200SORT_KEY_I16..BF16 sorted in the order (key_type, descending) of b200sort_sort_keys16 (float16 and
+ * bfloat16: IEEE-754 totalOrder on the bits), and beside them d_idx_out[i] = the position that d_keys_out[i] held in
+ * its segment of the input, as int64: the index in the array (1-D), the column (rows), i - d_offsets[s] (offsets).
+ * The result is the STABLE sort of (key, position) pairs in both directions: without NaN and -0.0 it equals
+ * torch.sort(x, stable=True, descending=...) in values and indices, byte for byte, and for rows
+ * torch.sort(x, dim=-1, stable=True, descending=...).  There is no index input: the first executed pass makes the
+ * positions as it loads the keys, they travel between the two passes as int32 in d_tmp_idx (n int32 of scratch), and
+ * the last executed pass stores them as int64.  DESIGN section 4.2j.
+ * d_keys_in may equal d_keys_out (in place); otherwise d_keys_in is only read.  d_tmp_keys: n keys of scratch.  Key
+ * pointers need only 2-byte alignment.  Workspaces are those of the 16-bit sorts: b200sort_keys16_workspace_bytes(n)
+ * for the 1-D form (n >= 2), b200sort_segmented16_workspace_bytes(n, num_segments) for the segmented form (n >= 1).
+ * Key type outside B200SORT_KEY_I16..BF16, descending not 0/1, n or num_segments > B200SORT_MAX_N, NULL pointers with
+ * n > 0 (d_offsets: with num_segments > 0), odd key pointers, d_idx_out not 8-byte aligned -> B200SORT_ERR_INVALID;
+ * missing, small or misaligned workspace -> B200SORT_ERR_WORKSPACE; all checked before any device work, in the order
+ * of b200sort_radix_pairs_keys16.  The 32-bit indices entry points reject the 16-bit key types and these reject every
+ * other type.  n == 0 returns B200SORT_OK without touching the device; the 1-D form sorts n == 1 with a memset of
+ * d_idx_out (and a copy of the key when out of place).  The 1-D form follows b200sort_radix_pairs_keys16: the same
+ * histogram and scan, its two passes with the same self-test gate and ballot-ranked fallback, skipped passes
+ * (b200sort_radix_set_skip applies, and with skipping off n = 2^30 -> B200SORT_ERR_INVALID), then one final kernel
+ * that copies the keys as the pairs sort's final copy does and writes 0..n-1 when both passes were skipped.  The
+ * segmented form follows b200sort_segmented_pairs_keys16: offsets as there, clamped on the device.  A call enqueues the
+ * same kernels for every n >= 2 and every distribution (1-D: one memset and five kernels; segmented: those of
+ * b200sort_segmented_pairs_keys16), never synchronises and never reads device results on the host, so it can be
+ * captured in a CUDA graph once b200sort_device_check() has run. */
+int    b200sort_radix_sort_indices_keys16(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                          int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                          void *d_ws, size_t ws_bytes, void *stream);
+int    b200sort_segmented_sort_indices_keys16(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                              int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                              const int32_t *d_offsets, size_t num_segments,
+                                              void *d_ws, size_t ws_bytes, void *stream);
 
 /* ---- segmented sort of 64-bit keys: int64, uint64 and float64 -------------------------------------------
  * The segmented sort above on the 8-byte keys of b200sort_sort_keys64: segment i = keys[d_offsets[i] ..

@@ -66,6 +66,8 @@ SIGNATURES = {
     "b200sort_segmented_pairs_keys64": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_radix_sort_indices_keys": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_segmented_sort_indices_keys": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_radix_sort_indices_keys16": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp]),
+    "b200sort_segmented_sort_indices_keys16": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
     "b200sort_radix_histogram_i32": (_i, [_vp, _sz, _vp, _vp]),
     "b200sort_radix_pass_i32": (_i, [_vp, _vp, _sz, _i, _vp, _sz, _vp]),
     "b200sort_block_sort_tile": (_sz, []),

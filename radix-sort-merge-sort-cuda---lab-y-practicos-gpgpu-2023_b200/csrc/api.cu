@@ -475,6 +475,7 @@ int b200sort_radix_pairs_keys(int key_type, int descending, const void *d_keys_i
 
 // Argument checks of the sort with indices that come before the workspace, in the order and with the statuses of
 // b200sort_radix_pairs_keys, every pointer required with n > 0, plus the 8-byte alignment of the index output.
+// (16-bit keys: check_indices16_args.)
 static int check_indices_args(int key_type, int descending, SignXor *order, size_t n, const void *keys_in,
                               const void *keys_out, const int64_t *idx_out, const void *tmp_keys, const int32_t *tmp_idx) {
     if (!key_order(key_type, descending, order)) return B200SORT_ERR_INVALID;
@@ -563,6 +564,29 @@ int b200sort_radix_pairs_keys16(int key_type, int descending, const void *d_keys
     return radix16_sort(static_cast<const uint16_t *>(d_keys_in), static_cast<uint16_t *>(d_keys_out),
                         static_cast<uint16_t *>(d_tmp_keys), d_vals_in, d_vals_out, d_tmp_vals, n, d_ws, ws_bytes,
                         static_cast<cudaStream_t>(stream), order);
+}
+
+// Argument checks of the 16-bit sort with indices before the workspace: those of b200sort_radix_pairs_keys16 in its
+// order and with its statuses (every pointer required with n > 0, 2-byte key pointers), plus the 8-byte alignment of
+// the index output.
+static int check_indices16_args(int key_type, int descending, SignXor16 *order, size_t n, const void *keys_in,
+                                const void *keys_out, const int64_t *idx_out, const void *tmp_keys,
+                                const int32_t *tmp_idx) {
+    B200_TRY(check_keys16_args(key_type, descending, order, n, keys_in, keys_out, tmp_keys, true));
+    if (n > 0 && (idx_out == nullptr || tmp_idx == nullptr)) return B200SORT_ERR_INVALID;
+    if ((reinterpret_cast<uintptr_t>(idx_out) & 7) != 0) return B200SORT_ERR_INVALID;
+    return B200SORT_OK;
+}
+
+int b200sort_radix_sort_indices_keys16(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                       int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                       void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor16 order;
+    B200_TRY(check_indices16_args(key_type, descending, &order, n, d_keys_in, d_keys_out, d_idx_out, d_tmp_keys,
+                                  d_tmp_idx));
+    return radix16_sort_indices(static_cast<const uint16_t *>(d_keys_in), static_cast<uint16_t *>(d_keys_out),
+                                static_cast<uint16_t *>(d_tmp_keys), d_idx_out, d_tmp_idx, n, d_ws, ws_bytes,
+                                static_cast<cudaStream_t>(stream), order);
 }
 
 // Argument checks of the segmented entry points, in the order and with the statuses of b200sort_sort_keys.
@@ -677,6 +701,20 @@ int b200sort_segmented_pairs_keys16(int key_type, int descending, const void *d_
     return segmented16_sort(static_cast<const uint16_t *>(d_keys_in), static_cast<uint16_t *>(d_keys_out),
                             static_cast<uint16_t *>(d_tmp_keys), d_vals_in, d_vals_out, d_tmp_vals, n, d_offsets,
                             num_segments, d_ws, static_cast<cudaStream_t>(stream), order);
+}
+
+int b200sort_segmented_sort_indices_keys16(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
+                                           int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
+                                           const int32_t *d_offsets, size_t num_segments,
+                                           void *d_ws, size_t ws_bytes, void *stream) {
+    SignXor16 order;
+    B200_TRY(check_indices16_args(key_type, descending, &order, n, d_keys_in, d_keys_out, d_idx_out, d_tmp_keys,
+                                  d_tmp_idx));
+    B200_TRY(check_segmented16_args(n, d_offsets, num_segments, d_ws, ws_bytes));
+    if (n == 0) return B200SORT_OK;
+    return segmented16_sort_indices(static_cast<const uint16_t *>(d_keys_in), static_cast<uint16_t *>(d_keys_out),
+                                    static_cast<uint16_t *>(d_tmp_keys), d_idx_out, d_tmp_idx, n, d_offsets,
+                                    num_segments, d_ws, static_cast<cudaStream_t>(stream), order);
 }
 
 // Argument checks of the 64-bit segmented entry points before the workspace: those of b200sort_segmented_sort_keys in

@@ -14,9 +14,12 @@
 //   r3  radix16_onesweep_kernel x2      the 64-bit sort's stable onesweep pass (radix64.cu) on 2-byte keys and
 //                                       8192-key tiles: the low byte of the image, then the high byte
 //   r4  radix16_final_copy_kernel       tmp -> out (or in -> out) when the plan did not land in out
+//   with indices (DESIGN section 4.2j): r3 as radix16_onesweep_indices_kernel, whose values are made by the first
+//   executed pass and stored as int64 by the last; r4 as radix16_final_indices_kernel, which also writes 0..n-1 when
+//   both passes were skipped
 //
-// A call enqueues one memset and the same kernels whatever n (>= 2) and the data (3 for keys, 5 for pairs), and the
-// host never reads what the device computes: the sort is stream-ordered and can be captured in a CUDA graph.
+// A call enqueues one memset and the same kernels whatever n (>= 2) and the data (3 for keys, 5 for pairs or indices),
+// and the host never reads what the device computes: the sort is stream-ordered and can be captured in a CUDA graph.
 #include "radix16.cuh"
 #include "radix.cuh"
 #include "radix_digit.cuh"
@@ -324,11 +327,17 @@ __device__ __forceinline__ uint32_t digit16(uint32_t k, int pass, SignXor16 o) {
 // radix64_onesweep_kernel on 2-byte keys (see there): tickets, {flag:2, count:30} look-back, ranks from lane-ordered
 // shared atomics (SAFE = 1: the ballot form), staging in digit order.  Slots past n in the last tile hold the key
 // whose image is 0xFFFF: digit 255 in both passes, ranked after every real key, staged at the end, never written.
-template <int IPT, int SAFE>
-__global__ void __launch_bounds__(kP16Threads, IPT <= 16 ? 2 : 1)
-radix16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const int32_t *vin, int32_t *vout,
-                        int32_t *vtmp, uint32_t n, int pass, R16Control *ctl, uint32_t *status, uint32_t *status_next,
-                        SignXor16 order, uint32_t pad_key)
+// IDX = 1: the values are the keys' input positions (b200sort_radix_sort_indices_keys16).  vin and vout are unused,
+// vtmp holds n int32 positions between the two passes and idx_out is the int64 index output.  The first executed pass
+// (pass 0, or pass 1 when pass 0 is skipped) makes the positions instead of loading them; the last executed pass
+// (pass 1, or pass 0 when pass 1 is skipped) stores them as int64 into idx_out; only when both passes execute does pass
+// 0 write them as int32 into vtmp for pass 1.  The index output is never read, so unlike the keys it does not follow
+// src_sel / dst_sel: an in-place sort with one executed pass still stores its indices directly.
+template <int IPT, int SAFE, int IDX>
+__device__ __forceinline__ void
+radix16_onesweep_body(const uint16_t *in, uint16_t *out, uint16_t *tmp, const int32_t *vin, int32_t *vout,
+                      int32_t *vtmp, uint32_t n, int pass, R16Control *ctl, uint32_t *status, uint32_t *status_next,
+                      SignXor16 order, uint32_t pad_key, int64_t *idx_out)
 {
     constexpr uint32_t kTile = kP16Threads * IPT;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -345,6 +354,11 @@ radix16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const 
     uint16_t *dst = sel_buf16<uint16_t>(ctl->dst_sel[pass], nullptr, tmp, out);
     const int32_t *vsrc = sel_buf16<const int32_t>(ctl->src_sel[pass], vin, vtmp, vout);
     int32_t *vdst = sel_buf16<int32_t>(ctl->dst_sel[pass], nullptr, vtmp, vout);
+    bool make = false, wide = false;                            // IDX: first / last executed pass
+    if constexpr (IDX != 0) {
+        make = pass == 0 || ctl->skip[0] != 0;
+        wide = pass == 1 || ctl->skip[1] != 0;
+    }
     const uint32_t *base = ctl->base[pass];
     uint32_t *wcnt = sm.cnt[warp];
     const uint32_t wofs = warp * (32 * IPT) + lane;
@@ -365,7 +379,8 @@ radix16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const 
         for (int i = 0; i < IPT; ++i) {
             const uint32_t at = wofs + i * 32;                   // warp-striped: tile order = memory order
             key[i] = at < valid ? src[start + at] : pad_key;
-            val[i] = at < valid ? vsrc[start + at] : 0;
+            if constexpr (IDX != 0) val[i] = make ? (int32_t)(start + at) : (at < valid ? vtmp[start + at] : 0);
+            else val[i] = at < valid ? vsrc[start + at] : 0;
         }
 #pragma unroll
         for (int i = 0; i < IPT; ++i) {
@@ -425,11 +440,41 @@ radix16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const 
             B200_CHECK_AT(2, pos < n);
             if (pos < n) {
                 dst[pos] = (uint16_t)k;
-                vdst[pos] = sm.vals[i];
+                if constexpr (IDX != 0) {
+                    if (wide) {
+                        B200_CHECK((reinterpret_cast<uintptr_t>(idx_out) & 7) == 0);
+                        idx_out[pos] = sm.vals[i];
+                    } else {
+                        vtmp[pos] = sm.vals[i];
+                    }
+                } else {
+                    vdst[pos] = sm.vals[i];
+                }
             }
         }
         __syncthreads();                                         // shared memory free for the next tile
     }
+}
+
+template <int IPT, int SAFE>
+__global__ void __launch_bounds__(kP16Threads, IPT <= 16 ? 2 : 1)
+radix16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const int32_t *vin, int32_t *vout,
+                        int32_t *vtmp, uint32_t n, int pass, R16Control *ctl, uint32_t *status, uint32_t *status_next,
+                        SignXor16 order, uint32_t pad_key)
+{
+    radix16_onesweep_body<IPT, SAFE, 0>(in, out, tmp, vin, vout, vtmp, n, pass, ctl, status, status_next, order,
+                                        pad_key, nullptr);
+}
+
+// The pass of the sort with indices (IDX above): tmp_idx holds n int32, idx_out is the int64 index output.
+template <int IPT, int SAFE>
+__global__ void __launch_bounds__(kP16Threads, IPT <= 16 ? 2 : 1)
+radix16_onesweep_indices_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, int32_t *tmp_idx, int64_t *idx_out,
+                                uint32_t n, int pass, R16Control *ctl, uint32_t *status, uint32_t *status_next,
+                                SignXor16 order, uint32_t pad_key)
+{
+    radix16_onesweep_body<IPT, SAFE, 1>(in, out, tmp, nullptr, nullptr, tmp_idx, n, pass, ctl, status, status_next,
+                                        order, pad_key, idx_out);
 }
 
 // ---- r4 -------------------------------------------------------------------------------------------------------------
@@ -444,6 +489,24 @@ radix16_final_copy_kernel(const uint16_t *in, uint16_t *out, const uint16_t *tmp
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         out[i] = src[i];
         vout[i] = vsrc[i];
+    }
+}
+
+// The final step of the sort with indices, in place of the final copy.  Keys: the final copy's plan.  Indices: with
+// both passes skipped (one bit pattern holds every key) the sort is the identity and they are 0..n-1; otherwise the
+// last executed pass has stored them.
+__global__ void __launch_bounds__(256)
+radix16_final_indices_kernel(const uint16_t *in, uint16_t *out, const uint16_t *tmp, int64_t *idx_out, uint32_t n,
+                             const R16Control *ctl)
+{
+    const uint32_t sel = ctl->final_copy;
+    const bool identity = ctl->skip[0] != 0 && ctl->skip[1] != 0;
+    if (sel == 0 && !identity) return;
+    const uint16_t *src = sel == kSelIn ? in : tmp;
+    B200_CHECK((reinterpret_cast<uintptr_t>(idx_out) & 7) == 0);
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        if (sel != 0) out[i] = src[i];
+        if (identity) idx_out[i] = i;
     }
 }
 
@@ -568,6 +631,61 @@ int radix16_sort(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, const i
     const size_t blocks = div_up(n, 256);
     radix16_final_copy_kernel<<<(unsigned)(blocks < (size_t)kNumSMs * 8 ? blocks : (size_t)kNumSMs * 8), 256, 0, s>>>(
         d_in, d_out, d_tmp, v_in, v_out, v_tmp, n32, ctl);
+    B200_LAUNCH_CHECK();
+    return B200SORT_OK;
+}
+
+// ---- sort with indices -------------------------------------------------------------------------------------------
+// The pairs pipeline with the values made on the device: memset, histogram, scan, two passes, one final kernel.
+template <int SAFE>
+static int launch_indices_passes(const uint16_t *in, uint16_t *out, uint16_t *tmp, int32_t *tmp_idx, int64_t *idx_out,
+                                 uint32_t n, R16Control *ctl, uint32_t *const *status, SignXor16 order, cudaStream_t s) {
+    constexpr size_t smem = sizeof(R16PassSmem<kP16Ipt>);
+    auto *fn = radix16_onesweep_indices_kernel<kP16Ipt, SAFE>;
+    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
+    const size_t tiles = div_up(n, (size_t)kP16Threads * kP16Ipt);
+    const unsigned grid = (unsigned)(tiles < 2 * (size_t)kNumSMs ? tiles : 2 * (size_t)kNumSMs);
+    const uint32_t pad = image16(0xffffu, inverse16(order));
+    for (int pass = 0; pass < 2; ++pass) {
+        fn<<<grid, kP16Threads, smem, s>>>(in, out, tmp, tmp_idx, idx_out, n, pass, ctl, status[pass],
+                                           pass == 0 ? status[1] : nullptr, order, pad);
+        B200_LAUNCH_CHECK();
+    }
+    return B200SORT_OK;
+}
+
+int radix16_sort_indices(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx,
+                         size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s, SignXor16 order) {
+    if (n == 0) return B200SORT_OK;
+    if (n == 1) {
+        if (d_in != d_out) B200_CUDA_TRY(cudaMemcpyAsync(d_out, d_in, sizeof(uint16_t), cudaMemcpyDeviceToDevice, s));
+        B200_CUDA_TRY(cudaMemsetAsync(idx_out, 0, sizeof(int64_t), s));
+        return B200SORT_OK;
+    }
+    if (d_ws == nullptr || (reinterpret_cast<uintptr_t>(d_ws) & 255) != 0 || ws_bytes < radix16_workspace_bytes(n))
+        return B200SORT_ERR_WORKSPACE;
+    const int skip = radix_skip_enabled();
+    if (n >= ((size_t)1 << 30) && !skip) return B200SORT_ERR_INVALID;   // the 30-bit status counts, see radix16_sort
+    const bool safe = !radix_atomic_order_ok();
+    auto *ctl = static_cast<R16Control *>(d_ws);
+    const size_t hgrid = h16_grid(n), rows = r16_rows(n);
+    uint32_t *part = reinterpret_cast<uint32_t *>(static_cast<unsigned char *>(d_ws) + kR16ControlBytes);
+    uint32_t *status[2];
+    status[0] = part + hgrid * kImages16;
+    status[1] = status[0] + rows * kRadixBins;
+    const uint32_t n32 = (uint32_t)n;
+
+    B200_CUDA_TRY(cudaMemsetAsync(ctl, 0, kR16ZeroBytes, s));
+    B200_TRY(launch_histogram<kH16Runs>(d_in, n32, part, (unsigned)hgrid, ctl, status[0], rows * kRadixBins, order, s));
+    radix16_scan_kernel<<<kScan16Blocks, kRadixBins, 0, s>>>(part, (uint32_t)hgrid, n32, ctl, (uint32_t)skip,
+                                                             d_in == d_out ? 1u : 0u);
+    B200_LAUNCH_CHECK();
+    if (safe) B200_TRY(launch_indices_passes<1>(d_in, d_out, d_tmp, tmp_idx, idx_out, n32, ctl, status, order, s));
+    else      B200_TRY(launch_indices_passes<0>(d_in, d_out, d_tmp, tmp_idx, idx_out, n32, ctl, status, order, s));
+    const size_t blocks = div_up(n, 256);
+    radix16_final_indices_kernel<<<(unsigned)(blocks < (size_t)kNumSMs * 8 ? blocks : (size_t)kNumSMs * 8), 256, 0, s>>>(
+        d_in, d_out, d_tmp, idx_out, n32, ctl);
     B200_LAUNCH_CHECK();
     return B200SORT_OK;
 }

@@ -37,6 +37,11 @@ size_t radix16_workspace_bytes(size_t n);
 // pointers; the workspace and the 30-bit count limit of the pairs are checked here, before any device work.
 int radix16_sort(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, const int32_t *v_in, int32_t *v_out,
                  int32_t *v_tmp, size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s, SignXor16 order);
+// Sort with indices: the keys sorted stably as by the pairs sort, and idx_out[i] = the input position of d_out[i], as
+// int64 (no index input; tmp_idx holds n int32 of scratch).  d_in may equal d_out.  Same workspace and checks as the
+// pairs sort; n == 1 writes idx_out[0] = 0 without a workspace.
+int radix16_sort_indices(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx,
+                         size_t n, void *d_ws, size_t ws_bytes, cudaStream_t s, SignXor16 order);
 unsigned long long radix16_check_failures(unsigned long long *per_site);
 
 }  // namespace b200sort

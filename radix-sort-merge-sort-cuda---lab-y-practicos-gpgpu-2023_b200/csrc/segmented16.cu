@@ -12,6 +12,10 @@
 //   g4  seg16_warp_kernel         class 1: a warp per segment
 //   g5  seg16_small_kernel x2     classes 2 and 3: a CTA per segment, both passes in shared memory
 //
+// VALS: 0 keys only, 1 a 32-bit value beside every key, kVals16Idx the key's position in its segment (sort with
+// indices, DESIGN section 4.2j): made where the key is first loaded, never read from memory, and stored as int64 into
+// the index output (vout viewed as int32) where it is stored for the last time.
+//
 // The onesweep passes and the small-segment CTAs rank with lane-ordered shared-memory atomics like the 1-D kernels,
 // behind the same self-test (radix_atomic_order_ok); SAFE = 1 is their ballot-ranked form.  Keys are read and
 // written as 2-byte words, so a segment may begin at any 2-byte boundary.
@@ -35,6 +39,7 @@ size_t segmented16_class_max(int c) {
     }
 }
 
+constexpr int kVals16Idx = 2;
 constexpr int kSeg16Warps = kSeg16Threads / 32;
 constexpr int kWarp16SegMax = (int)kSeg16Max1;                // 128
 constexpr int kWarp16SegIpt = kWarp16SegMax / 32;
@@ -84,9 +89,10 @@ __device__ __forceinline__ uint32_t seg16_digit(uint32_t k, int pass, SignXor16 
 }
 
 // ---- g0 -------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-seg16_classify_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
-                      const int32_t *offsets, uint32_t num_segments, Seg16Control *ctl, Seg16Lists lists, uint32_t *hist)
+template <int IDX>
+__device__ __forceinline__ void
+seg16_classify_body(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
+                    const int32_t *offsets, uint32_t num_segments, Seg16Control *ctl, Seg16Lists lists, uint32_t *hist)
 {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < num_segments; i += gridDim.x * blockDim.x) {
         const int32_t o0 = offsets[i], o1 = offsets[i + 1];
@@ -94,7 +100,14 @@ seg16_classify_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int
         const uint32_t e = o1 < (int32_t)b ? b : ((uint32_t)o1 > n ? n : (uint32_t)o1);
         const uint32_t len = e - b;
         if (len == 1 && in != out) out[b] = in[b];
-        if (len == 1 && vin != nullptr && vin != vout) vout[b] = vin[b];
+        if constexpr (IDX != 0) {
+            if (len == 1) {
+                B200_CHECK((reinterpret_cast<uintptr_t>(vout) & 7) == 0);
+                reinterpret_cast<int64_t *>(vout)[b] = 0;
+            }
+        } else if (len == 1 && vin != nullptr && vin != vout) {
+            vout[b] = vin[b];
+        }
         // class c - 1; 4 = nothing to sort.  One atomicAdd per class and warp (segmented.cu).
         const int c = len <= kSeg16Max0 ? 4 : len <= kSeg16Max1 ? 0 : len <= kSeg16Max2 ? 1 : len <= kSeg16Max3 ? 2 : 3;
         const uint32_t active = __activemask();
@@ -114,6 +127,21 @@ seg16_classify_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int
             for (int w = 0; w < kSeg16Passes * kRadixBins / 4; ++w) h[w] = make_uint4(0, 0, 0, 0);
         }
     }
+}
+__global__ void __launch_bounds__(256)
+seg16_classify_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
+                      const int32_t *offsets, uint32_t num_segments, Seg16Control *ctl, Seg16Lists lists, uint32_t *hist)
+{
+    seg16_classify_body<0>(in, out, vin, vout, n, offsets, num_segments, ctl, lists, hist);
+}
+// Sort with indices: a segment of one key gets index 0 (vout is the int64 index output viewed as int32); nothing is
+// written for an empty one.
+__global__ void __launch_bounds__(256)
+seg16_classify_indices_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t *vout, uint32_t n,
+                              const int32_t *offsets, uint32_t num_segments, Seg16Control *ctl, Seg16Lists lists,
+                              uint32_t *hist)
+{
+    seg16_classify_body<1>(in, out, vin, vout, n, offsets, num_segments, ctl, lists, hist);
 }
 
 // ---- g1 -------------------------------------------------------------------------------------------------------------
@@ -221,7 +249,9 @@ struct Seg16PassSmem {
 // count, and key i of digit d goes to
 //   segment begin + segment base[d] + (keys of digit d in earlier tiles of the segment) + tile-local rank.
 // Slots past the segment's end are neither ranked nor staged.  Pass 0 reads in and writes tmp, pass 1 reads tmp and
-// writes out, so out of place the input is only read.
+// writes out, so out of place the input is only read.  VALS = kVals16Idx: pass 0 makes the positions and writes them
+// as int32 into vtmp (n int32 of its own, so the index 0 that the classify kernel wrote for a segment of one key is
+// never overwritten); pass 1 reads them there and stores them as int64 into vout.
 template <int VALS, int SAFE>
 __global__ void __launch_bounds__(kSeg16Threads, 2)
 seg16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const int32_t *vin, int32_t *vout,
@@ -264,12 +294,18 @@ seg16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const in
 
         // kr: the key in the low half, its rank among the warp's keys of its digit (< kSeg16Tile) in the high half
         uint32_t kr[kSeg16Ipt];
-        int32_t val[VALS ? kSeg16Ipt : 1];
+        int32_t val[VALS == 1 ? kSeg16Ipt : 1];
 #pragma unroll
         for (int i = 0; i < kSeg16Ipt; ++i) {
             const uint32_t at = wofs + i * 32;                // warp-striped: tile order = memory order
             kr[i] = at < valid ? src[begin + start + at] : 0u;
-            if constexpr (VALS != 0) val[i] = at < valid ? vsrc[begin + start + at] : 0;
+            if constexpr (VALS == kVals16Idx) {
+                // the index is not held through the ranking (that spills): pass 0 makes it and pass 1 loads it when
+                // the key is staged; here pass 1 only asks L2 for its line
+                if (pass != 0 && at < valid) asm volatile("prefetch.global.L2 [%0];" :: "l"(vsrc + begin + start + at));
+            } else if constexpr (VALS != 0) {
+                val[i] = at < valid ? vsrc[begin + start + at] : 0;
+            }
         }
 #pragma unroll
         for (int i = 0; i < kSeg16Ipt; ++i) {
@@ -326,7 +362,12 @@ seg16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const in
                 B200_CHECK_AT(1, at < kSeg16Tile);
                 if (at < kSeg16Tile) {
                     sm.keys[at] = (uint16_t)key;
-                    if constexpr (VALS != 0) sm.vals[at] = val[i];
+                    if constexpr (VALS == kVals16Idx) {
+                        const uint32_t p = start + wofs + i * 32;
+                        sm.vals[at] = pass == 0 ? (int32_t)p : vsrc[begin + p];
+                    } else if constexpr (VALS != 0) {
+                        sm.vals[at] = val[i];
+                    }
                 }
             }
         }
@@ -337,7 +378,16 @@ seg16_onesweep_kernel(const uint16_t *in, uint16_t *out, uint16_t *tmp, const in
             B200_CHECK_AT(15, pos < len);
             if (pos < len) {                                   // only malformed offsets fail this
                 dst[begin + pos] = (uint16_t)kk;
-                if constexpr (VALS != 0) vdst[begin + pos] = sm.vals[i];
+                if constexpr (VALS == kVals16Idx) {
+                    if (pass == kSeg16Passes - 1) {
+                        B200_CHECK((reinterpret_cast<uintptr_t>(vout) & 7) == 0);
+                        reinterpret_cast<int64_t *>(vout)[begin + pos] = sm.vals[i];
+                    } else {
+                        vdst[begin + pos] = sm.vals[i];
+                    }
+                } else if constexpr (VALS != 0) {
+                    vdst[begin + pos] = sm.vals[i];
+                }
             }
         }
         __syncthreads();                                       // shared memory free for the next tile
@@ -366,7 +416,8 @@ seg16_warp_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t
         for (int q = 0; q < kWarp16SegIpt; ++q) {
             const uint32_t i = lane + 32 * q;
             key[q] = i < len ? in[seg.x + i] : 0u;
-            if constexpr (VALS != 0) val[q] = i < len ? vin[seg.x + i] : 0;
+            if constexpr (VALS == kVals16Idx) val[q] = (int32_t)i;
+            else if constexpr (VALS != 0) val[q] = i < len ? vin[seg.x + i] : 0;
             img[q] = image16(key[q], order);
             pos[q] = 0;
             if (i < len) img_s[i] = img[q];
@@ -382,7 +433,12 @@ seg16_warp_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t
             if (lane + 32 * q < len) {
                 B200_CHECK_AT(15, pos[q] < len);
                 out[seg.x + pos[q]] = (uint16_t)key[q];
-                if constexpr (VALS != 0) vout[seg.x + pos[q]] = val[q];
+                if constexpr (VALS == kVals16Idx) {
+                    B200_CHECK((reinterpret_cast<uintptr_t>(vout) & 7) == 0);
+                    reinterpret_cast<int64_t *>(vout)[seg.x + pos[q]] = val[q];
+                } else if constexpr (VALS != 0) {
+                    vout[seg.x + pos[q]] = val[q];
+                }
             }
         }
         __syncwarp();                                          // img_s free for the warp's next segment
@@ -393,6 +449,8 @@ seg16_warp_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_t
 // Classes 2 and 3: one segment of n <= THREADS * IPT keys sorted in one CTA, radix_small_body's scheme on 16-bit
 // images: the images sit in shared memory, each pass ranks the real keys with the warp's counters (slots past n are
 // neither ranked nor moved), scans the 256 digits and scatters into the other buffer; values follow their keys.
+// VALS = kVals16Idx: the value buffer starts as 0..n-1 (vin is not read) and vout is the segment's int64 index output
+// viewed as int32.
 // Shared memory: values [2][tile] (VALS), warp counters [warps][256], scan sums [8], images [2][tile].
 constexpr size_t seg16_small_smem_bytes(int threads, int ipt, int vals) {
     return (size_t)2 * threads * ipt * (vals ? 4 : 0) + (size_t)(threads / 32) * kRadixBins * 4 + 32 +
@@ -417,7 +475,9 @@ __device__ __forceinline__ void seg16_small_body(const uint16_t *in, uint16_t *o
     const uint32_t wofs = warp * (32 * IPT) + lane;
 
     for (uint32_t i = tid; i < n; i += THREADS) s_buf[i] = (uint16_t)image16(in[i], order);
-    if constexpr (VALS != 0)
+    if constexpr (VALS == kVals16Idx)
+        for (uint32_t i = tid; i < n; i += THREADS) s_vbuf[i] = (int32_t)i;
+    else if constexpr (VALS != 0)
         for (uint32_t i = tid; i < n; i += THREADS) s_vbuf[i] = vin[i];
     __syncthreads();
 
@@ -476,7 +536,12 @@ __device__ __forceinline__ void seg16_small_body(const uint16_t *in, uint16_t *o
     const SignXor16 inv = inverse16(order);
     const uint16_t *res = s_buf + cur * kTile;
     for (uint32_t i = tid; i < n; i += THREADS) out[i] = (uint16_t)image16(res[i], inv);
-    if constexpr (VALS != 0) {
+    if constexpr (VALS == kVals16Idx) {
+        const int32_t *vres = s_vbuf + cur * kTile;
+        int64_t *wide = reinterpret_cast<int64_t *>(vout);
+        B200_CHECK((reinterpret_cast<uintptr_t>(wide) & 7) == 0);
+        for (uint32_t i = tid; i < n; i += THREADS) wide[i] = vres[i];
+    } else if constexpr (VALS != 0) {
         const int32_t *vres = s_vbuf + cur * kTile;
         for (uint32_t i = tid; i < n; i += THREADS) vout[i] = vres[i];
     }
@@ -490,8 +555,12 @@ seg16_small_kernel(const uint16_t *in, uint16_t *out, const int32_t *vin, int32_
     const uint32_t count = ctl->count[c] < cap ? ctl->count[c] : cap;
     for (uint32_t s = blockIdx.x; s < count; s += gridDim.x) {
         const uint2 seg = list[s];
-        seg16_small_body<THREADS, IPT, VALS, SAFE>(in + seg.x, out + seg.x, seg.y - seg.x, order,
-                                                   VALS ? vin + seg.x : nullptr, VALS ? vout + seg.x : nullptr);
+        if constexpr (VALS == kVals16Idx)
+            seg16_small_body<THREADS, IPT, VALS, SAFE>(in + seg.x, out + seg.x, seg.y - seg.x, order, nullptr,
+                                                       reinterpret_cast<int32_t *>(reinterpret_cast<int64_t *>(vout) + seg.x));
+        else
+            seg16_small_body<THREADS, IPT, VALS, SAFE>(in + seg.x, out + seg.x, seg.y - seg.x, order,
+                                                       VALS ? vin + seg.x : nullptr, VALS ? vout + seg.x : nullptr);
         __syncthreads();                                       // shared memory free for the next segment
     }
 }
@@ -533,7 +602,7 @@ static int seg16_sort_impl(const uint16_t *in, uint16_t *out, uint16_t *tmp, con
     const uint32_t cap_large = (uint32_t)L.cap[3];
 
     B200_CUDA_TRY(cudaMemsetAsync(ctl, 0, sizeof(Seg16Control), s));
-    seg16_classify_kernel<<<seg16_grid(div_up(S, 256), (size_t)kNumSMs * 8), 256, 0, s>>>(
+    (VALS == kVals16Idx ? seg16_classify_indices_kernel : seg16_classify_kernel)<<<seg16_grid(div_up(S, 256), (size_t)kNumSMs * 8), 256, 0, s>>>(
         in, out, vin, vout, (uint32_t)n, offsets, (uint32_t)S, ctl, lists, hist);
     B200_LAUNCH_CHECK();
     seg16_tile_plan_kernel<<<1, kPlan16Threads, 0, s>>>(ctl, lists.list[3], cap_large, prefix, (uint32_t)L.rows);
@@ -572,6 +641,16 @@ int segmented16_sort(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, con
                     : seg16_sort_impl<0, 0>(d_in, d_out, d_tmp, nullptr, nullptr, nullptr, n, d_offsets, num_segments, d_ws, s, order);
     return safe ? seg16_sort_impl<1, 1>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, d_offsets, num_segments, d_ws, s, order)
                 : seg16_sort_impl<1, 0>(d_in, d_out, d_tmp, v_in, v_out, v_tmp, n, d_offsets, num_segments, d_ws, s, order);
+}
+
+int segmented16_sort_indices(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx,
+                             size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws, cudaStream_t s,
+                             SignXor16 order) {
+    if (num_segments == 0) return B200SORT_OK;
+    auto *idx32 = reinterpret_cast<int32_t *>(idx_out);
+    return radix_atomic_order_ok()
+               ? seg16_sort_impl<kVals16Idx, 0>(d_in, d_out, d_tmp, nullptr, idx32, tmp_idx, n, d_offsets, num_segments, d_ws, s, order)
+               : seg16_sort_impl<kVals16Idx, 1>(d_in, d_out, d_tmp, nullptr, idx32, tmp_idx, n, d_offsets, num_segments, d_ws, s, order);
 }
 
 unsigned long long segmented16_check_failures(unsigned long long *per_site) { return tu_check_failures(per_site); }

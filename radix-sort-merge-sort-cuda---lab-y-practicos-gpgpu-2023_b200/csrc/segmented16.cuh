@@ -24,6 +24,11 @@ size_t segmented16_workspace_bytes(size_t n, size_t num_segments);
 int segmented16_sort(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, const int32_t *v_in, int32_t *v_out,
                      int32_t *v_tmp, size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws,
                      cudaStream_t s, SignXor16 order);
+// Sort with indices: idx_out[i] = position of d_out[i] inside its segment, as int64 (no index input).  tmp_idx holds
+// n int32.  Checked by the caller like segmented16_sort.
+int segmented16_sort_indices(const uint16_t *d_in, uint16_t *d_out, uint16_t *d_tmp, int64_t *idx_out, int32_t *tmp_idx,
+                             size_t n, const int32_t *d_offsets, size_t num_segments, void *d_ws, cudaStream_t s,
+                             SignXor16 order);
 unsigned long long segmented16_check_failures(unsigned long long *per_site);
 
 }  // namespace b200sort

@@ -16,12 +16,13 @@ KEY_F32 = 2
 _ALGOS = {"radix": ALGO_RADIX, "merge": ALGO_MERGE}
 
 
-def _key_type(torch, x) -> int:
+def _key_type(torch, x, others: str = "") -> int:
     types = {torch.int32: KEY_I32, torch.uint32: KEY_U32, torch.float32: KEY_F32}
     if not isinstance(x, torch.Tensor):
         raise TypeError(f"expected a torch.Tensor, got {type(x).__name__}")
     if x.dtype not in types:
-        raise TypeError(f"keys must be torch.int32, torch.uint32 or torch.float32, got {x.dtype}")
+        raise TypeError(f"keys must be torch.int32, torch.uint32 or torch.float32, got {x.dtype}"
+                        + (f" ({others})" if others else ""))
     return types[x.dtype]
 
 
@@ -111,7 +112,7 @@ def sort_with_indices(x, *, descending: bool = False):
     """
     import torch
 
-    key_type = _key_type(torch, x)
+    key_type = _key_type(torch, x, "16-bit keys: b200sort.sort16_with_indices")
     _check_layout(x, "keys")
     n = x.numel()
     values = torch.empty_like(x)

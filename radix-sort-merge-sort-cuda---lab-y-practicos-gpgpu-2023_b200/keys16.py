@@ -1,5 +1,5 @@
 """Sorting torch tensors of int16, uint16, float16 or bfloat16 keys, ascending or descending (b200sort_sort_keys16,
-b200sort_radix_pairs_keys16 in include/b200sort.h).
+b200sort_radix_pairs_keys16, b200sort_radix_sort_indices_keys16 in include/b200sort.h).
 
 float16 and bfloat16 keys are ordered by IEEE-754 totalOrder on their bit patterns, as float32 keys are in
 ``b200sort.sort``: -NaN < -inf < negatives < -0.0 < +0.0 < positives < +inf < +NaN, NaNs of one sign by payload.
@@ -60,12 +60,9 @@ def sort16_by_key(keys, values, *, descending: bool = False):
     """``(sorted keys, values in the same order)``: a STABLE sort of (16-bit key, int32 value) pairs by key.
 
     ``keys``: 1-D CUDA tensor of int16, uint16, float16 or bfloat16; ``values``: int32 of the same length on the
-    same device.  Equal keys keep their input order in both directions.  The inputs are left untouched.  argsort::
-
-        order = sort16_by_key(x, torch.arange(n, dtype=torch.int32, device=x.device))[1]
-
-    On inputs without NaN and -0.0 this equals ``torch.sort(x, stable=True, descending=descending)``, values and
-    indices (as int32).
+    same device.  Equal keys keep their input order in both directions.  The inputs are left untouched.  For the
+    sorted keys with their int64 positions (what ``torch.sort`` returns) call ``sort16_with_indices``: it makes the
+    positions on the device instead of reading them.
     """
     import torch
 
@@ -92,3 +89,32 @@ def sort16_by_key(keys, values, *, descending: bool = False):
                                                 k_out.data_ptr(), v_out.data_ptr(), k_tmp.data_ptr(), v_tmp.data_ptr(),
                                                 n, ws_ptr, ws_bytes, stream))
     return k_out, v_out
+
+
+def sort16_with_indices(x, *, descending: bool = False):
+    """``(values, indices)``: ``x`` sorted, and the int64 position in ``x`` of every value.
+
+    ``x``: 1-D contiguous CUDA tensor of int16, uint16, float16 or bfloat16; it is left untouched.  The sort is STABLE
+    in both directions (equal keys keep their input order), so on inputs without NaN and -0.0 the result equals
+    ``torch.sort(x, stable=True, descending=descending)``, values and indices, dtype for dtype; float16 and bfloat16
+    otherwise follow IEEE-754 totalOrder (see the module docstring).  No index array is read: the first radix pass
+    makes the positions and the last stores them as int64.  Runs on ``torch.cuda.current_stream(x.device)``.
+    """
+    import torch
+
+    key_type = _key_type(torch, x, "32-bit keys: b200sort.sort_with_indices")
+    _check_layout(x, "keys")
+    n = x.numel()
+    values = torch.empty_like(x)
+    indices = torch.empty(n, dtype=torch.int64, device=x.device)
+    if n == 0:
+        return values, indices
+    with torch.cuda.device(x.device):
+        k_tmp = torch.empty_like(x)
+        i_tmp = torch.empty(n, dtype=torch.int32, device=x.device)
+        ws, ws_ptr, ws_bytes = _workspace(torch, n, x.device)
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        check(lib().b200sort_radix_sort_indices_keys16(key_type, int(bool(descending)), x.data_ptr(), values.data_ptr(),
+                                                       indices.data_ptr(), k_tmp.data_ptr(), i_tmp.data_ptr(), n,
+                                                       ws_ptr, ws_bytes, stream))
+    return values, indices

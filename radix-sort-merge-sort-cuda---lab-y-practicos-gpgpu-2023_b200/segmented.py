@@ -117,7 +117,7 @@ def segmented_sort_with_indices(keys, offsets=None, *, descending: bool = False)
     """
     import torch
 
-    key_type = _key_type(torch, keys)
+    key_type = _key_type(torch, keys, "16-bit keys: b200sort.segmented_sort16_with_indices")
     n, offs, segments = _segments(torch, keys, offsets)
     values = torch.empty_like(keys)
     indices = torch.empty(keys.shape, dtype=torch.int64, device=keys.device)

@@ -2,7 +2,8 @@
 """What compute-sanitizer runs (tools/sanitize.sh): every kernel family once at smoke sizes, each result checked
 against the oracle.  `python tools/sanitize_target.py [big | keys16 | segmented16]` -- `big` adds one 2^20-key radix sort; `keys16` runs
 only the 16-bit sorts, `segmented16` only the segmented sort of 16-bit keys,
-`segmented64` only the segmented sort of 64-bit keys, `indices` only the sorts with int64 indices."""
+`segmented64` only the segmented sort of 64-bit keys, `indices` only the sorts with int64 indices, `indices16` only
+the sorts of 16-bit keys with int64 indices."""
 import ctypes
 import os
 import sys
@@ -94,6 +95,24 @@ def indices_runs():
     print(f"  ok segmented sort with indices, n={int(offs[-1])}, {offs.size - 1} segments, every order", flush=True)
 
 
+def indices16_runs():
+    """Sort with indices of 16-bit keys: 1-D in every order and every pass plan, in place and copied, and the
+    segmented form on a ragged mix covering every size class, in every order."""
+    import key_orders16 as ko16
+    from test_sort_indices16_gpu import check_1d, check_seg, dup_keys, plan_keys, ragged_offsets
+    for kt, desc in ko16.ORDERS:
+        for in_place in (False, True):
+            check_1d(dup_keys((1 << 20) + 7, kt, kt + desc), kt, desc, in_place, "1-D", word_offset=1)
+            for S in (set(), {0}, {1}, {0, 1}):
+                check_1d(plan_keys(70001, S, (kt, desc), kt + desc), kt, desc, in_place, f"plan {sorted(S)}")
+    print("  ok 1-D sort of 16-bit keys with indices, every order and pass plan", flush=True)
+    offs = ragged_offsets(5, total_segments=2000, big=1)
+    for kt, desc in ko16.ORDERS:
+        check_seg(dup_keys(int(offs[-1]), kt, desc), offs, kt, desc, desc == 1, "segmented", word_offset=3)
+    print(f"  ok segmented sort of 16-bit keys with indices, n={int(offs[-1])}, {offs.size - 1} segments, every order",
+          flush=True)
+
+
 def report_checked():
     sites = (ctypes.c_ulonglong * 16)()
     fails = int(L.b200sort_debug_check_failures_by_site(ctypes.cast(sites, ctypes.c_void_p)))
@@ -119,6 +138,12 @@ if len(sys.argv) > 1 and sys.argv[1] == "segmented64":  # only the segmented sor
     sys.exit(0)
 if len(sys.argv) > 1 and sys.argv[1] == "indices":      # only the sorts with int64 indices
     indices_runs()
+    if L.b200sort_debug_checked_build():
+        report_checked()
+    print("SANITIZE TARGET PASSED", flush=True)
+    sys.exit(0)
+if len(sys.argv) > 1 and sys.argv[1] == "indices16":    # only the sorts of 16-bit keys with int64 indices
+    indices16_runs()
     if L.b200sort_debug_checked_build():
         report_checked()
     print("SANITIZE TARGET PASSED", flush=True)
