@@ -83,8 +83,10 @@ int         b200sort_last_cuda_error(void);
 const char *b200sort_last_cuda_error_string(void);
 /* B200SORT_OK iff the current device exists and is compute capability 10.x.  Also the explicit per-device
  * initialisation: runs the lane-order self-test of the radix sort for the current device if it has not run
- * yet (allocates, launches on a private stream, BLOCKS).  Call it once per device before capturing CUDA
- * graphs or timing: the first sort on a device otherwise does it lazily. */
+ * yet (launches on a private stream and BLOCKS; allocates nothing).  Call it once per device before timing: the
+ * first sort on a device otherwise does it lazily.  That lazy test may run inside a CUDA graph capture, on this
+ * thread or another: it switches the thread to relaxed capture mode for its few calls, which stay outside the graph,
+ * and caches only a verdict its kernel returned. */
 int         b200sort_device_check(void);
 
 /* ---- device-array sorts (the layer measured against the HBM roofline) --------------------------
@@ -182,7 +184,7 @@ int    b200sort_radix_pairs_keys(int key_type, int descending, const void *d_key
  * Like the other radix sorts the passes rank with lane-ordered shared-memory atomics only after the self-test of
  * b200sort_radix_i32 has passed on the device; otherwise, or with B200SORT_RANK_SAFE=1, their ballot-ranked form runs.
  * A call enqueues one memset and the same ten kernels for every n >= 2 and every distribution, never synchronises and
- * never reads device results on the host, so it can be captured in a CUDA graph once b200sort_device_check() has run.
+ * never reads device results on the host, so it can be captured in a CUDA graph.
  * Arrays of up to 8192 keys pay that whole sequence too: there is no one-CTA path for 64-bit keys.
  * d_in may equal d_out (in place); otherwise d_in is only read.  d_tmp: n keys of scratch.  Workspace:
  * b200sort_keys64_workspace_bytes(n) bytes, 256-byte aligned, sized from n alone.
@@ -225,8 +227,7 @@ int    b200sort_radix_pairs_keys64(int key_type, int descending, const void *d_k
  * Its passes rank like the other radix sorts: lane-ordered shared-memory atomics after the self-test has passed on
  * the device, otherwise, or with B200SORT_RANK_SAFE=1, the ballot-ranked form.  b200sort_radix_set_variant applies to
  * neither.  A call enqueues one memset and the same kernels for every n >= 2 and every distribution (3 for keys, 5
- * for pairs), never synchronises and never reads device results on the host, so it can be captured in a CUDA graph
- * (pairs once b200sort_device_check() has run).
+ * for pairs), never synchronises and never reads device results on the host, so it can be captured in a CUDA graph.
  * Key pointers need only 2-byte alignment.  d_in may equal d_out (in place); otherwise d_in is only read.
  * Workspace: b200sort_keys16_workspace_bytes(n) bytes, 256-byte aligned, sized from n alone, for keys and pairs.
  * Key type outside B200SORT_KEY_I16..BF16, descending not 0/1, n > B200SORT_MAX_N, NULL data pointers with n > 0, key
@@ -251,10 +252,9 @@ int    b200sort_radix_pairs_keys16(int key_type, int descending, const void *d_k
  * num_segments + 1 int32 with d_offsets[0] = 0, d_offsets[num_segments] = n, non-decreasing; empty segments allowed.
  * Each segment comes out sorted in the order (key_type, descending) of b200sort_sort_keys; keys never cross segments.
  * The host never reads d_offsets: a call is stream-ordered, enqueues the same kernels whatever the number of segments
- * (no host loop over segments, no host synchronisation), and can be captured in a CUDA graph once
- * b200sort_device_check() has run on the device.  Malformed offsets (decreasing, negative, past n) give an undefined
- * order but never an access out of bounds: every segment is clamped to [0, n] on the device, and the checked build
- * counts what the clamps caught at check site 15.
+ * (no host loop over segments, no host synchronisation), and can be captured in a CUDA graph.  Malformed offsets
+ * (decreasing, negative, past n) give an undefined order but never an access out of bounds: every segment is clamped
+ * to [0, n] on the device, and the checked build counts what the clamps caught at check site 15.
  * Segments are routed by length to size classes (b200sort_segmented_class_max): copies for length 0-1, a warp per
  * segment, a CTA per segment sorted in shared memory (two capacities), and above that a segmented onesweep whose tiles
  * never straddle a segment.  Like the 1-D radix sort, the ranking kernels rely on lane-ordered shared-memory atomics
@@ -301,7 +301,7 @@ size_t b200sort_segmented_class_max(int c);
  * B200SORT_ERR_INVALID).  The segmented form follows b200sort_segmented_pairs_keys: offsets as there, clamped on the
  * device.  A call enqueues the same kernels for every n >= 2 and every distribution (1-D: one memset and six kernels,
  * five with skipping off; segmented: those of b200sort_segmented_pairs_keys), never synchronises and never reads
- * device results on the host, so it can be captured in a CUDA graph once b200sort_device_check() has run. */
+ * device results on the host, so it can be captured in a CUDA graph. */
 int    b200sort_radix_sort_indices_keys(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
                                         int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
                                         void *d_ws, size_t ws_bytes, void *stream);
@@ -322,7 +322,7 @@ int    b200sort_segmented_sort_indices_keys(int key_type, int descending, const 
  * never reads, segments clamped to [0, n] on the device, malformed offsets giving an undefined order but no access
  * out of bounds (the checked build counts the clamps at check site 15).
  * A call enqueues one memset and the same eight kernels whatever the number of segments and the data, never
- * synchronises, and can be captured in a CUDA graph once b200sort_device_check() has run.  Size classes
+ * synchronises, and can be captured in a CUDA graph.  Size classes
  * (b200sort_segmented16_class_max): copies for length 0-1, a warp per segment, a CTA per segment sorted in shared
  * memory by two 8-bit passes (two capacities), and above that a segmented onesweep of two passes whose tiles never
  * straddle a segment.  The ranking kernels use lane-ordered shared-memory atomics only after the self-test of
@@ -372,7 +372,7 @@ int    b200sort_segmented_pairs_keys16(int key_type, int descending, const void 
  * segmented form follows b200sort_segmented_pairs_keys16: offsets as there, clamped on the device.  A call enqueues the
  * same kernels for every n >= 2 and every distribution (1-D: one memset and five kernels; segmented: those of
  * b200sort_segmented_pairs_keys16), never synchronises and never reads device results on the host, so it can be
- * captured in a CUDA graph once b200sort_device_check() has run. */
+ * captured in a CUDA graph. */
 int    b200sort_radix_sort_indices_keys16(int key_type, int descending, const void *d_keys_in, void *d_keys_out,
                                           int64_t *d_idx_out, void *d_tmp_keys, int32_t *d_tmp_idx, size_t n,
                                           void *d_ws, size_t ws_bytes, void *stream);
@@ -398,7 +398,7 @@ int    b200sort_segmented_sort_indices_keys16(int key_type, int descending, cons
  * share the digit, and the onesweep class skips pass p when that holds in each of its segments (one large segment
  * whose keys differ in digit p makes pass p run for all of them).  Rows of int64 ids below 2^32 thus run at most 4
  * of the 8 passes.  A call still enqueues one memset and the same fifteen kernels whatever the number of segments
- * and the data, never synchronises, and can be captured in a CUDA graph once b200sort_device_check() has run.  The
+ * and the data, never synchronises, and can be captured in a CUDA graph.  The
  * ranking kernels use lane-ordered shared-memory atomics only after the self-test of b200sort_radix_i32 has passed on
  * the device; otherwise, or with B200SORT_RANK_SAFE=1, their ballot-ranked forms run.  b200sort_radix_set_variant
  * and b200sort_radix_set_skip are ignored: skipping is always on.  DESIGN section 4.2h.

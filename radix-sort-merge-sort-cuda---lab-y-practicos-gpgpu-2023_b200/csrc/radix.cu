@@ -244,9 +244,15 @@ std::atomic<int> g_atomic_order[kMaxDevices];
 std::mutex g_selftest_mu;
 struct AtomicOrderInit { AtomicOrderInit() { for (auto &a : g_atomic_order) a.store(-1); } } g_atomic_order_init;
 
+// The self-test's flag word: one per device, as every __device__ variable is, so the test allocates nothing.
+__device__ uint32_t g_selftest_bad;
+
 // Runs the self-test on the current device unless its verdict is cached.  Called from b200sort_device_check()
-// (the explicit init) and, as a fallback, lazily from the first sort on a device: it allocates, launches on
-// a private stream and BLOCKS, so callers that capture CUDA graphs must call b200sort_device_check() first.
+// (the explicit init) and, as a fallback, lazily from the first sort on a device: it launches on a private stream and
+// BLOCKS.  It may run while this thread or another one captures a CUDA graph (a first sort inside torch.cuda.graph):
+// it switches this thread to the relaxed capture mode for the test, so the capture neither forbids nor sees its calls,
+// and it allocates and frees nothing.  Only a verdict read back from the kernel is cached; if a CUDA call fails, the
+// caller runs the ballot-ranked shape and the next call tries again.
 int atomic_order_ok() {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) { cudaGetLastError(); return 0; }
@@ -257,20 +263,23 @@ int atomic_order_ok() {
     if (v >= 0) return v;
     const char *env = getenv("B200SORT_RANK_SAFE");
     if (env != nullptr && env[0] == '1') { g_atomic_order[dev].store(0); return 0; }
+    cudaStreamCaptureMode mode = cudaStreamCaptureModeRelaxed;
+    if (cudaThreadExchangeStreamCaptureMode(&mode) != cudaSuccess) { cudaGetLastError(); return 0; }
     uint32_t *d_bad = nullptr, h_bad = 1;
     cudaStream_t st = nullptr;
-    bool ok = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) == cudaSuccess &&
-              cudaMalloc(&d_bad, sizeof(uint32_t)) == cudaSuccess &&
+    bool ok = cudaGetSymbolAddress(reinterpret_cast<void **>(&d_bad), g_selftest_bad) == cudaSuccess &&
+              cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) == cudaSuccess &&
               cudaMemsetAsync(d_bad, 0, sizeof(uint32_t), st) == cudaSuccess;
     if (ok) {
         radix_atomic_order_selftest_kernel<<<kNumSMs * 2, 512, 0, st>>>(d_bad);
         ++g_launch_count;
-        ok = cudaMemcpyAsync(&h_bad, d_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, st) == cudaSuccess &&
+        ok = cudaGetLastError() == cudaSuccess &&
+             cudaMemcpyAsync(&h_bad, d_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, st) == cudaSuccess &&
              cudaStreamSynchronize(st) == cudaSuccess;
     }
-    if (!ok) { cudaGetLastError(); h_bad = 1; }
-    if (d_bad) cudaFree(d_bad);
     if (st) cudaStreamDestroy(st);
+    cudaThreadExchangeStreamCaptureMode(&mode);                  // the caller's mode again
+    if (!ok) { cudaGetLastError(); return 0; }                  // no verdict: the safe shape, for this call only
     v = (h_bad == 0) ? 1 : 0;
     g_atomic_order[dev].store(v, std::memory_order_release);
     return v;
@@ -601,8 +610,8 @@ int radix_sort_pairs(const int32_t *d_in, int32_t *d_out, int32_t *d_tmp, const 
     if (keys && !safe && pairs_ipt() != 10) return B200SORT_ERR_INVALID;   // the generic pairs kernel has 5120-key tiles
     B200_TRY(ensure_hist_attr(keys));
     auto *ctl = static_cast<RadixControl *>(d_ws);
-    const size_t tiles = div_up(n, radix_pairs_tile());
-    const size_t rows = tiles + div_up(tiles, (size_t)kLookGroup);
+    const size_t tiles = div_up(n, 512u * (size_t)(safe ? 10 : pairs_ipt()));   // radix_pairs_tile(), from the
+    const size_t rows = tiles + div_up(tiles, (size_t)kLookGroup);             // verdict this call runs on
     uint32_t *status[2];
     status[0] = reinterpret_cast<uint32_t *>(static_cast<unsigned char *>(d_ws) + kRadixControlBytes);
     status[1] = status[0] + rows * kRadixBins;

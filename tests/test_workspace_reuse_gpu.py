@@ -1,5 +1,6 @@
 """A reused, never-cleared workspace and guarded buffers for the 16-bit, segmented, merge and lab sorts, stale state
-left by one entry point for another, and CUDA graph replay of the 32-bit 1-D sorts.
+left by one entry point for another (the 64-bit and the indices sorts among them), and CUDA graph replay of the 32-bit
+1-D sorts.
 
 Every device-array entry point takes a caller-owned workspace and must rewrite whatever it reads there before reading
 it: real callers (torch's caching allocator, a benchmark loop, a replayed graph) hand it back holding the previous
@@ -14,8 +15,9 @@ crashes, so this module looks for both:
   * the 32-bit entry points captured once in a CUDA graph and replayed on data that takes other device-side plans.
 
 Everything goes through the C-ABI; torch only owns the memory.  References are stable numpy argsorts of the key
-images (tests/key_orders.py, tests/key_orders16.py), per segment for the segmented sorts (np.lexsort), and
-oracle.radix_sort for the lab pipeline; results are compared byte for byte.
+images (tests/key_orders.py, key_orders16.py, key_orders64.py), per segment for the segmented sorts (np.lexsort), with
+the argsort itself (made segment-local) as the reference of the int64 indices, and oracle.radix_sort for the lab
+pipeline; results are compared byte for byte.
 """
 import functools
 
@@ -25,11 +27,13 @@ import pytest
 import digit_patterns as dp
 import key_orders as ko
 import key_orders16 as ko16
+import key_orders64 as ko64
 import oracle
 from b200sort import datagen
 from b200sort._lib import ALGO_LAB, ALGO_MERGE, ALGO_RADIX, check, lib
 from helpers import stream_ptr
 from test_keys16_gpu import random_keys as keys16_of
+from test_keys64_gpu import random_keys as keys64_of
 from test_segmented_cpu import segment_ids
 from test_segmented_gpu import mixed_keys as keys32_of, ragged_offsets
 
@@ -47,6 +51,11 @@ I32 = (ko.KEY_I32, 0)
 # count 2-byte words, so 1, 3 and 7 are 2, 6 and 14 bytes
 OFFS16 = [(0, 0, 0, 0, 0, 0), (1, 3, 7, 1, 2, 3), (3, 7, 1, 2, 3, 0), (7, 1, 3, 3, 0, 1)]
 OFFS32 = [(0, 0, 0, 0, 0, 0), (1, 2, 3, 1, 2, 3), (2, 3, 1, 2, 3, 0), (3, 1, 2, 3, 0, 1)]
+# 8-byte keys and int64 indices need 8-byte alignment: even word offsets
+OFFS64 = [(0, 0, 0, 0, 0, 0), (2, 0, 2, 1, 2, 3)]
+# image masks whose zero bytes make the digit passes over them skippable: 16-bit pass 1, 32-bit passes 1 and 3,
+# 64-bit passes 1, 3, 5 and 7
+MASKED = {16: 0x00FF, 32: 0x00FF00FF, 64: 0x00FF00FF00FF00FF}
 
 # family: (key bits, pairs, scratch keys); the C-ABI entry points beside each
 FAMILIES = {
@@ -60,17 +69,28 @@ FAMILIES = {
     "keys": (32, False, True),          # b200sort_sort_keys, with `algo`
     "pairs_i32": (32, True, True),      # b200sort_radix_pairs_i32 / b200sort_radix_pairs_copy_i32
     "pairs": (32, True, True),          # b200sort_radix_pairs_keys
+    "keys64": (64, False, True),        # b200sort_sort_keys64
+    "pairs64": (64, True, True),        # b200sort_radix_pairs_keys64
+    "seg64": (64, False, True),         # b200sort_segmented_sort_keys64
+    "seg64_pairs": (64, True, True),    # b200sort_segmented_pairs_keys64
+    "idx": (32, False, True),           # b200sort_radix_sort_indices_keys
+    "seg_idx": (32, False, True),       # b200sort_segmented_sort_indices_keys
+    "idx16": (16, False, True),         # b200sort_radix_sort_indices_keys16
+    "seg_idx16": (16, False, True),     # b200sort_segmented_sort_indices_keys16
 }
+# the families that return int64 indices (into an 8-byte buffer) and take n int32 of index scratch
+INDICES = {"idx", "seg_idx", "idx16", "seg_idx16"}
 
 
 def _ko(width: int):
-    return ko16 if width == 16 else ko
+    return {16: ko16, 32: ko, 64: ko64}[width]
 
 
 # ---- segment layouts ---------------------------------------------------------------------------------------------
 def _class_bounds(width: int):
     L = lib()
-    f = L.b200sort_segmented16_class_max if width == 16 else L.b200sort_segmented_class_max
+    f = {16: L.b200sort_segmented16_class_max, 32: L.b200sort_segmented_class_max,
+         64: L.b200sort_segmented64_class_max}[width]
     out, c = [], 0
     while f(c):
         out.append(f(c))
@@ -100,10 +120,11 @@ def layout(name) -> np.ndarray:
         return np.concatenate([[0], tail + (1 << 22)]).astype(np.int32)
     if kind in ("many_large", "few_large"):
         # the same n and number of segments, so the same workspace layout: 200 segments of 40000 keys and 3896 empty
-        # ones, or 3 large segments among 4093 of 2..1024 keys
-        S, n = 4096, 200 * 40000
+        # ones, or 3 large segments among 4093 of 2..1024 keys (or S segments, `large` of them of 40000 keys)
+        S, large = name[1:] if len(name) > 1 else (4096, 200)
+        n = large * 40000
         if kind == "many_large":
-            lens = np.concatenate([np.full(200, 40000), np.zeros(S - 200, np.int64)])
+            lens = np.concatenate([np.full(large, 40000), np.zeros(S - large, np.int64)])
         else:
             small = np.random.default_rng(5).integers(2, 1025, S - 3)
             rest = n - int(small.sum())
@@ -121,11 +142,29 @@ RAGGED = ("ragged", 17, 3000, 2)
 ONE = ("one", (1 << 21) + 7)
 ROWS_2_17 = ("rows", 1 << 17, 64)
 LONG_RAGGED = ("long_ragged", 9)
+RAGGED_SMALL = ("ragged", 23, 3000, 0)                          # 1.75M keys: 12 onesweep-class segments
+MANY_LARGE_2M, FEW_LARGE_2M = ("many_large", 1024, 48), ("few_large", 1024, 48)     # 1.92M keys
+ROWS_9000 = ("rows", 9000, 232)                                  # 2.09M keys in onesweep-class rows
 
 
 def seg_ws_bytes(width: int, n: int, S: int) -> int:
     L = lib()
-    return (L.b200sort_segmented16_workspace_bytes if width == 16 else L.b200sort_segmented_workspace_bytes)(n, S)
+    return {16: L.b200sort_segmented16_workspace_bytes, 32: L.b200sort_segmented_workspace_bytes,
+            64: L.b200sort_segmented64_workspace_bytes}[width](n, S)
+
+
+def ws_need(fam: str, n: int, seg=None, algo: int = ALGO_RADIX) -> int:
+    """The workspace bytes of one call.  The indices sorts take those of the pairs sorts of their width."""
+    L = lib()
+    width = FAMILIES[fam][0]
+    if seg is not None:
+        offs = layout(seg)
+        return seg_ws_bytes(width, int(offs[-1]), offs.size - 1)
+    if width == 16:
+        return L.b200sort_keys16_workspace_bytes(n)
+    if width == 64:
+        return L.b200sort_keys64_workspace_bytes(n)
+    return L.b200sort_workspace_bytes(n, algo)
 
 
 # ---- the module's workspace and buffers ----------------------------------------------------------------------------
@@ -139,10 +178,10 @@ def workspace() -> dp.Workspace:
         needs = [L.b200sort_keys16_workspace_bytes(N16_BIG), L.b200sort_workspace_bytes(N32_BIG, ALGO_RADIX),
                  L.b200sort_workspace_bytes(N32_BIG, ALGO_MERGE)]
         seg = [(w, name) for w in (16, 32) for name in class_rows(w) + [RAGGED, ONE]]
-        seg += [(FAMILIES[job[0]][0], job[4]) for pair in STALE.values() for job in pair if job[4] is not None]
         for width, name in seg:
             offs = layout(name)
             needs.append(seg_ws_bytes(width, int(offs[-1]), offs.size - 1))
+        needs += [ws_need(job[0], job[1], job[4], job[5]) for pair in STALE.values() for job in pair]
         _ws = dp.Workspace(max(needs))
     return _ws
 
@@ -177,7 +216,8 @@ def _device_offsets(name):
 def run(fam: str, keys: np.ndarray, order, in_place: bool = False, offs=OFFS32[0], seg=None, algo: int = ALGO_RADIX,
         what: str = ""):
     """Sort `keys` by family `fam` (FAMILIES) with every array guarded, on the module workspace.  Pairs carry the
-    values arange(n).  seg: the layout name of the segmented families.  Returns (key words, values or None)."""
+    values arange(n).  seg: the layout name of the segmented families.  Returns (key words, values, int64 indices or
+    None)."""
     import torch
     L = lib()
     width, pairs, has_tmp = FAMILIES[fam]
@@ -193,15 +233,14 @@ def run(fam: str, keys: np.ndarray, order, in_place: bool = False, offs=OFFS32[0
         vin = _buf("vin", n, offs[3], 4).load(vals)
         vout = vin if in_place else _buf("vout", n, offs[4], 4).load()
         vtmp = _buf("vtmp", n, offs[5], 4).load()
+    if fam in INDICES:
+        iout = _buf("iout", n, 2 * (offs[4] & 1), 8).load()
+        itmp = _buf("itmp", n, offs[5], 4).load()
     if seg is not None:
         d_off = _device_offsets(seg)
         S = d_off.numel() - 1
         assert int(layout(seg)[-1]) == n
-        need = seg_ws_bytes(width, n, S)
-    elif width == 16:
-        need = L.b200sort_keys16_workspace_bytes(n)
-    else:
-        need = L.b200sort_workspace_bytes(n, algo)
+    need = ws_need(fam, n, seg, algo)
     ws = workspace()
     assert need + ws.GUARD <= ws.cap, f"{what}: the module workspace is sized without this call"
     before = ws.guard(need).cpu()
@@ -211,13 +250,26 @@ def run(fam: str, keys: np.ndarray, order, in_place: bool = False, offs=OFFS32[0
     elif fam == "pairs16":
         st = L.b200sort_radix_pairs_keys16(kt, desc, kin.ptr, vin.ptr, kout.ptr, vout.ptr, ktmp.ptr, vtmp.ptr, n,
                                            ws.ptr, need, s)
-    elif fam in ("seg16", "seg"):
-        f = L.b200sort_segmented_sort_keys16 if width == 16 else L.b200sort_segmented_sort_keys
+    elif fam in ("seg16", "seg", "seg64"):
+        f = {16: L.b200sort_segmented_sort_keys16, 32: L.b200sort_segmented_sort_keys,
+             64: L.b200sort_segmented_sort_keys64}[width]
         st = f(kt, desc, kin.ptr, kout.ptr, ktmp.ptr, n, d_off.data_ptr(), S, ws.ptr, need, s)
-    elif fam in ("seg16_pairs", "seg_pairs"):
-        f = L.b200sort_segmented_pairs_keys16 if width == 16 else L.b200sort_segmented_pairs_keys
+    elif fam in ("seg16_pairs", "seg_pairs", "seg64_pairs"):
+        f = {16: L.b200sort_segmented_pairs_keys16, 32: L.b200sort_segmented_pairs_keys,
+             64: L.b200sort_segmented_pairs_keys64}[width]
         st = f(kt, desc, kin.ptr, vin.ptr, kout.ptr, vout.ptr, ktmp.ptr, vtmp.ptr, n, d_off.data_ptr(), S, ws.ptr,
                need, s)
+    elif fam == "keys64":
+        st = L.b200sort_sort_keys64(kt, desc, kin.ptr, kout.ptr, ktmp.ptr, n, ws.ptr, need, s)
+    elif fam == "pairs64":
+        st = L.b200sort_radix_pairs_keys64(kt, desc, kin.ptr, vin.ptr, kout.ptr, vout.ptr, ktmp.ptr, vtmp.ptr, n,
+                                           ws.ptr, need, s)
+    elif fam in ("idx", "idx16"):
+        f = L.b200sort_radix_sort_indices_keys16 if width == 16 else L.b200sort_radix_sort_indices_keys
+        st = f(kt, desc, kin.ptr, kout.ptr, iout.ptr, ktmp.ptr, itmp.ptr, n, ws.ptr, need, s)
+    elif fam in ("seg_idx", "seg_idx16"):
+        f = L.b200sort_segmented_sort_indices_keys16 if width == 16 else L.b200sort_segmented_sort_indices_keys
+        st = f(kt, desc, kin.ptr, kout.ptr, iout.ptr, ktmp.ptr, itmp.ptr, n, d_off.data_ptr(), S, ws.ptr, need, s)
     elif fam == "i32":
         assert order == I32
         st = (L.b200sort_sort_i32(algo, kin.ptr, ktmp.ptr, n, ws.ptr, need, s) if in_place else
@@ -236,7 +288,7 @@ def run(fam: str, keys: np.ndarray, order, in_place: bool = False, offs=OFFS32[0
         raise ValueError(fam)
     check(st)
     torch.cuda.synchronize()
-    got = kout.read(f"{what} keys out")
+    got = kout.read(f"{what} keys out").view(words.dtype)
     if has_tmp:
         ktmp.read(f"{what} keys tmp")
     if not in_place:
@@ -247,6 +299,9 @@ def run(fam: str, keys: np.ndarray, order, in_place: bool = False, offs=OFFS32[0
         vtmp.read(f"{what} values tmp")
         if not in_place:
             assert vin.read(f"{what} values in").tobytes() == vals.tobytes(), f"{what}: the copy form modified its values"
+    if fam in INDICES:
+        got_vals = iout.read(f"{what} indices out").view(np.int64)
+        itmp.read(f"{what} indices tmp")
     assert torch.equal(ws.guard(need).cpu(), before), f"{what}: workspace written past ws_bytes = {need}"
     return got, got_vals
 
@@ -260,22 +315,28 @@ def assert_words(got: np.ndarray, want: np.ndarray, what: str):
 
 
 @functools.lru_cache(maxsize=8)
-def case(width: int, n: int, order, seed: int, seg=None):
-    """(keys, reference permutation) of random bit patterns with float specials: a stable argsort of the images,
-    segment by segment if `seg` names a layout (then n is the layout's)."""
+def case(width: int, n: int, order, seed: int, seg=None, data: str = "random"):
+    """(keys, reference permutation) of random bit patterns with float specials, or (data "masked") of random images
+    with the zero bytes of MASKED: a stable argsort of the images, segment by segment if `seg` names a layout (then n
+    is the layout's)."""
     kt, desc = order
     if seg is not None:
         n = int(layout(seg)[-1])
-    keys = keys16_of(n, kt, seed) if width == 16 else keys32_of(n, kt, seed)
-    img = _ko(width).image(keys, kt, desc)
+    keys = {16: keys16_of, 32: keys32_of, 64: keys64_of}[width](n, kt, seed)
+    k = _ko(width)
+    if data == "masked":
+        w = k.bits(keys)
+        keys = k.inverse(w & w.dtype.type(MASKED[width]), kt, desc)
+    img = k.image(keys, kt, desc)
     perm = (np.argsort(img, kind="stable") if seg is None else np.lexsort((img, segment_ids(layout(seg)))))
     return keys, perm
 
 
-def expect(fam: str, n: int, order, seed: int, what: str, seg=None, algo: int = ALGO_RADIX, **kw):
+def expect(fam: str, n: int, order, seed: int, what: str, seg=None, algo: int = ALGO_RADIX, data: str = "random",
+           **kw):
     """run() on the keys of case() and compare with the reference, byte for byte."""
     width = FAMILIES[fam][0]
-    keys, perm = case(width, n, order, seed, seg)
+    keys, perm = case(width, n, order, seed, seg, data)
     got, got_vals = run(fam, keys, order, seg=seg, algo=algo, what=what, **kw)
     if algo == ALGO_LAB:
         want = oracle.radix_sort(keys).view(np.uint32)
@@ -283,7 +344,13 @@ def expect(fam: str, n: int, order, seed: int, what: str, seg=None, algo: int = 
     else:
         want = _ko(width).bits(keys)[perm]
     assert_words(got, want, what)
-    if got_vals is not None:
+    if fam in INDICES:
+        pos = np.arange(keys.size, dtype=np.int64)
+        if seg is not None:                                              # positions inside the segment
+            offs = layout(seg).astype(np.int64)
+            pos -= offs[:-1][segment_ids(offs)]
+        assert_words(got_vals, pos[perm], what + " indices")
+    elif got_vals is not None:
         assert_words(got_vals, perm.astype(np.uint32), what + " values")
 
 
@@ -350,13 +417,15 @@ def test_lab_pipeline_guarded():
 
 
 # ---- 3. stale state from another call ------------------------------------------------------------------------------
-# A job: (family, n or None, order, seed, segment layout or None, algo, in place).  Each case runs A, then B twice on
-# the shared workspace without clearing it, and names the region of state B must rewrite before it reads it.
-def J(fam, n=None, order=I32, seed=0, seg=None, algo=ALGO_RADIX, in_place=False):
-    return (fam, n if seg is None else _n_of(seg), order, seed, seg, algo, in_place)
+# A job: (family, n or None, order, seed, segment layout or None, algo, in place, data).  Each case runs A, then B
+# twice on the shared workspace without clearing it, and names the region of state B must rewrite before it reads it.
+def J(fam, n=None, order=I32, seed=0, seg=None, algo=ALGO_RADIX, in_place=False, data="random"):
+    return (fam, n if seg is None else _n_of(seg), order, seed, seg, algo, in_place, data)
 
 
 BF16_D, U16_A, F32_D, U32_D = (ko16.KEY_BF16, 1), (ko16.KEY_U16, 0), (ko.KEY_F32, 1), (ko.KEY_U32, 1)
+F32_A, I32_D, F16_A = (ko.KEY_F32, 0), (ko.KEY_I32, 1), (ko16.KEY_F16, 0)
+F64_D, F64_A, U64_A, I64_D = (ko64.KEY_F64, 1), (ko64.KEY_F64, 0), (ko64.KEY_U64, 0), (ko64.KEY_I64, 1)
 STALE = {
     # the segmented sort's lists, histograms and status rows (flags and counts of 1024 full tiles) lie where the
     # 16-bit sort keeps the not-zeroed half of its control block (incl, digit bases, skip flags, buffer plan) and its
@@ -389,13 +458,55 @@ STALE = {
     "merge_big_then_small": (J("keys", (1 << 20) + 4099, F32_D, 20, algo=ALGO_MERGE),
                              J("keys", 100001, U32_D, 21, algo=ALGO_MERGE)),
     "lab_big_then_small": (J("i32", (1 << 20) + 4099, I32, 22, algo=ALGO_LAB), J("i32", 100001, I32, 23, algo=ALGO_LAB)),
+    # The 64-bit and the indices sorts.  The indices sorts use the pairs sorts' workspace layout, and which of their
+    # passes runs last, and so stores the int64 indices, is read on the device from the plan in the control block.
+    # A runs all four passes and leaves their skip flags (clear), buffer selectors, final-copy word, digit bases and
+    # status rows with flags; B's images have bytes 1 and 3 constant: its histogram's last block must rewrite
+    # every skip flag and selector, so that pass 2, not A's pass 3, stores the int64 indices
+    "pairs_then_idx_masked": (J("pairs", 300001, F32_D, 30), J("idx", 300001, U32_D, 31, data="masked")),
+    # the other way round: A leaves passes 1 and 3 flagged as skipped and a plan that ends in pass 2; B runs all four,
+    # so its histogram's last block must clear those flags and rewrite the plan before any pass reads them
+    "idx_masked_then_pairs": (J("idx", 300001, F32_A, 32, data="masked"), J("pairs", 300001, U32_D, 33)),
+    # 8 passes of tickets and digit counts, then 8 x 256 digit bases and the 64-bit plan over the 32-bit control
+    # block and its status rows: B's memset must cover its own zeroed half, its histogram the rest, its passes the rows
+    "keys64_big_then_idx": (J("keys64", (1 << 21) + 5, F64_D, 34), J("idx", (1 << 20) + 7, I32_D, 35)),
+    # the same layout (the 16-bit sorts' workspace): A leaves the block scans, high-byte counts, bases and a plan of
+    # two executed passes in the not-zeroed half of the control block; B's high image byte is constant, so pass 1 is
+    # skipped and pass 0 must store the int64 indices
+    "pairs16_then_idx16_masked": (J("pairs16", 65537, BF16_D, 36), J("idx16", 65537, F16_A, 37, data="masked")),
+    # the two passes' status rows with flags and the indices plan, then a counting sort whose per-CTA count rows and scan
+    # results lie on them
+    "idx16_big_then_keys16_small": (J("idx16", (1 << 21) + 3, BF16_D, 38), J("keys16", 8193, U16_A, 39)),
+    # the same layout: 48 large segments leave list entries, first keys, 8-pass histograms, prefix and status rows; B
+    # has 3 large segments, so list entries past its device count, and rows past its tiles, are stale
+    "seg64_many_large_then_few_large": (J("seg64_pairs", order=F64_D, seg=MANY_LARGE_2M, seed=40),
+                                        J("seg64_pairs", order=U64_A, seg=FEW_LARGE_2M, seed=41)),
+    # 232 onesweep-class rows leave the indices sort's lists, histograms and status rows; the 64-bit segmented
+    # sort keeps its control (the vary words among it), lists, first keys and histograms there
+    "seg_idx_rows_then_seg64_ragged": (J("seg_idx", order=F32_D, seg=ROWS_9000, seed=42),
+                                       J("seg64", order=I64_D, seg=RAGGED_SMALL, seed=43)),
+    # the 64-bit lists, first keys and 8-pass histograms where the 16-bit indices sort keeps its lists, histograms and
+    # status rows (rows of 128256 bf16 keys: top-p sampling over a vocabulary)
+    "seg64_then_seg_idx16": (J("seg64_pairs", order=U64_A, seg=RAGGED_SMALL, seed=44),
+                             J("seg_idx16", order=BF16_D, seg=("rows", 128256, 16), seed=45)),
+    # the same layout as the pairs sort: A executes all four passes, B (bytes 1 and 3 constant in every row) two,
+    # so its per-segment skip decisions and its last pass must be its own
+    "seg_pairs_then_seg_idx_masked": (J("seg_pairs", order=U32_D, seg=ROWS_9000, seed=50),
+                                      J("seg_idx", order=F32_D, seg=ROWS_9000, seed=51, data="masked")),
+    "keys64_big_then_small": (J("keys64", (1 << 21) + 5, U64_A, 46), J("keys64", 65537, F64_A, 47)),
+    "seg_idx_big_then_small": (J("seg_idx", order=U32_D, seg=ROWS_9000, seed=48),
+                               J("seg_idx", order=F32_A, seg=("rows", 8193, 127), seed=49)),
 }
 
 
 def do(job, what: str):
-    fam, n, order, seed, seg, algo, in_place = job
-    expect(fam, n, order, seed, what, seg=seg, algo=algo, in_place=in_place,
-           offs=(1, 1, 2, 3, 3, 0) if in_place else OFFS32[1] if FAMILIES[fam][0] == 32 else OFFS16[1])
+    fam, n, order, seed, seg, algo, in_place, data = job
+    width = FAMILIES[fam][0]
+    if in_place:
+        offs = (2, 2, 0, 3, 3, 0) if width == 64 else (1, 1, 2, 3, 3, 0)
+    else:
+        offs = {16: OFFS16, 32: OFFS32, 64: OFFS64}[width][1]
+    expect(fam, n, order, seed, what, seg=seg, algo=algo, in_place=in_place, data=data, offs=offs)
 
 
 @pytest.mark.parametrize("name", list(STALE))
@@ -416,6 +527,19 @@ def test_segment_layouts_target_what_they_name():
     assert (r == 0).any() and (r == 1).any() and (r > (1 << 20)).sum() == 2
     lr = np.diff(layout(LONG_RAGGED))
     assert lr[0] == 1 << 22 and lr.size > 1000
+    many, few = layout(MANY_LARGE_2M), layout(FEW_LARGE_2M)
+    assert many[-1] == few[-1] == 48 * 40000 and many.size == few.size == 1025
+    big64 = lib().b200sort_segmented64_class_max(3)
+    assert int((np.diff(many) > big64).sum()) == 48 and int((np.diff(few) > big64).sum()) == 3
+    r = np.diff(layout(RAGGED_SMALL))
+    assert (r == 0).any() and (r == 1).any() and (r > big64).sum() >= 10
+    for name in ("pairs_then_idx_masked", "idx_masked_then_pairs", "pairs16_then_idx16_masked",
+                 "seg_pairs_then_seg_idx_masked"):                      # A and B execute different pass sets
+        assert [job[7] for job in STALE[name]].count("masked") == 1, name
+        for fam, n, order, seed, seg, _, _, data in STALE[name]:
+            width = FAMILIES[fam][0]
+            img = _ko(width).image(case(width, n, order, seed, seg, data)[0], *order)
+            assert (data == "masked") == (not (img & ~img.dtype.type(MASKED[width])).any()), (name, fam)
 
 
 # ---- 4. graph capture and replay of the 32-bit 1-D entry points ---------------------------------------------------
